@@ -3,7 +3,7 @@
 bench.py -- headline benchmark of the matten_b200 hot path (BASELINE.json metric:
 crystals/sec, inference forward, at N B200s, next to the CPU reference path).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], SURVEY.md section 8d "config 2"): 512 synthetic crystals per
 GPU, 64-atom diamond-cubic supercells, r_cut 5 A (N = 32 768 atoms, E = 917 504 edges), lmax-2
@@ -23,6 +23,7 @@ import sys
 import tempfile
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -188,13 +189,14 @@ def cpu_baseline(num_crystals: int, steps: int, warmup: int, seed: int = 0):
     with torch.no_grad():
         for i in range(warmup + steps):
             t0 = time.perf_counter()
-            model(b)
+            out = model(b)
             dt = time.perf_counter() - t0
             if i >= warmup:
                 times.append(dt)
     times.sort()
     med = times[len(times) // 2]
     return {"value": num_crystals / med, "unit": "crystals/s", "cores": cores, "kind": kind,
+            "outputs": {"elastic_tensor_full": out},
             "sample": f"{num_crystals} of the 512 crystals per step ({b['edge_index'].shape[1]} edges; the 512 are "
                       f"these 64 unique crystals tiled 8x with fresh jitter), median of {steps} steps after {warmup} "
                       f"warm-up, torch {torch.__version__} CPU fp32, "
@@ -244,12 +246,29 @@ def predict_config1(dev):
             "note": "BASELINE.md config 1 (B=100, N=473, E=14380); it publishes no timing for it"}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory: str, outputs) -> None:
+    """Writes each prediction of the last timed step as <directory>/<name>.npy: the inputs and weights are seeded, so
+    two builds run with the same arguments can be compared output for output."""
+    arrays = {name: t.detach().cpu().numpy() for name, t in outputs.items()}
+    nbytes = sum(a.nbytes for a in arrays.values())
+    if nbytes > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {nbytes} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
     sample = CPU_SAMPLE
-    res = cpu_baseline(sample, max(1, min(args.steps, 10)), max(1, min(args.warmup, 2)))
+    res = cpu_baseline(sample, args.steps, args.warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res["outputs"])
     line = {
         "impl": "reference", "metric": "crystals/sec (inference fwd)", "value": res["value"], "unit": "crystals/s",
         "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": res["ms_per_step"],
@@ -302,8 +321,8 @@ def run_ours(args):
 
     def step_resident():
         if captured is not None:
-            return captured(resident, check=False)["elastic_tensor_full"]
-        return model(resident, check=False)["elastic_tensor_full"]
+            return captured(resident, check=False)
+        return model(resident, check=False)
 
     out_host = torch.empty((B, 6), dtype=torch.float32).pin_memory()
     d2h_bytes = out_host.numel() * out_host.element_size()
@@ -373,11 +392,13 @@ def run_ours(args):
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record()
         for _ in range(args.steps):
-            out = step_resident()
+            preds = step_resident()
         ev1.record()
         barrier()
         ms_res = max_over_ranks(ev0.elapsed_time(ev1) / args.steps)
-        assert torch.isfinite(out).all()
+        assert torch.isfinite(preds["elastic_tensor_full"]).all()
+        # copied now: the end-to-end steps below replay the same graph into the same output buffers
+        last_preds = {k: v.cpu() for k, v in preds.items()} if args.dump_outputs else None
         # per-kernel view of the same step: a CUDA graph replay cannot carry per-kernel events and does not pass
         # through the library's launch counter, so the conv durations (CUDA events around each mt_conv_fwd on the
         # launching stream) and the launch count come from K kernel-by-kernel steps of the identical forward
@@ -536,6 +557,8 @@ def run_ours(args):
         if world == 1 and not args.no_cpu_baseline:
             res = cpu_baseline(CPU_SAMPLE, 5, 2)
             line["cpu_baseline"] = {k: res[k] for k in ("value", "unit", "cores", "kind", "sample", "same_config")}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_preds)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
@@ -554,7 +577,12 @@ def main():
     ap.add_argument("--no-predict", action="store_true", help="skip the config-1 predict() measurement")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: 512 crystals per GPU; strong: the 512 crystals split over the GPUs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the predictions of the last one as DIR/<name>.npy "
+                         "(under torchrun: rank 0's batch)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

@@ -62,9 +62,8 @@ def test_load_checkpoint_with_missing_classes(tmp_path):
     assert "state_dict" in P.load_checkpoint(tmp_path / "sd.pt")
 
 
-def test_predict_requires_cuda_when_absent():
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
+def test_predict_requires_cuda_when_absent(monkeypatch):
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)
     with pytest.raises(RuntimeError, match="no CPU fallback"):
         P.predict({"lattice": np.eye(3) * 4, "species": ["Si"], "coords": [[0, 0, 0]]})
 
