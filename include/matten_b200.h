@@ -109,6 +109,39 @@ int mt_edge_radial(int dtype, const void* edge_len, int64_t E, int mode, int num
                    double start, double end, int cutoff, double poly_p, const void* bessel_w,
                    void* edge_emb, mt_stream stream);
 
+/* Backward of the edge geometry (first derivatives only), what autograd does in the reference through
+ * with_edge_vectors, SphericalHarmonics and the radial bases.  Deterministic: no float atomics.
+ *
+ * Backward of a2 (reference src/matten/nn/_nequip.py:167-176): grad_vec[e] = J_Y(vec[e])^T grad_sh[e], including
+ * the v / max(|v|, 1e-12) normalisation when normalize != 0.  grad_sh [E,(lmax+1)^2] -> grad_vec [E,3]. */
+int mt_edge_sh_bwd(int dtype, const void* edge_vec, const void* grad_sh, int64_t E, int lmax, int normalize,
+                   void* grad_vec, mt_stream stream);
+
+/* Backward of a3 / a3' with respect to the length (reference src/matten/nn/embedding.py:185-203 for mode 0,
+ * src/matten/nn/_nequip.py:43-126 for mode 1): grad_len[e] = sum_k grad_emb[e,k] d edge_emb[e,k] / d len[e], the
+ * k-sum in order.  Arguments as in mt_edge_radial (mode 0 or 1); grad_emb [E,num_basis] -> grad_len [E].  The
+ * masks of mode 0 and the r < end factor of mode 1 have zero derivative. */
+int mt_edge_radial_bwd(int dtype, const void* edge_len, const void* grad_emb, int64_t E, int mode, int num_basis,
+                       double start, double end, int cutoff, double poly_p, const void* bessel_w, void* grad_len,
+                       mt_stream stream);
+
+/* Backward of a1 (reference src/matten/nn/_nequip.py:214-268):
+ *   dv[e]          = grad_vec[e] + grad_len[e] vec[e] / |vec[e]|     (0 for the length term where |vec[e]| = 0)
+ *   grad_pos[n]    = sum_{ei[1,e] = n} dv[e] - sum_{ei[0,e] = n} dv[e]
+ *   grad_cell[g]  += shift[e] (x) dv[e]  over the edges whose sender is in graph g
+ * edge_vec [E,3] is the forward's output; grad_vec [E,3] and grad_len [E] may be NULL (no gradient).  The sums run
+ * over the receiver CSR (rowptr [N+1], perm [E] of mt_csr_by_key on edge_index[1]) and the sender CSR of the
+ * receiver-sorted list (sender_ptr [N+1], sender_perm [E], as for mt_conv_bwd), in CSR order.  graph_ptr [B+1] int32
+ * (first node of every graph; nodes of a graph contiguous) may be NULL when B == 1.  edge_cell_shift [E,3] may be NULL
+ * (no periodic images); then grad_cell must be NULL.  Outputs grad_pos [N,3] and grad_cell [B,3,3] (either may be
+ * NULL).  workspace: mt_edge_vectors_bwd_workspace_bytes bytes. */
+size_t mt_edge_vectors_bwd_workspace_bytes(int dtype, int64_t E, int64_t B);
+int mt_edge_vectors_bwd(int dtype, const void* edge_vec, const void* grad_vec, const void* grad_len,
+                        const void* edge_cell_shift, const int32_t* rowptr, const int32_t* perm,
+                        const int32_t* sender_ptr, const int32_t* sender_perm, const int32_t* graph_ptr, int64_t N,
+                        int64_t E, int64_t B, void* grad_pos, void* grad_cell, void* workspace,
+                        size_t workspace_bytes, mt_stream stream);
+
 /* ------------------------------------------------------------------------- *
  * Index bookkeeping (bit-exact integer work).
  * ------------------------------------------------------------------------- */
@@ -291,6 +324,17 @@ int mt_conv_bwd(const mt_conv_plan* plan, int dtype, const void* x, const void* 
                 double avg_num_neighbors, const void* num_neigh, const void* grad_out, void* grad_x,
                 void* const* grad_mlp_weights, void* workspace, size_t workspace_bytes, int64_t N, int64_t E,
                 mt_stream stream);
+/* mt_conv_bwd plus the gradients with respect to the edge inputs (reference src/matten/nn/utils.py:260-263, the
+ * sh and edge_embedding arguments of tp(x[src], sh, weight_nn(edge_embedding))), in the caller's edge order:
+ *   grad_sh  [E,y_dim]        : dL/d sh
+ *   grad_emb [E,mlp_sizes[0]] : dL/d edge_embedding
+ * Either may be NULL; with both NULL this is mt_conv_bwd.  Same workspace as mt_conv_bwd. */
+int mt_conv_bwd_full(const mt_conv_plan* plan, int dtype, const void* x, const void* sh, const void* emb,
+                     const void* const* mlp_weights, const int32_t* rowptr, const int32_t* perm,
+                     const int32_t* src_sorted, const int32_t* sender_ptr, const int32_t* sender_perm,
+                     double avg_num_neighbors, const void* num_neigh, const void* grad_out, void* grad_x,
+                     void* const* grad_mlp_weights, void* grad_sh, void* grad_emb, void* workspace,
+                     size_t workspace_bytes, int64_t N, int64_t E, mt_stream stream);
 
 /* ------------------------------------------------------------------------- *
  * a8 / a11 / a13 / a14: irreps-wise linear maps.

@@ -67,6 +67,10 @@ SIGNATURES = {
     "mt_edge_vectors": (_I, [_I, _V, _V, _V, _V, _V, _L, _L, _L, _V, _V, _V, _V]),
     "mt_edge_sh": (_I, [_I, _V, _L, _I, _I, _V, _V]),
     "mt_edge_radial": (_I, [_I, _V, _L, _I, _I, _D, _D, _I, _D, _V, _V, _V]),
+    "mt_edge_sh_bwd": (_I, [_I, _V, _V, _L, _I, _I, _V, _V]),
+    "mt_edge_radial_bwd": (_I, [_I, _V, _V, _L, _I, _I, _D, _D, _I, _D, _V, _V, _V]),
+    "mt_edge_vectors_bwd_workspace_bytes": (_Z, [_I, _L, _L]),
+    "mt_edge_vectors_bwd": (_I, [_I, _V, _V, _V, _V, _V, _V, _V, _V, _V, _L, _L, _L, _V, _V, _V, _Z, _V]),
     "mt_csr_workspace_bytes": (_Z, [_L, _L]),
     "mt_csr_by_key": (_I, [_V, _L, _L, _V, _V, _V, _Z, _V, _V]),
     "mt_gather_i64_to_i32": (_I, [_V, _V, _L, _V, _V]),
@@ -85,6 +89,8 @@ SIGNATURES = {
     "mt_conv_bwd_workspace_bytes": (_Z, [C.POINTER(ConvPlanStruct), _I, _L, _L]),
     "mt_conv_bwd": (_I, [C.POINTER(ConvPlanStruct), _I, _V, _V, _V, C.POINTER(_V), _V, _V, _V, _V, _V, _D, _V, _V, _V,
                          C.POINTER(_V), _V, _Z, _L, _L, _V]),
+    "mt_conv_bwd_full": (_I, [C.POINTER(ConvPlanStruct), _I, _V, _V, _V, C.POINTER(_V), _V, _V, _V, _V, _V, _D, _V, _V,
+                              _V, C.POINTER(_V), _V, _V, _V, _Z, _L, _L, _V]),
     "mt_linear_bwd_workspace_bytes": (_Z, [_I, _L]),
     "mt_linear_bwd": (_I, [_I, C.POINTER(LinBlockStruct), _I, _I, _I, _I, _L, _V, _V, _V, _V, _V, _V, _I, _V, _I, _V,
                            _Z, _L, _V]),

@@ -3,14 +3,30 @@ Autograd bindings of the CUDA ops: every ``torch.autograd.Function`` below runs 
 C ABI in both directions (``ops.*_fwd`` / ``ops.*_bwd``).  torch only records the graph and owns the memory.
 
 Gradients are produced for what the reference trains (model/model.py: every ``nn.Parameter`` of the backbone and
-the heads) and for node features; positions / cells / edge attributes are inputs of the tensor-property models and
-get no gradient (``None``).
+the heads), for node features, and -- first derivatives only -- for the geometry: the convolution passes gradients to
+its edge inputs (spherical harmonics, radial embedding), and ``EdgeShFn`` / ``EdgeRadialFn`` / ``EdgeVectorsFn`` carry
+them on to edge vectors, positions and the cell.  The geometry functions are ``once_differentiable``: a second
+derivative through them (energy / force-style training) raises instead of returning silent zeros.
 """
 from __future__ import annotations
 
 import torch
+from torch.autograd.function import once_differentiable
 
 from . import ops
+
+
+def _first_order(backward):
+    """Backward of a geometry function: first derivatives only.  ``create_graph=True`` raises here (``torch`` runs a
+    backward with grad mode on exactly then) instead of leaving a gradient that a second backward cannot follow."""
+
+    def wrapper(ctx, *grads):
+        if torch.is_grad_enabled():
+            raise RuntimeError("matten_b200: second derivatives through the geometry (create_graph=True) are not "
+                               "supported")
+        return backward(ctx, *grads)
+
+    return wrapper
 
 
 def _sender_csr(graph, N: int):
@@ -40,16 +56,17 @@ class ConvFn(torch.autograd.Function):
     def backward(ctx, g):
         x, sh, emb, nn_, *ws = ctx.saved_tensors
         num_neigh = nn_ if nn_.numel() else None
-        need_x = ctx.needs_input_grad[0]
+        need_x, need_sh, need_emb = ctx.needs_input_grad[:3]
         need_w = any(ctx.needs_input_grad[7:])
         graph = ctx.graph
         sptr, sperm = _sender_csr(graph, x.shape[0]) if need_x else (None, None)
-        gx, gws = ops.conv_bwd(ctx.handle, x.detach(), sh.detach(), emb.detach(), [w.detach() for w in ws],
-                               graph.rowptr, graph.perm, graph.src_sorted, sptr, sperm, ctx.avg, num_neigh,
-                               g.contiguous(), need_x, need_w)
+        gx, gws, gsh, gemb = ops.conv_bwd_full(ctx.handle, x.detach(), sh.detach(), emb.detach(),
+                                               [w.detach() for w in ws], graph.rowptr, graph.perm, graph.src_sorted,
+                                               sptr, sperm, ctx.avg, num_neigh, g.contiguous(), need_x, need_w,
+                                               need_sh, need_emb)
         if gws is None:
             gws = [None] * ctx.nw
-        return (gx, None, None, None, None, None, None, *gws)
+        return (gx, gsh, gemb, None, None, None, None, *gws)
 
 
 class LinearFn(torch.autograd.Function):
@@ -132,22 +149,107 @@ class SegmentReduceFn(torch.autograd.Function):
         return ops.segment_reduce_bwd(g.contiguous(), ctx.ptr, ctx.N, ctx.reduce), None, None
 
 
-class BesselRadialFn(torch.autograd.Function):
-    """BesselBasis x PolynomialCutoff with trainable frequencies (reference src/matten/nn/_nequip.py:80-126):
-    d out[e,k] / d w_k = (2 / r_max^2) cos(w_k r / r_max) env(r); summed over edges in fixed order."""
+class EdgeRadialFn(torch.autograd.Function):
+    """Radial basis of the edge lengths (ops.edge_radial, modes 0 and 1) with gradients to the lengths and, for the
+    trainable BesselBasis (reference src/matten/nn/_nequip.py:80-126), to the frequencies:
+    d out[e,k] / d w_k = (2 / r_max^2) cos(w_k r / r_max) env(r), summed over edges in fixed order."""
 
     @staticmethod
-    def forward(ctx, bessel_w, length, num_basis, start, end, cutoff, poly_p):
-        ctx.args = (num_basis, start, end, cutoff, poly_p)
-        ctx.save_for_backward(bessel_w, length)
-        return ops.edge_radial(length, 1, num_basis, start, end, cutoff, poly_p, bessel_w.detach())
+    def forward(ctx, length, bessel_w, mode, num_basis, start, end, cutoff, poly_p):
+        ctx.args = (mode, num_basis, start, end, cutoff, poly_p)
+        bw = None if bessel_w is None else bessel_w.detach()
+        ctx.save_for_backward(length, bw)
+        return ops.edge_radial(length.detach(), mode, num_basis, start, end, cutoff, poly_p, bw)
 
     @staticmethod
+    @_first_order
+    @once_differentiable
     def backward(ctx, g):
-        w, length = ctx.saved_tensors
-        num_basis, start, end, cutoff, poly_p = ctx.args
-        dw = ops.edge_radial(length, 2, num_basis, start, end, cutoff, poly_p, w.detach())
-        return ops.col_reduce(g.contiguous(), None, dw, None), None, None, None, None, None, None
+        length, w = ctx.saved_tensors
+        mode, num_basis, start, end, cutoff, poly_p = ctx.args
+        g = g.contiguous()
+        glen = gw = None
+        if ctx.needs_input_grad[0]:
+            glen = ops.edge_radial_bwd(length, g, mode, num_basis, start, end, cutoff, poly_p, w)
+        if ctx.needs_input_grad[1]:
+            dw = ops.edge_radial(length, 2, num_basis, start, end, cutoff, poly_p, w)
+            gw = ops.col_reduce(g, None, dw, None)
+        return glen, gw, None, None, None, None, None, None
+
+
+class EdgeShFn(torch.autograd.Function):
+    """Spherical harmonics of the edge vectors (reference src/matten/nn/_nequip.py:167-176)."""
+
+    @staticmethod
+    def forward(ctx, vec, lmax, normalize):
+        ctx.args = (lmax, normalize)
+        ctx.save_for_backward(vec)
+        return ops.edge_sh(vec.detach(), lmax, normalize)
+
+    @staticmethod
+    @_first_order
+    @once_differentiable
+    def backward(ctx, g):
+        (vec,) = ctx.saved_tensors
+        return ops.edge_sh_bwd(vec, g.contiguous(), *ctx.args), None, None
+
+
+class EdgeVectorsFn(torch.autograd.Function):
+    """Edge vectors and lengths from positions and cells (reference src/matten/nn/_nequip.py:214-268).  The position
+    gradient is summed over the receiver CSR and the sender CSR of ``graph``, the cell gradient per graph over the
+    sender CSR: fixed order, no atomics."""
+
+    @staticmethod
+    def forward(ctx, pos, cell, graph, shift, batch):
+        vec, ln = ops.edge_vectors(pos.detach(), graph.edge_index, shift, None if cell is None else cell.detach(),
+                                   batch, graph.flag)
+        ctx.graph, ctx.shift, ctx.batch, ctx.N = graph, shift, batch, pos.shape[0]
+        ctx.cell_shape = None if cell is None else cell.shape
+        ctx.save_for_backward(vec)
+        ctx.set_materialize_grads(False)
+        return vec, ln
+
+    @staticmethod
+    @_first_order
+    @once_differentiable
+    def backward(ctx, gvec, glen):
+        (vec,) = ctx.saved_tensors
+        need_pos, need_cell = ctx.needs_input_grad[:2]
+        need_cell = need_cell and ctx.cell_shape is not None
+        if not (need_pos or need_cell) or (gvec is None and glen is None):
+            return None, None, None, None, None
+        graph = ctx.graph
+        B = 1 if ctx.cell_shape is None else ctx.cell_shape.numel() // 9
+        sptr, sperm = _sender_csr(graph, ctx.N)
+        gptr = graph.graph_ptr(ctx.batch, B) if (need_cell and B > 1) else None
+        gpos, gcell = ops.edge_vectors_bwd(vec, gvec, glen, ctx.shift, graph.rowptr, graph.perm, sptr, sperm, gptr,
+                                           ctx.N, B, need_pos, need_cell)
+        return gpos, (gcell.reshape(ctx.cell_shape) if need_cell else None), None, None, None
+
+
+class VectorLengthsFn(torch.autograd.Function):
+    """|v| of precomputed edge vectors; backward d|v|/dv = v / |v| (0 at v = 0, as torch.linalg.norm)."""
+
+    @staticmethod
+    def forward(ctx, vec):
+        from .functional import vector_lengths
+
+        ctx.save_for_backward(vec)
+        return vector_lengths(vec.detach())
+
+    @staticmethod
+    @_first_order
+    @once_differentiable
+    def backward(ctx, g):
+        (vec,) = ctx.saved_tensors
+        E = vec.shape[0]
+        # the edge-vector backward on a graph in which every edge is its own receiver and nothing is sent:
+        # grad_pos[e] = dv[e] = g[e] v[e] / |v[e]|
+        ar = torch.arange(E + 1, dtype=torch.int32, device=vec.device)
+        none_sent = torch.zeros(E + 1, dtype=torch.int32, device=vec.device)
+        gv, _ = ops.edge_vectors_bwd(vec, None, g.contiguous(), None, ar, ar[:E], none_sent, ar[:E], None, E, 1,
+                                     True, False)
+        return gv
 
 
 class InstanceNormFn(torch.autograd.Function):

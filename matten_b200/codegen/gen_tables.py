@@ -168,6 +168,48 @@ def _emit_sh(lmax: int) -> str:
     return "\n".join(L)
 
 
+def _emit_sh_vjp(lmax: int) -> str:
+    """Forward-mode tangents through the recursion of ``_emit_sh``, one per input axis d, contracted with the
+    output gradient: gu[d] = sum_k g[k] d out[k] / d u_d (u the unit vector; no normalisation)."""
+    L = []
+    L.append("// gu[d] = sum_k g[k] d sh_component(u)[k] / d u_d for d = 0, 1, 2 (vector-Jacobian product of sh_component).")
+    L.append("template <int LMAXV, typename T> __device__ __forceinline__ void sh_component_vjp(T x, T y, T z, const T* __restrict__ g, T* __restrict__ gu) {")
+    L.append("  gu[0] = T(0); gu[1] = T(0); gu[2] = T(0);")
+    L.append("  if constexpr (LMAXV >= 1) {")
+    L.append("    const T n1[3] = {x, y, z};")
+    L.append("    #pragma unroll")
+    L.append("    for (int d = 0; d < 3; ++d) {")
+    L.append("      const T t1[3] = {T(d == 0 ? 1 : 0), T(d == 1 ? 1 : 0), T(d == 2 ? 1 : 0)};")
+    L.append(f"      T s = {_lit(math.sqrt(3.0))} * (g[1] * t1[0] + g[2] * t1[1] + g[3] * t1[2]);")
+    prev, tprev = "n1", "t1"
+    for l in range(1, lmax):
+        C = _sh_recursion_coeff(l)
+        d = 2 * (l + 1) + 1
+        L.append(f"      if constexpr (LMAXV >= {l + 1}) {{")
+        L.append(f"        T n{l + 1}[{d}], t{l + 1}[{d}];")
+        for k in range(d):
+            terms, tterms = [], []
+            for i in range(3):
+                for j in range(2 * l + 1):
+                    v = C[k, i, j].item()
+                    if abs(v) > EPS:
+                        terms.append(f"{_lit(v)} * n1[{i}] * {prev}[{j}]")
+                        tterms.append(f"{_lit(v)} * (t1[{i}] * {prev}[{j}] + n1[{i}] * {tprev}[{j}])")
+            L.append(f"        n{l + 1}[{k}] = " + " + ".join(terms) + ";")
+            L.append(f"        t{l + 1}[{k}] = " + " + ".join(tterms) + ";")
+        base = (l + 1) ** 2
+        L.append(f"        T q = T(0);\n        #pragma unroll\n        for (int k = 0; k < {d}; ++k) q = fma(g[{base} + k], t{l + 1}[k], q);")
+        L.append(f"        s = fma({_lit(math.sqrt(2 * (l + 1) + 1))}, q, s);")
+        prev, tprev = f"n{l + 1}", f"t{l + 1}"
+    for l in range(1, lmax):
+        L.append("      }")
+    L.append("      gu[d] = s;")
+    L.append("    }")
+    L.append("  }")
+    L.append("}")
+    return "\n".join(L)
+
+
 def generate() -> str:
     types = cg_types()
     L = []
@@ -200,6 +242,7 @@ def generate() -> str:
     L.append("  }")
     L.append("}")
     L.append(_emit_sh(LMAX))
+    L.append(_emit_sh_vjp(LMAX))
     L.append("}  // namespace mt")
     return "\n".join(L) + "\n"
 

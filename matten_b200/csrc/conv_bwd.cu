@@ -1,4 +1,4 @@
-// Host side of mt_conv_bwd (include/matten_b200.h): workspace carve-up and the K0..K4 launches.
+// Host side of mt_conv_bwd / mt_conv_bwd_full (include/matten_b200.h): workspace carve-up and the K0..K4 launches.
 #include <stdlib.h>
 
 #include "conv_bwd.cuh"
@@ -72,12 +72,62 @@ static int launch_last(const ConvBwdParams& p, cudaStream_t st) {
   return MT_OK;
 }
 
+// K1: tile geometry from the shared-memory budget (two CTAs per SM when possible)
+template <typename T, bool EG>
+static int launch_conv_bwd_k1(ConvBwdParams& p, int64_t N, int64_t E, cudaStream_t st) {
+  const double avg_deg = N > 0 ? (double)E / (double)N : 1.0;
+  const size_t fixed = (size_t)p.num_paths * 16;
+  // resident CTAs per SM the register budget allows (launch bounds of conv_bwd_kernel) -> shared-memory budget per CTA:
+  // the kernel alternates staging / GEMM / contraction phases between barriers, so more small CTAs hide more of it
+  // tuning overrides are read from the environment ONCE per process: nothing on the call path touches getenv
+  static const int env_threads = [] { const char* e = getenv("MT_BWD_THREADS"); return (e && *e) ? atoi(e) : 0; }();
+  static const int env_ctas = [] { const char* e = getenv("MT_BWD_CTAS"); return (e && *e) ? atoi(e) : 0; }();
+  const int threads1 = env_threads > 0 ? env_threads : 128;  // more, smaller CTAs hide the phase barriers better (r1 sweep)
+  const int per_sm_regs = env_ctas > 0 ? env_ctas : ((sizeof(T) == 4 ? 3 : 2) * (256 / threads1));
+  const size_t budget = (size_t)(227 * 1024) / per_sm_regs - 1024;
+  // EG: one sh-gradient partial row per (item, staged edge)
+  const size_t per_edge_eg = EG ? (size_t)p.num_items * p.y_dim : 0;
+  int EC = 32, TN = 1;
+  size_t smem = 0;
+  for (;;) {
+    TN = (int)((double)EC / (avg_deg > 1.0 ? avg_deg : 1.0));
+    if (TN < 1) TN = 1;
+    if (TN > 16) TN = 16;
+    for (;;) {
+      smem = fixed + ((size_t)EC * (p.hs_stride + p.xs_stride + p.y_dim + p.wt_stride + per_edge_eg) + (size_t)TN * (p.out_dim + 1)) * sizeof(T) +
+             (size_t)EC * sizeof(int);
+      if (smem <= budget || TN == 1) break;
+      TN = TN / 2;
+    }
+    if (smem <= budget || EC == 8) break;
+    EC /= 2;
+  }
+  MT_REQUIRE(smem <= 227 * 1024, "conv_bwd tile needs %zu bytes of shared memory", smem);
+  p.chunk_edges = EC;
+  p.tile_nodes = TN;
+  static thread_local size_t cfg1 = 0;
+  if (smem > cfg1) {
+    MT_CUDA_OK(cudaFuncSetAttribute(conv_bwd_kernel<T, EG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    cfg1 = smem;
+  }
+  const int64_t tiles = ceil_div<int64_t>(N, TN);
+  int per_sm = (int)((size_t)(227 * 1024) / (smem + 1024));
+  if (per_sm > per_sm_regs) per_sm = per_sm_regs;
+  if (per_sm < 1) per_sm = 1;
+  int64_t grid = (int64_t)kNumSMs * per_sm;
+  if (grid > tiles) grid = tiles;
+  conv_bwd_kernel<T, EG><<<(int)grid, threads1, smem, st>>>(p);
+  MT_LAUNCH_OK();
+  return MT_OK;
+}
+
 template <typename T>
 static int conv_bwd_impl(const mt_conv_plan* plan, const void* x, const void* sh, const void* emb,
                          const void* const* mlp_weights, const int32_t* rowptr, const int32_t* perm,
                          const int32_t* src_sorted, const int32_t* sender_ptr, const int32_t* sender_perm, double avg,
                          const void* num_neigh, const void* grad_out, void* grad_x, void* const* grad_w,
-                         void* workspace, size_t workspace_bytes, int64_t N, int64_t E, cudaStream_t st, int dtype) {
+                         void* grad_sh, void* grad_emb, void* workspace, size_t workspace_bytes, int64_t N, int64_t E,
+                         cudaStream_t st, int dtype) {
   const int nl = plan->mlp_num_layers;
   const int H = plan->mlp_sizes[nl - 1], Wn = plan->mlp_sizes[nl];
   if (E == 0) {  // no edges: all gradients are zero
@@ -112,6 +162,8 @@ static int conv_bwd_impl(const mt_conv_plan* plan, const void* x, const void* sh
   p.wt_stride = Wn;
   p.rs = L.rs;
   p.hid_eb = L.hid_eb;
+  p.gsh = grad_sh;
+  p.gemb = grad_emb;
 
   // the MLP shape of the matten configs in fp32 takes the lane-per-edge kernels
   const bool fast_mlp = sizeof(T) == 4 && nl == 3 && p.sizes[0] <= 8 && p.sizes[1] == 32 && p.sizes[2] == 32 &&
@@ -134,56 +186,17 @@ static int conv_bwd_impl(const mt_conv_plan* plan, const void* x, const void* sh
     edge_hidden_kernel<T><<<grid0, 256, smem0, st>>>(p);
     MT_LAUNCH_OK();
   }
-  // K1: tile geometry from the shared-memory budget (two CTAs per SM when possible)
   {
-    const double avg_deg = N > 0 ? (double)E / (double)N : 1.0;
-    const size_t fixed = (size_t)p.num_paths * 16;
-    // resident CTAs per SM the register budget allows (launch bounds of conv_bwd_kernel) -> shared-memory budget per CTA:
-    // the kernel alternates staging / GEMM / contraction phases between barriers, so more small CTAs hide more of it
-    // tuning overrides are read from the environment ONCE per process: nothing on the call path touches getenv
-    static const int env_threads = [] { const char* e = getenv("MT_BWD_THREADS"); return (e && *e) ? atoi(e) : 0; }();
-    static const int env_ctas = [] { const char* e = getenv("MT_BWD_CTAS"); return (e && *e) ? atoi(e) : 0; }();
-    const int threads1 = env_threads > 0 ? env_threads : 128;  // more, smaller CTAs hide the phase barriers better (r1 sweep)
-    const int per_sm_regs = env_ctas > 0 ? env_ctas : ((sizeof(T) == 4 ? 3 : 2) * (256 / threads1));
-    const size_t budget = (size_t)(227 * 1024) / per_sm_regs - 1024;
-    int EC = 32, TN = 1;
-    size_t smem = 0;
-    for (;;) {
-      TN = (int)((double)EC / (avg_deg > 1.0 ? avg_deg : 1.0));
-      if (TN < 1) TN = 1;
-      if (TN > 16) TN = 16;
-      for (;;) {
-        smem = fixed + ((size_t)EC * (p.hs_stride + p.xs_stride + p.y_dim + p.wt_stride) + (size_t)TN * (p.out_dim + 1)) * sizeof(T) +
-               (size_t)EC * sizeof(int);
-        if (smem <= budget || TN == 1) break;
-        TN = TN / 2;
-      }
-      if (smem <= budget || EC == 8) break;
-      EC /= 2;
-    }
-    MT_REQUIRE(smem <= 227 * 1024, "conv_bwd tile needs %zu bytes of shared memory", smem);
-    p.chunk_edges = EC;
-    p.tile_nodes = TN;
-    static thread_local size_t cfg1 = 0;
-    if (smem > cfg1) {
-      MT_CUDA_OK(cudaFuncSetAttribute(conv_bwd_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      cfg1 = smem;
-    }
-    const int64_t tiles = ceil_div<int64_t>(N, TN);
-    int per_sm = (int)((size_t)(227 * 1024) / (smem + 1024));
-    if (per_sm > per_sm_regs) per_sm = per_sm_regs;
-    if (per_sm < 1) per_sm = 1;
-    int64_t grid = (int64_t)kNumSMs * per_sm;
-    if (grid > tiles) grid = tiles;
-    conv_bwd_kernel<T><<<(int)grid, threads1, smem, st>>>(p);
-    MT_LAUNCH_OK();
+    const int rc = grad_sh ? launch_conv_bwd_k1<T, true>(p, N, E, st) : launch_conv_bwd_k1<T, false>(p, N, E, st);
+    if (rc != MT_OK) return rc;
   }
   // per-sender sum of the per-edge input gradients
   if (grad_x) {
     int rc = mt_segment_sum_gather(dtype, p.DXE, sender_perm, sender_ptr, p.x_dim, N, E, grad_x, st);
     if (rc != MT_OK) return rc;
   }
-  if (grad_w) {
+  // K2 / K3 give the weight gradients and, through da of the first layer, the embedding gradient
+  if (grad_w || grad_emb) {
     int rc = MT_OK;
     switch (pad_hp_bwd(H)) {
       case 8: rc = launch_last<T, 8>(p, st); break;
@@ -192,20 +205,28 @@ static int conv_bwd_impl(const mt_conv_plan* plan, const void* x, const void* sh
       default: rc = launch_last<T, 64>(p, st); break;
     }
     if (rc != MT_OK) return rc;
-    {
+    if (grad_w) {
       const int64_t cnt = (int64_t)H * Wn;
       reduce_partials_kernel<T><<<(unsigned)ceil_div<int64_t>(cnt, 32), 256, 0, st>>>(
           static_cast<const T*>(p.PARTL), cnt, p.grid2, 0, cnt, T(1) / sqrt(T(H)), static_cast<T*>(grad_w[nl - 1]));
       MT_LAUNCH_OK();
     }
-    if (fast_mlp) {
+    if (nl == 1) {
+      if (grad_emb) {
+        int64_t ge = ceil_div<int64_t>(E * H, 256);
+        if (ge > (int64_t)kNumSMs * 8) ge = (int64_t)kNumSMs * 8;
+        emb_grad_last_kernel<T><<<(unsigned)ge, 256, 0, st>>>(p);
+        MT_LAUNCH_OK();
+      }
+    } else if (fast_mlp) {
       int64_t gf = ceil_div<int64_t>(ceil_div<int64_t>(E, 32), kHidFastWarps);
       if (gf > kHidFastCtas) gf = kHidFastCtas;
-      mlp_bwd_hidden_fast_kernel<<<(unsigned)gf, 32 * kHidFastWarps, 0, st>>>(p);
+      if (grad_emb) mlp_bwd_hidden_fast_kernel<true><<<(unsigned)gf, 32 * kHidFastWarps, 0, st>>>(p);
+      else mlp_bwd_hidden_fast_kernel<false><<<(unsigned)gf, 32 * kHidFastWarps, 0, st>>>(p);
       MT_LAUNCH_OK();
       const int nparts = (int)gf * kHidFastWarps;
       int64_t off = 0;
-      for (int l = 0; l + 1 < nl; ++l) {
+      for (int l = 0; grad_w && l + 1 < nl; ++l) {
         const int64_t cnt = (int64_t)p.sizes[l] * p.sizes[l + 1];
         reduce_partials_kernel<T><<<(unsigned)ceil_div<int64_t>(cnt, 32), 256, 0, st>>>(
             static_cast<const T*>(p.PARTH), p.hid_numel, nparts, off, cnt, T(1) / sqrt(T(p.sizes[l])),
@@ -213,18 +234,29 @@ static int conv_bwd_impl(const mt_conv_plan* plan, const void* x, const void* sh
         MT_LAUNCH_OK();
         off += cnt;
       }
-    } else if (nl > 1) {
+    } else {
       const size_t smem3 = ((size_t)3 * p.hid_eb * p.rs + (size_t)p.rs * p.rs + p.hid_numel) * sizeof(T);
       MT_REQUIRE(smem3 <= 227 * 1024, "hidden MLP too large for the backward kernel");
-      static thread_local size_t cfg3 = 0;
-      if (smem3 > cfg3) {
-        MT_CUDA_OK(cudaFuncSetAttribute(mlp_bwd_hidden_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3));
-        cfg3 = smem3;
+      if (grad_emb) {
+        static thread_local size_t cfg3e = 0;
+        if (smem3 > cfg3e) {
+          MT_CUDA_OK(cudaFuncSetAttribute(mlp_bwd_hidden_kernel<T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          (int)smem3));
+          cfg3e = smem3;
+        }
+        mlp_bwd_hidden_kernel<T, true><<<p.grid3, 256, smem3, st>>>(p);
+      } else {
+        static thread_local size_t cfg3 = 0;
+        if (smem3 > cfg3) {
+          MT_CUDA_OK(cudaFuncSetAttribute(mlp_bwd_hidden_kernel<T, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          (int)smem3));
+          cfg3 = smem3;
+        }
+        mlp_bwd_hidden_kernel<T, false><<<p.grid3, 256, smem3, st>>>(p);
       }
-      mlp_bwd_hidden_kernel<T><<<p.grid3, 256, smem3, st>>>(p);
       MT_LAUNCH_OK();
       int64_t off = 0;
-      for (int l = 0; l + 1 < nl; ++l) {
+      for (int l = 0; grad_w && l + 1 < nl; ++l) {
         const int64_t cnt = (int64_t)p.sizes[l] * p.sizes[l + 1];
         reduce_partials_kernel<T><<<(unsigned)ceil_div<int64_t>(cnt, 32), 256, 0, st>>>(
             static_cast<const T*>(p.PARTH), p.hid_numel, p.grid3, off, cnt, T(1) / sqrt(T(p.sizes[l])),
@@ -249,12 +281,12 @@ size_t mt_conv_bwd_workspace_bytes(const mt_conv_plan* plan, int dtype, int64_t 
   return bwd_layout(plan, dtype == MT_F64 ? 8 : 4, E).total;
 }
 
-int mt_conv_bwd(const mt_conv_plan* plan, int dtype, const void* x, const void* sh, const void* emb,
-                const void* const* mlp_weights, const int32_t* rowptr, const int32_t* perm,
-                const int32_t* src_sorted, const int32_t* sender_ptr, const int32_t* sender_perm,
-                double avg_num_neighbors, const void* num_neigh, const void* grad_out, void* grad_x,
-                void* const* grad_mlp_weights, void* workspace, size_t workspace_bytes, int64_t N, int64_t E,
-                mt_stream stream) {
+int mt_conv_bwd_full(const mt_conv_plan* plan, int dtype, const void* x, const void* sh, const void* emb,
+                     const void* const* mlp_weights, const int32_t* rowptr, const int32_t* perm,
+                     const int32_t* src_sorted, const int32_t* sender_ptr, const int32_t* sender_perm,
+                     double avg_num_neighbors, const void* num_neigh, const void* grad_out, void* grad_x,
+                     void* const* grad_mlp_weights, void* grad_sh, void* grad_emb, void* workspace,
+                     size_t workspace_bytes, int64_t N, int64_t E, mt_stream stream) {
   MT_ENTRY_GUARD();
   MT_REQUIRE(plan != nullptr, "null plan");
   MT_REQUIRE(plan->bw_num_items > 0 && plan->bw_item_hdr && plan->bw_lane_tab && plan->bw_path_tab,
@@ -275,10 +307,21 @@ int mt_conv_bwd(const mt_conv_plan* plan, int dtype, const void* x, const void* 
   }
   MT_DISPATCH_DTYPE(dtype, {
     return conv_bwd_impl<T>(plan, x, sh, emb, mlp_weights, rowptr, perm, src_sorted, sender_ptr, sender_perm,
-                            avg_num_neighbors, num_neigh, grad_out, grad_x, grad_mlp_weights, workspace,
-                            workspace_bytes, N, E, as_stream(stream), dtype);
+                            avg_num_neighbors, num_neigh, grad_out, grad_x, grad_mlp_weights, grad_sh, grad_emb,
+                            workspace, workspace_bytes, N, E, as_stream(stream), dtype);
   });
   return MT_OK;
+}
+
+int mt_conv_bwd(const mt_conv_plan* plan, int dtype, const void* x, const void* sh, const void* emb,
+                const void* const* mlp_weights, const int32_t* rowptr, const int32_t* perm,
+                const int32_t* src_sorted, const int32_t* sender_ptr, const int32_t* sender_perm,
+                double avg_num_neighbors, const void* num_neigh, const void* grad_out, void* grad_x,
+                void* const* grad_mlp_weights, void* workspace, size_t workspace_bytes, int64_t N, int64_t E,
+                mt_stream stream) {
+  return mt_conv_bwd_full(plan, dtype, x, sh, emb, mlp_weights, rowptr, perm, src_sorted, sender_ptr, sender_perm,
+                          avg_num_neighbors, num_neigh, grad_out, grad_x, grad_mlp_weights, nullptr, nullptr,
+                          workspace, workspace_bytes, N, E, stream);
 }
 
 }  // extern "C"

@@ -16,6 +16,14 @@
 //   K3 mlp_bwd_hidden_kernel   the hidden layers: dz = da * act'(z) * cst, dW_l partials, da_l
 //   K4 reduce_partials_kernel  fixed-order sum of the per-CTA partial weight gradients
 // and the per-sender sum of DXE rows over the sender CSR (segment_sum_gather, node_ops.cu).
+//
+// Gradients with respect to the edge inputs (mt_conv_bwd_full), in separate instantiations so that the plain backward
+// keeps its code:
+//   grad_sh   conv_bwd_kernel<T, true>: in phase B every lane also forms CG^T(x_u, g_u) w for the sh components of
+//             each path, reduced over the unit's channels by a fixed shuffle tree into one partial row per
+//             (item, staged edge) in shared memory; after phase B the rows are summed over the items in item order.
+//   grad_emb  dz0 W0^T / sqrt(fan_in) in K3 (both forms), or the column-group sum of K2's da_last for a one-layer MLP.
+// Both are written through perm (a permutation) in the caller's edge order.
 #pragma once
 #include "common.cuh"
 #include "generated/cg_gen.cuh"
@@ -59,6 +67,8 @@ struct ConvBwdParams {
   int ncg, grid2, grid3, hid_numel;
   int hid_eb;  // edges per chunk of K0 / K3
   int rs;  // row stride of the per-edge activation tiles of K0 / K3: largest input / hidden size + 1
+  void* gsh;   // [E][y_dim] gradient w.r.t. sh (original edge order), written by conv_bwd_kernel<T, true>
+  void* gemb;  // [E][sizes[0]] gradient w.r.t. the edge embedding (original edge order)
 };
 
 template <typename T>
@@ -127,15 +137,89 @@ __global__ void __launch_bounds__(256) edge_hidden_kernel(const ConvBwdParams p)
 }
 
 // ---------------------------------------------------------------------------------------------- K1
+// bwd_unit with the sh gradient: every lane of the warp runs the same trip count (idle lanes and lanes past the last
+// edge compute nothing and contribute zeros), so that the per-path sh partials can be summed over the cpw lanes of a
+// phase by a fixed xor-shuffle tree; the phase's first lane adds them to the (item, edge) row ysp[el][:] in path order.
 template <typename T, int L1>
+__device__ __forceinline__ void bwd_unit_eg(const ConvBwdParams& p, const int4* __restrict__ spath, int pfirst,
+                                            int pcount, int u, int xoff, const T* __restrict__ xs,
+                                            const T* __restrict__ ys, const T* __restrict__ wt,
+                                            const T* __restrict__ gs, const int* __restrict__ enode,
+                                            const T* __restrict__ sden, int el0, int el1, int phase, int nphase,
+                                            int c0, T* __restrict__ ysp) {
+  constexpr int D1 = 2 * L1 + 1;
+  T* __restrict__ DW = static_cast<T*>(p.DW);
+  T* __restrict__ DXE = static_cast<T*>(p.DXE);
+  const int cpw = 32 / nphase;
+  const bool leader = (threadIdx.x & (cpw - 1)) == 0;
+  const bool lane_on = u >= 0;
+  const int uu = lane_on ? u : 0;  // idle lanes read channel 0 (xoff is 0 for them) and discard the result
+  for (int base = el0; base < el1; base += nphase) {
+    const int el = base + phase;
+    const bool live = el < el1;
+    const bool on = lane_on && live;
+    const int elc = live ? el : el0;
+    T xv[D1], dxv[D1];
+    const T* xr = xs + (size_t)elc * p.xs_stride + xoff;
+#pragma unroll
+    for (int m = 0; m < D1; ++m) { xv[m] = xr[m]; dxv[m] = T(0); }
+    const T* wrow = wt + (size_t)elc * p.wt_stride;
+    const T* yrow = ys + (size_t)elc * p.y_dim;
+    const int nl_ = enode[elc];
+    const T* gn = gs + (size_t)nl_ * p.out_dim;
+    const T inv_den = sden[nl_];
+    T* dwrow = DW + (size_t)(c0 + elc) * p.Wn;
+    T* yp = ysp + (size_t)elc * p.y_dim;
+    for (int pk = 0; pk < pcount; ++pk) {
+      const int4 pt = spath[pfirst + pk];
+      const int c = pt.y + uu;
+      const T w = wrow[c] * inv_den;
+      switch (pt.x) {
+#define MT_BWD_EG_CASE(ID, A, B, C)                                           \
+  case ID:                                                                    \
+    if constexpr (A == L1) {                                                  \
+      constexpr int D2 = 2 * B + 1, D3 = 2 * C + 1;                           \
+      T yv[D2], gv[D3], dy[D2];                                               \
+      _Pragma("unroll") for (int m = 0; m < D2; ++m) { yv[m] = yrow[pt.z + m]; dy[m] = T(0); } \
+      const T* gr = gn + pt.w + uu * D3;                                      \
+      _Pragma("unroll") for (int m = 0; m < D3; ++m) gv[m] = gr[m];           \
+      if (on) {                                                               \
+        dwrow[c] = CG<A, B, C>::template dot<T>(xv, yv, gv) * inv_den;        \
+        CG<A, B, C>::template bwd_x<T>(yv, gv, w, dxv);                       \
+        CG<A, B, C>::template bwd_y<T>(xv, gv, w, dy);                        \
+      }                                                                       \
+      for (int o = cpw >> 1; o > 0; o >>= 1)                                  \
+        _Pragma("unroll") for (int m = 0; m < D2; ++m) dy[m] += __shfl_xor_sync(0xffffffffu, dy[m], o); \
+      if (leader && live)                                                     \
+        _Pragma("unroll") for (int m = 0; m < D2; ++m) yp[pt.z + m] += dy[m]; \
+    }                                                                         \
+    break;
+        MT_FOR_EACH_CG_TYPE(MT_BWD_EG_CASE)
+#undef MT_BWD_EG_CASE
+        default: break;
+      }
+    }
+    if (on) {
+      T* dxr = DXE + (size_t)(c0 + el) * p.x_dim + xoff;
+#pragma unroll
+      for (int m = 0; m < D1; ++m) dxr[m] = dxv[m];
+    }
+  }
+}
+
+template <typename T, int L1, bool EG>
 __device__ __forceinline__ void bwd_unit(const ConvBwdParams& p, const int4* __restrict__ spath, int pfirst, int pcount,
                                          int u, int xoff, const T* __restrict__ xs, const T* __restrict__ ys,
                                          const T* __restrict__ wt, const T* __restrict__ gs,
                                          const int* __restrict__ enode, const T* __restrict__ sden, int el0, int el1,
-                                         int phase, int nphase, int c0) {
+                                         int phase, int nphase, int c0, T* __restrict__ ysp) {
   constexpr int D1 = 2 * L1 + 1;
   T* __restrict__ DW = static_cast<T*>(p.DW);
   T* __restrict__ DXE = static_cast<T*>(p.DXE);
+  if constexpr (EG) {
+    bwd_unit_eg<T, L1>(p, spath, pfirst, pcount, u, xoff, xs, ys, wt, gs, enode, sden, el0, el1, phase, nphase, c0, ysp);
+    return;
+  }
   if (u < 0) return;
   for (int el = el0 + phase; el < el1; el += nphase) {
     T xv[D1], dxv[D1];
@@ -176,7 +260,7 @@ __device__ __forceinline__ void bwd_unit(const ConvBwdParams& p, const int4* __r
   }
 }
 
-template <typename T>
+template <typename T, bool EG>
 __global__ void __launch_bounds__(256, sizeof(T) == 4 ? 3 : 2) conv_bwd_kernel(const ConvBwdParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int EC = p.chunk_edges;
@@ -188,6 +272,7 @@ __global__ void __launch_bounds__(256, sizeof(T) == 4 ? 3 : 2) conv_bwd_kernel(c
   T* gs = wt + (size_t)EC * p.wt_stride;               // [tile_nodes][out_dim]
   T* sden = gs + (size_t)p.tile_nodes * p.out_dim;     // [tile_nodes] 1 / sqrt(#neighbours)
   int* enode = reinterpret_cast<int*>(sden + p.tile_nodes);  // [EC] receiver (tile-local) of every staged edge
+  T* ysp = reinterpret_cast<T*>(enode + EC);  // EG: [num_items][EC][y_dim] sh-gradient partials (EC % 8 == 0: aligned)
   __shared__ int s_counter;
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
@@ -239,6 +324,8 @@ __global__ void __launch_bounds__(256, sizeof(T) == 4 ? 3 : 2) conv_bwd_kernel(c
         while (j + 1 < tn && p.rowptr[n0 + j + 1] <= c0 + el) ++j;
         enode[el] = j;
       }
+      if constexpr (EG)
+        for (int t = tid; t < p.num_items * EC * p.y_dim; t += blockDim.x) ysp[t] = T(0);
       if (tid == 0) s_counter = 0;
       __syncthreads();
       // ------------------------------------------------------------ (A) per-edge weights into shared memory
@@ -289,13 +376,25 @@ __global__ void __launch_bounds__(256, sizeof(T) == 4 ? 3 : 2) conv_bwd_kernel(c
         const int cpw = hdr.y;
         const int phase = lane / cpw, nphase = 32 / cpw;
         const int lo = eb * 8, hi = min(lo + 8, ne);
+        T* yspi = ysp + (size_t)item * EC * p.y_dim;
         switch (hdr.x) {
-          case 0: bwd_unit<T, 0>(p, spath, hdr.z, hdr.w, ls.x, ls.y, xs, ys, wt, gs, enode, sden, lo, hi, phase, nphase, c0); break;
-          case 1: bwd_unit<T, 1>(p, spath, hdr.z, hdr.w, ls.x, ls.y, xs, ys, wt, gs, enode, sden, lo, hi, phase, nphase, c0); break;
-          case 2: bwd_unit<T, 2>(p, spath, hdr.z, hdr.w, ls.x, ls.y, xs, ys, wt, gs, enode, sden, lo, hi, phase, nphase, c0); break;
-          case 3: bwd_unit<T, 3>(p, spath, hdr.z, hdr.w, ls.x, ls.y, xs, ys, wt, gs, enode, sden, lo, hi, phase, nphase, c0); break;
-          case 4: bwd_unit<T, 4>(p, spath, hdr.z, hdr.w, ls.x, ls.y, xs, ys, wt, gs, enode, sden, lo, hi, phase, nphase, c0); break;
+          case 0: bwd_unit<T, 0, EG>(p, spath, hdr.z, hdr.w, ls.x, ls.y, xs, ys, wt, gs, enode, sden, lo, hi, phase, nphase, c0, yspi); break;
+          case 1: bwd_unit<T, 1, EG>(p, spath, hdr.z, hdr.w, ls.x, ls.y, xs, ys, wt, gs, enode, sden, lo, hi, phase, nphase, c0, yspi); break;
+          case 2: bwd_unit<T, 2, EG>(p, spath, hdr.z, hdr.w, ls.x, ls.y, xs, ys, wt, gs, enode, sden, lo, hi, phase, nphase, c0, yspi); break;
+          case 3: bwd_unit<T, 3, EG>(p, spath, hdr.z, hdr.w, ls.x, ls.y, xs, ys, wt, gs, enode, sden, lo, hi, phase, nphase, c0, yspi); break;
+          case 4: bwd_unit<T, 4, EG>(p, spath, hdr.z, hdr.w, ls.x, ls.y, xs, ys, wt, gs, enode, sden, lo, hi, phase, nphase, c0, yspi); break;
           default: break;
+        }
+      }
+      if constexpr (EG) {
+        // grad_sh of the chunk's edges: the item partials summed in item order
+        __syncthreads();
+        T* GSH = static_cast<T*>(p.gsh);
+        for (int t = tid; t < ne * p.y_dim; t += blockDim.x) {
+          const int el = t / p.y_dim, j = t - el * p.y_dim;
+          T s = T(0);
+          for (int it = 0; it < p.num_items; ++it) s += ysp[((size_t)it * EC + el) * p.y_dim + j];
+          GSH[(size_t)p.perm[c0 + el] * p.y_dim + j] = s;
         }
       }
     }
@@ -396,7 +495,7 @@ __global__ void __launch_bounds__(256) mlp_bwd_last_kernel(const ConvBwdParams p
 }
 
 // ---------------------------------------------------------------------------------------------- K3
-template <typename T>
+template <typename T, bool EMB>
 __global__ void __launch_bounds__(256) mlp_bwd_hidden_kernel(const ConvBwdParams p) {
   const int RS = p.rs, EB = p.hid_eb;
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -461,6 +560,14 @@ __global__ void __launch_bounds__(256) mlp_bwd_hidden_kernel(const ConvBwdParams
           T acc = T(0);
           for (int j = 0; j < fo; ++j) acc = fma(DZ[el * RS + j], Wl[k * (fo + 1) + j], acc);
           DA[el * RS + k] = acc;
+        }
+      } else if constexpr (EMB) {
+        // grad_emb[e][k] = sum_j DZ[e][j] W_0[k][j] / sqrt(fi)
+        for (int t = tid; t < ne * fi; t += blockDim.x) {
+          const int el = t / fi, k = t - el * fi;
+          T acc = T(0);
+          for (int j = 0; j < fo; ++j) acc = fma(DZ[el * RS + j], Wl[k * (fo + 1) + j], acc);
+          static_cast<T*>(p.gemb)[(size_t)p.perm[e0 + el] * fi + k] = acc;
         }
       }
     }
@@ -551,6 +658,7 @@ struct HidFastTile {
   float emb[32 * 8];   // [edge][k]
 };
 
+template <bool EMB>
 __global__ void __launch_bounds__(32 * kHidFastWarps) mlp_bwd_hidden_fast_kernel(const ConvBwdParams p) {
   __shared__ __align__(16) float sW1T[32 * 32];  // [j][i] = W1[i][j] / sqrt(32)
   __shared__ __align__(16) HidFastTile tiles[kHidFastWarps];
@@ -621,6 +729,18 @@ __global__ void __launch_bounds__(32 * kHidFastWarps) mlp_bwd_hidden_fast_kernel
         T.dz0[lane * 33 + 4 * i + q] = in ? dd[q] * (sg * (1.f + zz[q] * (1.f - sg))) * cst : 0.f;
       }
     }
+    if constexpr (EMB) {
+      // grad_emb[e][k] = sum_j dz0[e][j] W0[k][j] / sqrt(in0)  (W0 rows by warp-uniform loads)
+      const float* __restrict__ w0 = static_cast<const float*>(p.w[0]);
+      const float s0 = rsqrtf((float)in0);
+      float* ge = static_cast<float*>(p.gemb);
+      for (int k = 0; k < in0; ++k) {
+        float acc = 0.f;
+#pragma unroll 8
+        for (int j = 0; j < 32; ++j) acc = fmaf(T.dz0[lane * 33 + j], __ldg(w0 + k * 32 + j), acc);
+        if (in) ge[(size_t)p.perm[e] * in0 + k] = acc * s0;
+      }
+    }
     {
       const float* er = emb + (size_t)p.perm[es] * in0;
 #pragma unroll
@@ -656,6 +776,21 @@ __global__ void __launch_bounds__(32 * kHidFastWarps) mlp_bwd_hidden_fast_kernel
   float4* p1 = reinterpret_cast<float4*>(part + in0 * 32 + lane * 32);
 #pragma unroll
   for (int i = 0; i < 8; ++i) p1[i] = make_float4(gw1[2 * i].x, gw1[2 * i].y, gw1[2 * i + 1].x, gw1[2 * i + 1].y);
+}
+
+// grad_emb of a one-layer MLP (the embedding is the last layer's input): the fixed-order sum of K2's column-group
+// partials of da_last, written through perm.
+template <typename T>
+__global__ void __launch_bounds__(256) emb_grad_last_kernel(const ConvBwdParams p) {
+  const int H = p.sizes[0];
+  const T* __restrict__ DHP = static_cast<const T*>(p.DHP);
+  for (int64_t t = blockIdx.x * 256ll + threadIdx.x; t < p.E * H; t += (int64_t)gridDim.x * 256) {
+    const int64_t e = t / H;
+    const int k = (int)(t - e * H);
+    T s = T(0);
+    for (int cg = 0; cg < p.ncg; ++cg) s += DHP[((size_t)cg * p.E + e) * H + k];
+    static_cast<T*>(p.gemb)[(size_t)p.perm[e] * H + k] = s;
+  }
 }
 
 // ---------------------------------------------------------------------------------------------- K4

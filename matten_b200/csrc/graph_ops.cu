@@ -113,6 +113,145 @@ __global__ void __launch_bounds__(256) edge_radial_kernel(const T* __restrict__ 
 }
 
 // =========================================================================
+// backward of a1 - a3 (first derivatives; reference autograd through the same lines)
+// =========================================================================
+template <typename T, int LMAXV>
+__global__ void __launch_bounds__(256) edge_sh_bwd_kernel(const T* __restrict__ vec, const T* __restrict__ gsh,
+                                                          int64_t E, int normalize, T* __restrict__ gvec) {
+  constexpr int D = (LMAXV + 1) * (LMAXV + 1);
+  int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (e >= E) return;
+  T x = vec[e * 3 + 0], y = vec[e * 3 + 1], z = vec[e * 3 + 2];
+  T nr = T(1), n = T(1);
+  if (normalize) {
+    nr = sqrt(x * x + y * y + z * z);
+    n = nr > T(1e-12) ? nr : T(1e-12);
+    x /= n;
+    y /= n;
+    z /= n;
+  }
+  T g[D], gu[3];
+#pragma unroll
+  for (int k = 0; k < D; ++k) g[k] = gsh[e * D + k];
+  sh_component_vjp<LMAXV, T>(x, y, z, g, gu);
+  if (normalize) {
+    // d (v / max(|v|, eps)) / d v: (I - u u^T) / |v| above eps, I / eps below (the clamp has zero derivative)
+    const T ug = nr > T(1e-12) ? x * gu[0] + y * gu[1] + z * gu[2] : T(0);
+    gu[0] = (gu[0] - x * ug) / n;
+    gu[1] = (gu[1] - y * ug) / n;
+    gu[2] = (gu[2] - z * ug) / n;
+  }
+  gvec[e * 3 + 0] = gu[0];
+  gvec[e * 3 + 1] = gu[1];
+  gvec[e * 3 + 2] = gu[2];
+}
+
+template <typename T>
+__global__ void __launch_bounds__(256) edge_radial_bwd_kernel(const T* __restrict__ len, const T* __restrict__ g,
+                                                              int64_t E, int mode, int nb, T start, T end, int cutoff,
+                                                              T poly_p, const T* __restrict__ bessel_w,
+                                                              T* __restrict__ glen) {
+  int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (e >= E) return;
+  const T pi = T(3.14159265358979323846);
+  const T r = len[e];
+  const T* gr = g + e * nb;
+  T acc = T(0);
+  if (mode == 0) {
+    // d/dx [sqrt(2/c) sin(a x) / x] = sqrt(2/c) (a x cos(a x) - sin(a x)) / x^2, times the (constant) masks, sqrt(n)
+    const T x = r - start, c = end - start;
+    const T mask = cutoff ? ((((x / c) < T(1)) ? T(1) : T(0)) * ((T(0) < x) ? T(1) : T(0))) : T(1);
+    const T s = sqrt(T(2) / c) * mask * sqrt(T(nb));
+    for (int k = 0; k < nb; ++k) {
+      const T a = T(k + 1) * pi / c;
+      acc = fma(gr[k], s * (a * x * cos(a * x) - sin(a * x)) / (x * x), acc);
+    }
+  } else {
+    const T u = r / end, p = poly_p;
+    const T env = T(1) - ((p + T(1)) * (p + T(2)) / T(2)) * pow(u, p) + p * (p + T(2)) * pow(u, p + T(1)) -
+                  (p * (p + T(1)) / T(2)) * pow(u, p + T(2));
+    const T denv = (-((p + T(1)) * (p + T(2)) / T(2)) * p * pow(u, p - T(1)) +
+                    p * (p + T(2)) * (p + T(1)) * pow(u, p) - (p * (p + T(1)) / T(2)) * (p + T(2)) * pow(u, p + T(1))) /
+                   end;
+    const T inside = (r < end) ? T(1) : T(0);
+    for (int k = 0; k < nb; ++k) {
+      const T w = bessel_w ? bessel_w[k] : T(k + 1) * pi;
+      const T basis = (T(2) / end) * (sin(w * r / end) / r);
+      const T dbasis = (T(2) / end) * ((w / end) * r * cos(w * r / end) - sin(w * r / end)) / (r * r);
+      acc = fma(gr[k], (dbasis * env + basis * denv) * inside, acc);
+    }
+  }
+  glen[e] = acc;
+}
+
+// dv of every edge in receiver-sorted order (position i holds edge perm[i]), and shift (x) dv for the cell
+template <typename T>
+__global__ void __launch_bounds__(256) edge_dv_kernel(const T* __restrict__ vec, const T* __restrict__ gvec,
+                                                      const T* __restrict__ glen, const T* __restrict__ shift,
+                                                      const int32_t* __restrict__ perm, int64_t E,
+                                                      T* __restrict__ dvs, T* __restrict__ sdv) {
+  int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i >= E) return;
+  const int64_t e = perm[i];
+  T d[3] = {T(0), T(0), T(0)};
+  if (gvec) {
+    d[0] = gvec[e * 3 + 0];
+    d[1] = gvec[e * 3 + 1];
+    d[2] = gvec[e * 3 + 2];
+  }
+  if (glen) {
+    const T v0 = vec[e * 3 + 0], v1 = vec[e * 3 + 1], v2 = vec[e * 3 + 2];
+    const T n = sqrt(v0 * v0 + v1 * v1 + v2 * v2);
+    if (n > T(0)) {
+      const T s = glen[e] / n;
+      d[0] = fma(s, v0, d[0]);
+      d[1] = fma(s, v1, d[1]);
+      d[2] = fma(s, v2, d[2]);
+    }
+  }
+#pragma unroll
+  for (int c = 0; c < 3; ++c) dvs[i * 3 + c] = d[c];
+  if (sdv) {
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+      const T sa = shift[e * 3 + a];
+#pragma unroll
+      for (int b = 0; b < 3; ++b) sdv[i * 9 + a * 3 + b] = sa * d[b];
+    }
+  }
+}
+
+// grad_pos[n] = (sum of dv over the edges received by n) - (sum over the edges sent by n), both in CSR order
+template <typename T>
+__global__ void __launch_bounds__(256) pos_grad_kernel(const T* __restrict__ dvs, const int32_t* __restrict__ rowptr,
+                                                       const int32_t* __restrict__ sptr,
+                                                       const int32_t* __restrict__ sperm, int64_t N,
+                                                       T* __restrict__ gpos) {
+  int64_t n = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (n >= N) return;
+  T r[3] = {T(0), T(0), T(0)}, s[3] = {T(0), T(0), T(0)};
+  for (int32_t i = rowptr[n]; i < rowptr[n + 1]; ++i)
+#pragma unroll
+    for (int c = 0; c < 3; ++c) r[c] += dvs[(int64_t)i * 3 + c];
+  for (int32_t j = sptr[n]; j < sptr[n + 1]; ++j) {
+    const int64_t i = sperm[j];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) s[c] += dvs[i * 3 + c];
+  }
+#pragma unroll
+  for (int c = 0; c < 3; ++c) gpos[n * 3 + c] = r[c] - s[c];
+}
+
+// segment bounds of every graph in the sender CSR: the edges sent by nodes graph_ptr[g] .. graph_ptr[g+1]
+__global__ void __launch_bounds__(256) graph_edge_ptr_kernel(const int32_t* __restrict__ sptr,
+                                                             const int32_t* __restrict__ graph_ptr, int64_t B,
+                                                             int64_t N, int32_t* __restrict__ out) {
+  int64_t g = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (g > B) return;
+  out[g] = sptr[graph_ptr ? graph_ptr[g] : (g == 0 ? 0 : N)];
+}
+
+// =========================================================================
 // exclusive scan (int32), multi-level
 // =========================================================================
 constexpr int kScanThreads = 256;
@@ -524,6 +663,97 @@ int mt_edge_radial(int dtype, const void* edge_len, int64_t E, int mode, int num
 }
 
 static inline size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
+
+int mt_edge_sh_bwd(int dtype, const void* edge_vec, const void* grad_sh, int64_t E, int lmax, int normalize,
+                   void* grad_vec, mt_stream stream) {
+  MT_ENTRY_GUARD();
+  MT_REQUIRE(lmax >= 0 && lmax <= MT_LMAX, "lmax %d not supported (0..%d)", lmax, MT_LMAX);
+  MT_REQUIRE(E >= 0, "negative size");
+  if (E == 0) return MT_OK;
+  MT_REQUIRE(edge_vec && grad_sh && grad_vec, "null pointer");
+  cudaStream_t st = as_stream(stream);
+  unsigned g = grid_for(E, 256);
+#define MT_SH_BWD_CASE(L)                                                                                       \
+  case L:                                                                                                       \
+    edge_sh_bwd_kernel<T, L><<<g, 256, 0, st>>>((const T*)edge_vec, (const T*)grad_sh, E, normalize, (T*)grad_vec); \
+    break;
+  MT_DISPATCH_DTYPE(dtype, {
+    switch (lmax) {
+      MT_SH_BWD_CASE(0) MT_SH_BWD_CASE(1) MT_SH_BWD_CASE(2) MT_SH_BWD_CASE(3) MT_SH_BWD_CASE(4)
+    }
+  });
+#undef MT_SH_BWD_CASE
+  MT_LAUNCH_OK();
+  return MT_OK;
+}
+
+int mt_edge_radial_bwd(int dtype, const void* edge_len, const void* grad_emb, int64_t E, int mode, int num_basis,
+                       double start, double end, int cutoff, double poly_p, const void* bessel_w, void* grad_len,
+                       mt_stream stream) {
+  MT_ENTRY_GUARD();
+  MT_REQUIRE(mode == 0 || mode == 1, "radial backward mode %d", mode);
+  MT_REQUIRE(num_basis > 0 && end > start && E >= 0, "bad radial basis parameters");
+  if (E == 0) return MT_OK;
+  MT_REQUIRE(edge_len && grad_emb && grad_len, "null pointer");
+  MT_DISPATCH_DTYPE(dtype, {
+    edge_radial_bwd_kernel<T><<<grid_for(E, 256), 256, 0, as_stream(stream)>>>(
+        (const T*)edge_len, (const T*)grad_emb, E, mode, num_basis, (T)start, (T)end, cutoff, (T)poly_p,
+        (const T*)bessel_w, (T*)grad_len);
+  });
+  MT_LAUNCH_OK();
+  return MT_OK;
+}
+
+size_t mt_edge_vectors_bwd_workspace_bytes(int dtype, int64_t E, int64_t B) {
+  const size_t es = dtype == MT_F64 ? 8 : 4;
+  if (E < 0) E = 0;
+  if (B < 1) B = 1;
+  return align256((size_t)E * 3 * es) + align256((size_t)E * 9 * es) + align256((size_t)(B + 1) * 4);
+}
+
+int mt_edge_vectors_bwd(int dtype, const void* edge_vec, const void* grad_vec, const void* grad_len,
+                        const void* edge_cell_shift, const int32_t* rowptr, const int32_t* perm,
+                        const int32_t* sender_ptr, const int32_t* sender_perm, const int32_t* graph_ptr, int64_t N,
+                        int64_t E, int64_t B, void* grad_pos, void* grad_cell, void* workspace,
+                        size_t workspace_bytes, mt_stream stream) {
+  MT_ENTRY_GUARD();
+  MT_REQUIRE(N >= 0 && E >= 0 && B >= 0, "negative size");
+  MT_REQUIRE(grad_cell == nullptr || edge_cell_shift != nullptr, "grad_cell needs edge_cell_shift");
+  MT_REQUIRE(grad_cell == nullptr || B == 1 || graph_ptr != nullptr, "graph_ptr is required for more than one graph");
+  cudaStream_t st = as_stream(stream);
+  const size_t es = dtype == MT_F64 ? 8 : 4;
+  if (E == 0) {
+    if (grad_pos) MT_CUDA_OK(cudaMemsetAsync(grad_pos, 0, (size_t)N * 3 * es, st));
+    if (grad_cell) MT_CUDA_OK(cudaMemsetAsync(grad_cell, 0, (size_t)B * 9 * es, st));
+    return MT_OK;
+  }
+  if (grad_pos == nullptr && grad_cell == nullptr) return MT_OK;
+  MT_REQUIRE(edge_vec && rowptr && perm && sender_ptr && sender_perm, "null pointer");
+  MT_REQUIRE(workspace != nullptr && workspace_bytes >= mt_edge_vectors_bwd_workspace_bytes(dtype, E, B),
+             "edge_vectors_bwd workspace too small");
+  unsigned char* ws = static_cast<unsigned char*>(workspace);
+  void* dvs = ws;
+  void* sdv = grad_cell ? ws + align256((size_t)E * 3 * es) : nullptr;
+  int32_t* cptr = reinterpret_cast<int32_t*>(ws + align256((size_t)E * 3 * es) + align256((size_t)E * 9 * es));
+  MT_DISPATCH_DTYPE(dtype, {
+    edge_dv_kernel<T><<<grid_for(E, 256), 256, 0, st>>>((const T*)edge_vec, (const T*)grad_vec, (const T*)grad_len,
+                                                        (const T*)edge_cell_shift, perm, E, (T*)dvs, (T*)sdv);
+  });
+  MT_LAUNCH_OK();
+  if (grad_pos && N > 0) {
+    MT_DISPATCH_DTYPE(dtype, {
+      pos_grad_kernel<T><<<grid_for(N, 256), 256, 0, st>>>((const T*)dvs, rowptr, sender_ptr, sender_perm, N,
+                                                           (T*)grad_pos);
+    });
+    MT_LAUNCH_OK();
+  }
+  if (grad_cell && B > 0) {
+    graph_edge_ptr_kernel<<<grid_for(B + 1, 256), 256, 0, st>>>(sender_ptr, graph_ptr, B, N, cptr);
+    MT_LAUNCH_OK();
+    return mt_segment_sum_gather(dtype, sdv, sender_perm, cptr, 9, B, E, grad_cell, stream);
+  }
+  return MT_OK;
+}
 
 size_t mt_csr_workspace_bytes(int64_t num_keys, int64_t E) {
   if (E < 0) E = 0;

@@ -18,17 +18,27 @@ def _needs_grad(*ts) -> bool:
     return torch.is_grad_enabled() and any(isinstance(t, torch.Tensor) and t.requires_grad for t in ts)
 
 
-# ---- geometry (positions are inputs, not parameters: no gradient is recorded) ----
-def edge_vectors(pos, edge_index, shift, cell, batch, flag):
+# ---- geometry (first derivatives w.r.t. positions, cell and edge vectors are recorded when requested) ----
+def edge_vectors(pos, edge_index, shift, cell, batch, flag, graph=None):
+    """(vec, len) of every edge.  ``graph`` (a GraphCache of ``edge_index``) supplies the CSRs of the backward; one
+    is built when it is not given and a gradient is recorded."""
     if _needs_grad(pos, cell):
-        raise NotImplementedError("gradients w.r.t. positions / cell (forces, stress) are not part of the "
-                                  "matten tensor-property path")
-    return ops.edge_vectors(pos, edge_index, shift, cell, batch, flag)
+        from . import autograd as A
+        from .graph import GraphCache
+
+        if graph is None:
+            graph = GraphCache({"edge_index": edge_index, "pos": pos})
+        return A.EdgeVectorsFn.apply(pos, cell, graph, shift, batch)
+    return ops.edge_vectors(pos.detach(), edge_index, shift, None if cell is None else cell.detach(), batch, flag)
 
 
 def vector_lengths(vec):
     """|v| for precomputed edge vectors (reference _nequip.py:226-231) through the same kernel:
     pos = 0, shift = v, cell = I."""
+    if _needs_grad(vec):
+        from . import autograd as A
+
+        return A.VectorLengthsFn.apply(vec)
     E = vec.shape[0]
     z = torch.zeros((1, 3), dtype=vec.dtype, device=vec.device)
     ei = torch.zeros((2, E), dtype=torch.int64, device=vec.device)
@@ -38,16 +48,20 @@ def vector_lengths(vec):
 
 
 def edge_sh(vec, lmax: int, normalize: bool = True):
+    if _needs_grad(vec):
+        from . import autograd as A
+
+        return A.EdgeShFn.apply(vec, lmax, normalize)
     return ops.edge_sh(vec.detach(), lmax, normalize)
 
 
 def edge_radial(length, mode, num_basis, start, end, cutoff=True, poly_p=6.0, bessel_w=None):
-    if _needs_grad(bessel_w):
-        if mode != 1:
-            raise ValueError("trainable frequencies belong to the BesselBasis encoding (mode 1)")
+    if _needs_grad(bessel_w) and mode != 1:
+        raise ValueError("trainable frequencies belong to the BesselBasis encoding (mode 1)")
+    if _needs_grad(length, bessel_w):
         from . import autograd as A
 
-        return A.BesselRadialFn.apply(bessel_w, length.detach(), num_basis, start, end, cutoff, poly_p)
+        return A.EdgeRadialFn.apply(length, bessel_w, mode, num_basis, start, end, cutoff, poly_p)
     bw = bessel_w.detach() if bessel_w is not None else None
     return ops.edge_radial(length.detach(), mode, num_basis, start, end, cutoff, poly_p, bw)
 
@@ -81,11 +95,11 @@ def _layout(graph, sh, handle):
 
 def conv(handle: ops.ConvPlanHandle, x, sh, emb, mlp_weights: Sequence[torch.Tensor], graph,
          avg_num_neighbors: Optional[float], num_neigh=None):
-    if _needs_grad(x, *mlp_weights):
+    if _needs_grad(x, sh, emb, *mlp_weights):
         from . import autograd as A
 
         return A.ConvFn.apply(x, sh, emb, handle, graph, avg_num_neighbors, num_neigh, *mlp_weights)
-    return ops.conv_fwd(handle, x.detach(), sh, emb, [w.detach() for w in mlp_weights], graph.rowptr,
+    return ops.conv_fwd(handle, x.detach(), sh.detach(), emb.detach(), [w.detach() for w in mlp_weights], graph.rowptr,
                         graph.perm, graph.src_sorted, avg_num_neighbors, num_neigh, layout=_layout(graph, sh, handle))
 
 

@@ -22,7 +22,7 @@ def with_edge_vectors(data: DataKey.Type, with_lengths: bool = True) -> DataKey.
         return data
     g = get_graph(data)
     vec, ln = F.edge_vectors(data[DataKey.POSITIONS], g.edge_index, data.get(DataKey.EDGE_CELL_SHIFT),
-                             data.get(DataKey.CELL), data.get(DataKey.BATCH), g.flag)
+                             data.get(DataKey.CELL), data.get(DataKey.BATCH), g.flag, g)
     data[DataKey.EDGE_VECTORS] = vec
     data[DataKey.EDGE_LENGTH] = ln  # computed in the same pass; harmless when not requested
     return data

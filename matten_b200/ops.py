@@ -114,6 +114,8 @@ def edge_vectors(pos, edge_index, edge_cell_shift=None, cell=None, batch=None, f
             batch = _req(batch, "batch", torch.int64)
     vec = torch.empty((E, 3), dtype=pos.dtype, device=pos.device) if want_vec else None
     ln = torch.empty((E,), dtype=pos.dtype, device=pos.device) if want_len else None
+    if E == 0:  # nothing to compute (and an empty shift tensor has no data pointer)
+        return vec, ln
     check(lib.mt_edge_vectors(_dt(pos), _p(pos), _p(edge_index), _p(edge_cell_shift), _p(cell),
                               _p(batch) if B > 1 else None, N, E, B, _p(vec), _p(ln), _p(flag), _stream(pos)))
     return vec, ln
@@ -141,6 +143,64 @@ def edge_radial(edge_len, mode: int, num_basis: int, start: float, end: float, c
     check(lib.mt_edge_radial(_dt(edge_len), _p(edge_len), E, mode, num_basis, float(start), float(end),
                              int(cutoff), float(poly_p), _p(bessel_w), _p(out), _stream(edge_len)))
     return out
+
+
+@_on_device
+def edge_sh_bwd(edge_vec, grad_sh, lmax: int, normalize: bool = True):
+    """grad_vec [E,3] = J_Y(edge_vec)^T grad_sh (backward of edge_sh)."""
+    lib = _lib.load()
+    edge_vec = _req(edge_vec, "edge_vectors")
+    grad_sh = _req(grad_sh, "grad_sh", edge_vec.dtype)
+    E = edge_vec.shape[0]
+    out = torch.empty((E, 3), dtype=edge_vec.dtype, device=edge_vec.device)
+    check(lib.mt_edge_sh_bwd(_dt(edge_vec), _p(edge_vec), _p(grad_sh), E, lmax, int(normalize), _p(out),
+                             _stream(edge_vec)))
+    return out
+
+
+@_on_device
+def edge_radial_bwd(edge_len, grad_emb, mode: int, num_basis: int, start: float, end: float, cutoff: bool = True,
+                    poly_p: float = 6.0, bessel_w=None):
+    """grad_len [E] = sum_k grad_emb[:, k] d edge_radial[:, k] / d edge_len (modes 0 and 1)."""
+    lib = _lib.load()
+    edge_len = _req(edge_len, "edge_lengths")
+    grad_emb = _req(grad_emb, "grad_emb", edge_len.dtype)
+    E = edge_len.shape[0]
+    if bessel_w is not None:
+        bessel_w = _req(bessel_w, "bessel_weights", edge_len.dtype)
+    out = torch.empty((E,), dtype=edge_len.dtype, device=edge_len.device)
+    check(lib.mt_edge_radial_bwd(_dt(edge_len), _p(edge_len), _p(grad_emb), E, mode, num_basis, float(start),
+                                 float(end), int(cutoff), float(poly_p), _p(bessel_w), _p(out), _stream(edge_len)))
+    return out
+
+
+@_on_device
+def edge_vectors_bwd(edge_vec, grad_vec, grad_len, edge_cell_shift, rowptr, perm, sender_ptr, sender_perm,
+                     graph_ptr, N: int, B: int, want_pos: bool = True, want_cell: bool = True):
+    """(grad_pos [N,3] | None, grad_cell [B,3,3] | None): backward of edge_vectors, summed over the receiver CSR
+    (rowptr, perm) and the sender CSR of the receiver-sorted list (sender_ptr, sender_perm); graph_ptr [B+1] int32
+    may be None when B == 1."""
+    lib = _lib.load()
+    edge_vec = _req(edge_vec, "edge_vectors")
+    dt = edge_vec.dtype
+    E = edge_vec.shape[0]
+    grad_vec = None if grad_vec is None else _req(grad_vec, "grad_vec", dt)
+    grad_len = None if grad_len is None else _req(grad_len, "grad_len", dt)
+    want_cell = want_cell and edge_cell_shift is not None
+    if want_cell:
+        edge_cell_shift = _req(edge_cell_shift, "edge_cell_shift", dt)
+    if E == 0:
+        return (edge_vec.new_zeros((N, 3)) if want_pos else None,
+                edge_vec.new_zeros((B, 3, 3)) if want_cell else None)
+    gpos = torch.empty((N, 3), dtype=dt, device=edge_vec.device) if want_pos else None
+    gcell = torch.empty((B, 3, 3), dtype=dt, device=edge_vec.device) if want_cell else None
+    nbytes = lib.mt_edge_vectors_bwd_workspace_bytes(_dt(edge_vec), E, B)
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=edge_vec.device)
+    check(lib.mt_edge_vectors_bwd(_dt(edge_vec), _p(edge_vec), _p(grad_vec), _p(grad_len),
+                                  _p(edge_cell_shift) if want_cell else None, _p(rowptr), _p(perm), _p(sender_ptr),
+                                  _p(sender_perm), _p(graph_ptr), N, E, B, _p(gpos), _p(gcell), _p(ws), nbytes,
+                                  _stream(edge_vec)))
+    return gpos, gcell
 
 
 @_on_device
@@ -354,11 +414,21 @@ def conv_select_impl(name: str) -> str:
     return {v: k for k, v in _IMPLS.items()}[old]
 
 
-@_on_device
 def conv_bwd(handle: ConvPlanHandle, x, sh, emb, mlp_weights: Sequence[torch.Tensor], rowptr, perm, src_sorted,
              sender_ptr, sender_perm, avg_num_neighbors: Optional[float], num_neigh, grad_out,
              need_x: bool = True, need_w: bool = True):
     """Returns (grad_x | None, [grad of every MLP weight] | None)."""
+    gx, gws, _, _ = conv_bwd_full(handle, x, sh, emb, mlp_weights, rowptr, perm, src_sorted, sender_ptr, sender_perm,
+                                  avg_num_neighbors, num_neigh, grad_out, need_x, need_w)
+    return gx, gws
+
+
+@_on_device
+def conv_bwd_full(handle: ConvPlanHandle, x, sh, emb, mlp_weights: Sequence[torch.Tensor], rowptr, perm, src_sorted,
+                  sender_ptr, sender_perm, avg_num_neighbors: Optional[float], num_neigh, grad_out,
+                  need_x: bool = True, need_w: bool = True, need_sh: bool = False, need_emb: bool = False):
+    """Returns (grad_x | None, [grad of every MLP weight] | None, grad_sh | None, grad_emb | None); the edge
+    gradients are in the caller's edge order."""
     lib = _lib.load()
     x = _req(x, "node_features")
     sh = _req(sh, "edge_attrs", x.dtype)
@@ -370,15 +440,17 @@ def conv_bwd(handle: ConvPlanHandle, x, sh, emb, mlp_weights: Sequence[torch.Ten
     gx = torch.empty_like(x) if need_x else None
     gws = [torch.empty_like(w) for w in ws] if need_w else None
     gwptrs = (C.c_void_p * len(ws))(*[g.data_ptr() for g in gws]) if need_w else None
+    gsh = torch.empty_like(sh) if need_sh else None
+    gemb = torch.empty_like(emb) if need_emb else None
     if num_neigh is not None:
         num_neigh = _req(num_neigh, "num_neigh", x.dtype)
     nbytes = lib.mt_conv_bwd_workspace_bytes(C.byref(handle.struct), _dt(x), N, E)
     wsb = torch.empty(nbytes, dtype=torch.uint8, device=x.device) if nbytes else None
-    check(lib.mt_conv_bwd(C.byref(handle.struct), _dt(x), _p(x), _p(sh), _p(emb), wptrs, _p(rowptr), _p(perm),
-                          _p(src_sorted), _p(sender_ptr), _p(sender_perm),
-                          float(avg_num_neighbors) if avg_num_neighbors is not None else 0.0, _p(num_neigh),
-                          _p(grad_out), _p(gx), gwptrs, _p(wsb), nbytes, N, E, _stream(x)))
-    return gx, gws
+    check(lib.mt_conv_bwd_full(C.byref(handle.struct), _dt(x), _p(x), _p(sh), _p(emb), wptrs, _p(rowptr), _p(perm),
+                               _p(src_sorted), _p(sender_ptr), _p(sender_perm),
+                               float(avg_num_neighbors) if avg_num_neighbors is not None else 0.0, _p(num_neigh),
+                               _p(grad_out), _p(gx), gwptrs, _p(gsh), _p(gemb), _p(wsb), nbytes, N, E, _stream(x)))
+    return gx, gws, gsh, gemb
 
 
 # ----------------------------------------------------------------- linear --
