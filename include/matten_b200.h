@@ -104,7 +104,11 @@ int mt_edge_sh(int dtype, const void* edge_vec, int64_t E, int lmax, int normali
  *          Encoding, reference src/matten/nn/_nequip.py:43-126,180-210); bessel_w [n]
  *          holds the (trainable) frequencies, NULL means n*pi;
  *  mode 2: d(mode 1)/d bessel_w[k] per (edge, k) -- the frequency gradient is its column-wise
- *          product sum with the incoming gradient (mt_col_reduce). */
+ *          product sum with the incoming gradient (mt_col_reduce);
+ *  modes 3-6: e3nn.math.soft_one_hot_linspace(x, start, end, n, basis, cutoff) * sqrt(n) with basis
+ *          3 'gaussian', 4 'cosine', 5 'smooth_finite', 6 'fourier' (EdgeLengthEmbedding with that
+ *          basis).  Modes 3-5 without cutoff need n >= 2 (their centres are linspace(start, end, n)).
+ *  poly_p and bessel_w are read by modes 1 and 2 only; cutoff by modes 0 and 3-6. */
 int mt_edge_radial(int dtype, const void* edge_len, int64_t E, int mode, int num_basis,
                    double start, double end, int cutoff, double poly_p, const void* bessel_w,
                    void* edge_emb, mt_stream stream);
@@ -117,10 +121,11 @@ int mt_edge_radial(int dtype, const void* edge_len, int64_t E, int mode, int num
 int mt_edge_sh_bwd(int dtype, const void* edge_vec, const void* grad_sh, int64_t E, int lmax, int normalize,
                    void* grad_vec, mt_stream stream);
 
-/* Backward of a3 / a3' with respect to the length (reference src/matten/nn/embedding.py:185-203 for mode 0,
- * src/matten/nn/_nequip.py:43-126 for mode 1): grad_len[e] = sum_k grad_emb[e,k] d edge_emb[e,k] / d len[e], the
- * k-sum in order.  Arguments as in mt_edge_radial (mode 0 or 1); grad_emb [E,num_basis] -> grad_len [E].  The
- * masks of mode 0 and the r < end factor of mode 1 have zero derivative. */
+/* Backward of a3 / a3' with respect to the length (reference src/matten/nn/embedding.py:185-203 for modes 0 and
+ * 3-6, src/matten/nn/_nequip.py:43-126 for mode 1): grad_len[e] = sum_k grad_emb[e,k] d edge_emb[e,k] / d len[e],
+ * the k-sum in order.  Arguments as in mt_edge_radial (mode 0, 1 or 3-6); grad_emb [E,num_basis] -> grad_len [E].
+ * The masks of modes 0, 4 and 6 and the r < end factor of mode 1 have zero derivative; for mode 5 the derivative
+ * of exp(-1/t) is taken as 0 wherever exp(-1/t) is 0. */
 int mt_edge_radial_bwd(int dtype, const void* edge_len, const void* grad_emb, int64_t E, int mode, int num_basis,
                        double start, double end, int cutoff, double poly_p, const void* bessel_w, void* grad_len,
                        mt_stream stream);

@@ -150,8 +150,8 @@ class SegmentReduceFn(torch.autograd.Function):
 
 
 class EdgeRadialFn(torch.autograd.Function):
-    """Radial basis of the edge lengths (ops.edge_radial, modes 0 and 1) with gradients to the lengths and, for the
-    trainable BesselBasis (reference src/matten/nn/_nequip.py:80-126), to the frequencies:
+    """Radial basis of the edge lengths (ops.edge_radial, modes 0, 1 and 3-6) with gradients to the lengths and, for
+    the trainable BesselBasis (reference src/matten/nn/_nequip.py:80-126), to the frequencies:
     d out[e,k] / d w_k = (2 / r_max^2) cos(w_k r / r_max) env(r), summed over edges in fixed order."""
 
     @staticmethod

@@ -1,6 +1,7 @@
 // Edge geometry + index bookkeeping kernels (rows a1-a4 of SURVEY.md section 8).
 #include "common.cuh"
 #include "generated/cg_gen.cuh"
+#include "soft_one_hot.cuh"
 
 namespace mt {
 
@@ -98,7 +99,7 @@ __global__ void __launch_bounds__(256) edge_radial_kernel(const T* __restrict__ 
       v = v * (((x / c) < T(1)) ? T(1) : T(0)) * ((T(0) < x) ? T(1) : T(0));
     }
     v *= sqrt(T(nb));
-  } else {
+  } else if (mode <= 2) {
     T w = bessel_w ? bessel_w[k] : T(k + 1) * pi;
     // mode 2: derivative of the mode-1 value with respect to the frequency w_k (trainable BesselBasis)
     T basis = mode == 2 ? (T(2) / end) * (cos(w * r / end) / end) : (T(2) / end) * (sin(w * r / end) / r);
@@ -108,6 +109,8 @@ __global__ void __launch_bounds__(256) edge_radial_kernel(const T* __restrict__ 
             (p * (p + T(1)) / T(2)) * pow(u, p + T(2));
     env *= (r < end) ? T(1) : T(0);
     v = basis * env;
+  } else {
+    v = soft_one_hot<T, false>(mode, k, nb, r, start, end, cutoff);
   }
   out[t] = v;
 }
@@ -166,7 +169,7 @@ __global__ void __launch_bounds__(256) edge_radial_bwd_kernel(const T* __restric
       const T a = T(k + 1) * pi / c;
       acc = fma(gr[k], s * (a * x * cos(a * x) - sin(a * x)) / (x * x), acc);
     }
-  } else {
+  } else if (mode == 1) {
     const T u = r / end, p = poly_p;
     const T env = T(1) - ((p + T(1)) * (p + T(2)) / T(2)) * pow(u, p) + p * (p + T(2)) * pow(u, p + T(1)) -
                   (p * (p + T(1)) / T(2)) * pow(u, p + T(2));
@@ -180,6 +183,8 @@ __global__ void __launch_bounds__(256) edge_radial_bwd_kernel(const T* __restric
       const T dbasis = (T(2) / end) * ((w / end) * r * cos(w * r / end) - sin(w * r / end)) / (r * r);
       acc = fma(gr[k], (dbasis * env + basis * denv) * inside, acc);
     }
+  } else {
+    for (int k = 0; k < nb; ++k) acc = fma(gr[k], soft_one_hot<T, true>(mode, k, nb, r, start, end, cutoff), acc);
   }
   glen[e] = acc;
 }
@@ -645,12 +650,18 @@ int mt_edge_sh(int dtype, const void* edge_vec, int64_t E, int lmax, int normali
   return MT_OK;
 }
 
+// Without cutoff the centres of modes 3-5 are linspace(start, end, n), and their spacing needs n >= 2.
+static inline bool centred_basis_ok(int mode, int num_basis, int cutoff) {
+  return cutoff || num_basis >= 2 || mode < 3 || mode > 5;
+}
+
 int mt_edge_radial(int dtype, const void* edge_len, int64_t E, int mode, int num_basis, double start,
                    double end, int cutoff, double poly_p, const void* bessel_w, void* edge_emb,
                    mt_stream stream) {
   MT_ENTRY_GUARD();
-  MT_REQUIRE(mode >= 0 && mode <= 2, "radial mode %d", mode);
+  MT_REQUIRE(mode >= 0 && mode <= 6, "radial mode %d", mode);
   MT_REQUIRE(num_basis > 0 && end > start, "bad radial basis parameters");
+  MT_REQUIRE(centred_basis_ok(mode, num_basis, cutoff), "radial mode %d without cutoff needs num_basis >= 2", mode);
   if (E == 0) return MT_OK;
   MT_REQUIRE(edge_len && edge_emb, "null pointer");
   MT_DISPATCH_DTYPE(dtype, {
@@ -691,8 +702,9 @@ int mt_edge_radial_bwd(int dtype, const void* edge_len, const void* grad_emb, in
                        double start, double end, int cutoff, double poly_p, const void* bessel_w, void* grad_len,
                        mt_stream stream) {
   MT_ENTRY_GUARD();
-  MT_REQUIRE(mode == 0 || mode == 1, "radial backward mode %d", mode);
+  MT_REQUIRE(mode == 0 || mode == 1 || (mode >= 3 && mode <= 6), "radial backward mode %d", mode);
   MT_REQUIRE(num_basis > 0 && end > start && E >= 0, "bad radial basis parameters");
+  MT_REQUIRE(centred_basis_ok(mode, num_basis, cutoff), "radial mode %d without cutoff needs num_basis >= 2", mode);
   if (E == 0) return MT_OK;
   MT_REQUIRE(edge_len && grad_emb && grad_len, "null pointer");
   MT_DISPATCH_DTYPE(dtype, {

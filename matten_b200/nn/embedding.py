@@ -102,9 +102,14 @@ class SpeciesEmbedding(ModuleIrreps, torch.nn.Module):
         return data
 
 
+# e3nn soft_one_hot_linspace basis -> radial mode of ops.edge_radial (include/matten_b200.h, mt_edge_radial)
+_RADIAL_MODE = {"bessel": 0, "gaussian": 3, "cosine": 4, "smooth_finite": 5, "fourier": 6}
+
+
 class EdgeLengthEmbedding(ModuleIrreps, torch.nn.Module):
     """e3nn ``soft_one_hot_linspace`` of the edge length times sqrt(num_basis) (reference
-    src/matten/nn/embedding.py:158-203)."""
+    src/matten/nn/embedding.py:158-203), for any of e3nn's bases: bessel, gaussian, cosine, smooth_finite and
+    fourier."""
 
     REQUIRED_KEYS_IRREPS_IN = [DataKey.POSITIONS, DataKey.EDGE_INDEX]
 
@@ -112,14 +117,17 @@ class EdgeLengthEmbedding(ModuleIrreps, torch.nn.Module):
                  num_basis: int = 10, start: float = 0.0, end: float = 5.0, basis: str = "bessel",
                  cutoff: bool = True):
         super().__init__()
-        if basis != "bessel":
-            raise NotImplementedError("only the bessel basis used by every matten config is implemented")
+        if basis not in _RADIAL_MODE:
+            raise ValueError(f'basis="{basis}" is not a valid entry')
+        if basis in ("gaussian", "cosine", "smooth_finite") and not cutoff and num_basis < 2:
+            # the centres are linspace(start, end, num_basis), and their spacing is the width of each function
+            raise ValueError(f'basis="{basis}" without cutoff needs num_basis >= 2, got {num_basis}')
         self.num_basis, self.start, self.end, self.basis, self.cutoff = num_basis, start, end, basis, cutoff
         self.out_field = out_field
         self.init_irreps(irreps_in, irreps_out={out_field: Irreps(f"{num_basis}x0e")})
 
     def forward(self, data: DataKey.Type) -> DataKey.Type:
         data = with_edge_vectors(data, with_lengths=True)
-        data[self.out_field] = F.edge_radial(data[DataKey.EDGE_LENGTH], 0, self.num_basis, self.start, self.end,
-                                             self.cutoff)
+        data[self.out_field] = F.edge_radial(data[DataKey.EDGE_LENGTH], _RADIAL_MODE[self.basis], self.num_basis,
+                                             self.start, self.end, self.cutoff)
         return data

@@ -161,7 +161,7 @@ def edge_sh_bwd(edge_vec, grad_sh, lmax: int, normalize: bool = True):
 @_on_device
 def edge_radial_bwd(edge_len, grad_emb, mode: int, num_basis: int, start: float, end: float, cutoff: bool = True,
                     poly_p: float = 6.0, bessel_w=None):
-    """grad_len [E] = sum_k grad_emb[:, k] d edge_radial[:, k] / d edge_len (modes 0 and 1)."""
+    """grad_len [E] = sum_k grad_emb[:, k] d edge_radial[:, k] / d edge_len (modes 0, 1 and 3-6)."""
     lib = _lib.load()
     edge_len = _req(edge_len, "edge_lengths")
     grad_emb = _req(grad_emb, "grad_emb", edge_len.dtype)
