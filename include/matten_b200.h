@@ -279,10 +279,9 @@ typedef struct {
  *   (sum_{e: dst(e)=n} msg_e) / sqrt(avg_num_neighbors)        if num_neigh == NULL
  *   (sum ...)             / sqrt(num_neigh[n])                  otherwise (reference
  *   src/matten/nn/conv.py:116-120). Summation order is the CSR order: deterministic. */
-/* workspace (bytes) of the tcgen05 path: the receiver-sorted edge list in padded column order (every node's edges
- * padded to a multiple of 4 columns: original edge id and sender row per column), the last hidden activation of the
- * radial MLP as bf16 hi/mid/lo planes (192 B per column) and pair-interleaved sh rows.  0 when the plan / dtype runs
- * on the FMA-pipe kernel, which needs none. */
+/* workspace (bytes) of the tcgen05 path: room for the per-batch edge layout of mt_conv_layout_prepare, which a call
+ * without `layout` builds there, and the last hidden activation of the radial MLP as bf16 hi/mid/lo planes (192 B per
+ * column).  0 when the plan / dtype runs on the FMA-pipe kernel, which needs none. */
 size_t mt_conv_fwd_workspace_bytes(const mt_conv_plan* plan, int dtype, int64_t N, int64_t E);
 int mt_conv_fwd(const mt_conv_plan* plan, int dtype, const void* x, const void* sh,
                 const void* emb, const void* const* mlp_weights, const int32_t* rowptr,
@@ -294,7 +293,7 @@ int mt_conv_fwd(const mt_conv_plan* plan, int dtype, const void* x, const void* 
  * pair-interleaved spherical-harmonics rows.  Every PointConv layer of a forward shares the graph and edge_sh
  * (reference src/matten/model_factory/tfn_scalar_tensor.py:160-214: one spharm_edges module feeds all layers), so the
  * caller prepares them ONCE per batch and passes the buffer as `layout` to every mt_conv_fwd of that batch
- * (layout NULL: mt_conv_fwd rebuilds them in its workspace at every call).  fp32 only (the fp64 and FMA-pipe
+ * (layout NULL: mt_conv_fwd builds the same layout in its workspace at every call).  fp32 only (the fp64 and FMA-pipe
  * kernels ignore it); y_lmax is the largest degree of edge_sh, whose blocks must be 0 .. y_lmax in order.
  * layout: mt_conv_layout_bytes(y_lmax, N, E) bytes, 256-byte aligned. */
 size_t mt_conv_layout_bytes(int y_lmax, int64_t N, int64_t E);
@@ -303,8 +302,8 @@ int mt_conv_layout_prepare(int y_lmax, const void* sh, const int32_t* rowptr, co
                            mt_stream stream);
 
 /* Which fp32 kernel mt_conv_fwd uses: 0 = automatic (tcgen05 when the plan qualifies, else FMA pipes), 1 = tcgen05
- * only (MT_EINVAL when the plan does not qualify), 2 = FMA pipes only.  Process-wide; the initial value comes from
- * the environment variable MT_CONV_IMPL (auto / tc / fma), read once.  Returns the previous setting. */
+ * only (MT_EINVAL when the plan does not qualify), 2 = FMA pipes only.  Process-wide, initially 0.  Returns the
+ * previous setting. */
 int mt_conv_select_impl(int impl);
 /* Profiling aid: device buffer of >= 32 * 8 int64 that receives the per-warp phase timings (clock64 sums, slot
  * meanings in csrc/conv_fwd_tc.cuh) of CTA 0 of every following tcgen05 launch; NULL (default) turns it off. */

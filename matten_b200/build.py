@@ -26,7 +26,7 @@ NVCC_FLAGS = [
     "-Xcompiler", "-fPIC",
     "--expt-relaxed-constexpr",
     "-Xptxas", "-v",
-] + (["-DMT_TC_TIMING"] if os.environ.get("MT_TC_TIMING") else [])  # legacy switch (round 1); phase timing is now run time: TC_TIMING=1 tools/tc_check.py
+]
 
 PLAIN_SOURCES = ["api.cu", "graph_ops.cu", "node_ops.cu", "train_ops.cu", "norm_ops.cu", "conv.cu", "conv_fwd_tc.cu", "conv_bwd.cu"]
 CONV_INST = [(t, hp) for t in ("float", "double") for hp in (8, 16, 32, 64)]
@@ -79,9 +79,8 @@ def build(force: bool = False, jobs: int | None = None, verbose: bool = True) ->
         gen_tables.main()
     headers = _all_headers()
     stamp_path = os.path.join(OBJDIR, "stamp")
-    srcs = [os.path.join(CSRC, s) for s in PLAIN_SOURCES] + [os.path.join(CSRC, "conv_fwd_inst.cu")]
-    extra_srcs = [os.path.join(CSRC, s) for s in os.listdir(CSRC) if s.endswith(".cu")]
-    stamp = _deps_hash(list(set(srcs + headers + extra_srcs)))
+    srcs = [os.path.join(CSRC, s) for s in os.listdir(CSRC) if s.endswith(".cu")]
+    stamp = _deps_hash(srcs + headers)
     lib = os.path.join(LIBDIR, LIBNAME)
     if not force and os.path.exists(lib) and os.path.exists(stamp_path) and open(stamp_path).read() == stamp:
         return lib
@@ -93,14 +92,6 @@ def build(force: bool = False, jobs: int | None = None, verbose: bool = True) ->
         name = f"conv_fwd_{t}_{hp}"
         work.append((os.path.join(CSRC, "conv_fwd_inst.cu"), os.path.join(OBJDIR, name + ".o"),
                      [f"-DMT_INST_T={t}", f"-DMT_INST_HP={hp}"], os.path.join(OBJDIR, name + ".log")))
-    extra = os.path.join(CSRC, "extra_sources.txt")
-    if os.path.exists(extra):
-        for line in open(extra):
-            line = line.strip()
-            if line and not line.startswith("#"):
-                parts = line.split()
-                work.append((os.path.join(CSRC, parts[0]), os.path.join(OBJDIR, parts[1] + ".o"), parts[2:],
-                             os.path.join(OBJDIR, parts[1] + ".log")))
     jobs = jobs or min(len(work), os.cpu_count() or 4)
     if verbose:
         print(f"[matten_b200.build] compiling {len(work)} units with {jobs} jobs ...", file=sys.stderr)

@@ -68,6 +68,18 @@ __host__ __device__ constexpr I ceil_div(I a, I b) {
 
 __host__ __device__ __forceinline__ int64_t imin64(int64_t a, int64_t b) { return a < b ? a : b; }
 
+// workspace regions start at multiples of 256 bytes
+inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
+
+// padded size (8 / 16 / 32 / 64) of the last hidden layer of the radial MLP in the FMA-pipe kernels; -1: over 64
+inline int pad_hp(int h) {
+  if (h <= 8) return 8;
+  if (h <= 16) return 16;
+  if (h <= 32) return 32;
+  if (h <= 64) return 64;
+  return -1;
+}
+
 // ------------------------------------------------------------ packed fp32 --
 // Two fp32 lanes in one register pair: sm_100 issues FFMA2 / FMUL2 (two IEEE fp32 FMAs per instruction).  The
 // generated CG contractions are templates on the scalar type, so instantiating them with f2 processes two edges per

@@ -1,6 +1,4 @@
 // Host side of the fused convolution entry points (include/matten_b200.h: mt_conv_fwd).
-#include <stdlib.h>
-
 #include "conv_fwd.cuh"
 
 namespace mt {
@@ -21,36 +19,8 @@ int conv_fwd_tc_try(const mt_conv_plan* plan, const void* x, const void* sh, con
 size_t conv_fwd_tc_workspace_bytes(const mt_conv_plan* plan, int64_t N, int64_t E);
 void conv_fwd_tc_set_debug(void* p);
 
-// Tuning overrides (MT_CONV_*) are read from the environment ONCE per process: nothing on the call path touches getenv.
-struct ConvEnv {
-  int smem_kb, ec, tn, threads, ctas_per_sm, impl;
-  ConvEnv() {
-    auto geti = [](const char* name) {
-      const char* s = getenv(name);
-      return (s && *s) ? atoi(s) : -1;
-    };
-    smem_kb = geti("MT_CONV_SMEM_KB");
-    ec = geti("MT_CONV_EC");
-    tn = geti("MT_CONV_TN");
-    threads = geti("MT_CONV_THREADS");
-    ctas_per_sm = geti("MT_CONV_CTAS_PER_SM");
-    const char* s = getenv("MT_CONV_IMPL");
-    impl = (s && strcmp(s, "tc") == 0) ? 1 : ((s && strcmp(s, "fma") == 0) ? 2 : 0);
-  }
-};
-static ConvEnv& conv_env() {
-  static ConvEnv e;
-  return e;
-}
-static int env_or(int v, int dflt) { return v >= 0 ? v : dflt; }
-
-static int pad_hp(int h) {
-  if (h <= 8) return 8;
-  if (h <= 16) return 16;
-  if (h <= 32) return 32;
-  if (h <= 64) return 64;
-  return -1;
-}
+// fp32 kernel of mt_conv_fwd (mt_conv_select_impl): 0 automatic, 1 tcgen05 only, 2 FMA pipes only
+static int g_conv_impl = 0;
 
 static int validate_plan(const mt_conv_plan* plan) {
   MT_REQUIRE(plan != nullptr, "null plan");
@@ -100,18 +70,17 @@ static int conv_fwd_impl(const mt_conv_plan* plan, const void* x, const void* sh
 
   // chunk size from the shared-memory budget
   const size_t per_edge = (size_t)(2 * hp_max + p.xs_stride + p.y_dim) * sizeof(T);
-  size_t budget = (size_t)env_or(conv_env().smem_kb, sizeof(T) == 4 ? 64 : 96) * 1024;
+  const size_t budget = (size_t)(sizeof(T) == 4 ? 64 : 96) * 1024;
   int EC = (int)(budget / per_edge);
   EC = EC / 8 * 8;
   if (EC > 256) EC = 256;
   if (EC < 8) EC = 8;
-  EC = env_or(conv_env().ec, EC);
   p.chunk_edges = EC;
   double avg_deg = N > 0 ? (double)E / (double)N : 1.0;
   int TN = (int)((double)EC / (avg_deg > 1.0 ? avg_deg : 1.0));
   if (TN < 1) TN = 1;
   if (TN > 32) TN = 32;
-  p.tile_nodes = env_or(conv_env().tn, TN);
+  p.tile_nodes = TN;
   size_t hidden_w = 0;
   for (int i = 0; i + 1 < p.nl; ++i) hidden_w += (size_t)p.sizes[i] * p.sizes[i + 1];
   const size_t smem = (size_t)EC * per_edge + hidden_w * sizeof(T);
@@ -121,15 +90,13 @@ static int conv_fwd_impl(const mt_conv_plan* plan, const void* x, const void* sh
   // (CTAs/SM x threads) = (3 x 256) / (2 x 256) / (2 x 128): sh lmax 2: 4.6 / 5.5 / 8.7; lmax 3: 16.3 / 15.2 / 25.7;
   // lmax 4: 45.0 / 36.5 / 17.0.
   const int sh_lmax = p.y_dim >= 25 ? 4 : (p.y_dim >= 16 ? 3 : 2);
-  const int threads = env_or(conv_env().threads, (sizeof(T) == 4 && sh_lmax >= 4) ? 128 : 256);
-  MT_REQUIRE(threads >= 32 && threads <= 256 && threads % 32 == 0, "MT_CONV_THREADS must be 32..256");
+  const int threads = (sizeof(T) == 4 && sh_lmax >= 4) ? 128 : 256;
   int64_t tiles = ceil_div<int64_t>(N, p.tile_nodes);
   int ctas_per_sm = (int)((227 * 1024) / (smem + 1024));
   if (ctas_per_sm < 1) ctas_per_sm = 1;
   const int reg_limit = sizeof(T) == 4 ? (HP <= 32 ? 3 : 2) : 1;  // conv_fwd_min_blocks<T, HP>()
   if (ctas_per_sm > reg_limit) ctas_per_sm = reg_limit;
   if (sizeof(T) == 4 && sh_lmax >= 3 && ctas_per_sm > 2) ctas_per_sm = 2;
-  ctas_per_sm = env_or(conv_env().ctas_per_sm, ctas_per_sm);
   int64_t grid = (int64_t)kNumSMs * ctas_per_sm;
   if (grid > tiles) grid = tiles;
   if (grid < 1) grid = 1;
@@ -151,13 +118,13 @@ extern "C" {
 void mt_conv_set_debug_buffer(void* device_buffer) { conv_fwd_tc_set_debug(device_buffer); }
 
 int mt_conv_select_impl(int impl) {
-  const int old = conv_env().impl;
-  if (impl >= 0 && impl <= 2) conv_env().impl = impl;
+  const int old = g_conv_impl;
+  if (impl >= 0 && impl <= 2) g_conv_impl = impl;
   return old;
 }
 
 size_t mt_conv_fwd_workspace_bytes(const mt_conv_plan* plan, int dtype, int64_t N, int64_t E) {
-  if (plan == nullptr || dtype != MT_F32 || conv_env().impl == 2) return 0;
+  if (plan == nullptr || dtype != MT_F32 || g_conv_impl == 2) return 0;
   return conv_fwd_tc_workspace_bytes(plan, N, E);
 }
 
@@ -178,7 +145,7 @@ int mt_conv_fwd(const mt_conv_plan* plan, int dtype, const void* x, const void* 
   // fp32: Blackwell tensor-core path (radial MLP on tcgen05, weights in TMEM) when the plan qualifies;
   // mt_conv_select_impl(2) forces the FMA-pipe kernel (used by the tests to cross-check the two)
   if (dtype == MT_F32) {
-    const int impl = conv_env().impl;
+    const int impl = g_conv_impl;
     if (impl != 2) {
       int used = 0;
       rc = conv_fwd_tc_try(plan, x, sh, emb, mlp_weights, rowptr, perm, src_sorted, avg_num_neighbors, num_neigh,

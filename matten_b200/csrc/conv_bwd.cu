@@ -1,19 +1,7 @@
 // Host side of mt_conv_bwd / mt_conv_bwd_full (include/matten_b200.h): workspace carve-up and the K0..K4 launches.
-#include <stdlib.h>
-
 #include "conv_bwd.cuh"
 
 namespace mt {
-
-static size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
-
-static int pad_hp_bwd(int h) {
-  if (h <= 8) return 8;
-  if (h <= 16) return 16;
-  if (h <= 32) return 32;
-  if (h <= 64) return 64;
-  return -1;
-}
 
 struct BwdLayout {
   size_t z_off[MT_MAX_MLP_LAYERS];
@@ -79,11 +67,8 @@ static int launch_conv_bwd_k1(ConvBwdParams& p, int64_t N, int64_t E, cudaStream
   const size_t fixed = (size_t)p.num_paths * 16;
   // resident CTAs per SM the register budget allows (launch bounds of conv_bwd_kernel) -> shared-memory budget per CTA:
   // the kernel alternates staging / GEMM / contraction phases between barriers, so more small CTAs hide more of it
-  // tuning overrides are read from the environment ONCE per process: nothing on the call path touches getenv
-  static const int env_threads = [] { const char* e = getenv("MT_BWD_THREADS"); return (e && *e) ? atoi(e) : 0; }();
-  static const int env_ctas = [] { const char* e = getenv("MT_BWD_CTAS"); return (e && *e) ? atoi(e) : 0; }();
-  const int threads1 = env_threads > 0 ? env_threads : 128;  // more, smaller CTAs hide the phase barriers better (r1 sweep)
-  const int per_sm_regs = env_ctas > 0 ? env_ctas : ((sizeof(T) == 4 ? 3 : 2) * (256 / threads1));
+  const int threads1 = 128;  // more, smaller CTAs hide the phase barriers better (r1 sweep)
+  const int per_sm_regs = (sizeof(T) == 4 ? 3 : 2) * (256 / threads1);
   const size_t budget = (size_t)(227 * 1024) / per_sm_regs - 1024;
   // EG: one sh-gradient partial row per (item, staged edge)
   const size_t per_edge_eg = EG ? (size_t)p.num_items * p.y_dim : 0;
@@ -198,7 +183,7 @@ static int conv_bwd_impl(const mt_conv_plan* plan, const void* x, const void* sh
   // K2 / K3 give the weight gradients and, through da of the first layer, the embedding gradient
   if (grad_w || grad_emb) {
     int rc = MT_OK;
-    switch (pad_hp_bwd(H)) {
+    switch (pad_hp(H)) {
       case 8: rc = launch_last<T, 8>(p, st); break;
       case 16: rc = launch_last<T, 16>(p, st); break;
       case 32: rc = launch_last<T, 32>(p, st); break;

@@ -175,7 +175,7 @@ __device__ __forceinline__ void bwd_unit_eg(const ConvBwdParams& p, const int4* 
       const int c = pt.y + uu;
       const T w = wrow[c] * inv_den;
       switch (pt.x) {
-#define MT_BWD_EG_CASE(ID, A, B, C)                                           \
+#define MT_CONV_BWD_EG_CASE(ID, A, B, C)                                           \
   case ID:                                                                    \
     if constexpr (A == L1) {                                                  \
       constexpr int D2 = 2 * B + 1, D3 = 2 * C + 1;                           \
@@ -194,8 +194,8 @@ __device__ __forceinline__ void bwd_unit_eg(const ConvBwdParams& p, const int4* 
         _Pragma("unroll") for (int m = 0; m < D2; ++m) yp[pt.z + m] += dy[m]; \
     }                                                                         \
     break;
-        MT_FOR_EACH_CG_TYPE(MT_BWD_EG_CASE)
-#undef MT_BWD_EG_CASE
+        MT_FOR_EACH_CG_TYPE(MT_CONV_BWD_EG_CASE)
+#undef MT_CONV_BWD_EG_CASE
         default: break;
       }
     }
@@ -237,7 +237,7 @@ __device__ __forceinline__ void bwd_unit(const ConvBwdParams& p, const int4* __r
       const int c = pt.y + u;
       const T w = wrow[c] * inv_den;
       switch (pt.x) {
-#define MT_BWD_CASE(ID, A, B, C)                                   \
+#define MT_CONV_BWD_CASE(ID, A, B, C)                                   \
   case ID:                                                         \
     if constexpr (A == L1) {                                       \
       constexpr int D2 = 2 * B + 1, D3 = 2 * C + 1;                \
@@ -249,8 +249,8 @@ __device__ __forceinline__ void bwd_unit(const ConvBwdParams& p, const int4* __r
       CG<A, B, C>::template bwd_x<T>(yv, gv, w, dxv);              \
     }                                                              \
     break;
-        MT_FOR_EACH_CG_TYPE(MT_BWD_CASE)
-#undef MT_BWD_CASE
+        MT_FOR_EACH_CG_TYPE(MT_CONV_BWD_CASE)
+#undef MT_CONV_BWD_CASE
         default: break;
       }
     }

@@ -39,38 +39,9 @@ static bool tc_plan_qualifies(const mt_conv_plan* plan) {
   return true;
 }
 
-static inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
-
-// workspace: the padded column order of the receiver-sorted edge list and what the fused kernel streams per column
-struct TcWorkspace {
-  size_t rowptr_pad, scan_tmp, orig_pad, src_pad, hplanes, ypairs, total;
-  int64_t cols_max;
-  size_t scan_bytes;
-};
-static TcWorkspace tc_workspace(const mt_conv_plan* plan, int64_t N, int64_t E) {
-  TcWorkspace w;
-  w.cols_max = (E + 3 * N + 3) & ~(int64_t)3;
-  if (w.cols_max < 4) w.cols_max = 4;
-  w.scan_bytes = 0;
-  cub::DeviceScan::ExclusiveSum(nullptr, w.scan_bytes, (const int32_t*)nullptr, (int32_t*)nullptr, (int)(N + 1));
-  size_t o = 0;
-  w.rowptr_pad = o;
-  o += align256((size_t)(N + 1) * 4 * 2);  // padded degrees, then their scan
-  w.scan_tmp = o;
-  o += align256(w.scan_bytes);
-  w.orig_pad = o;
-  o += align256((size_t)w.cols_max * 4);
-  w.src_pad = o;
-  o += align256((size_t)w.cols_max * 4);
-  w.hplanes = o;
-  o += align256((size_t)w.cols_max * 192);
-  w.ypairs = o;
-  o += align256((size_t)(w.cols_max / 2) * 2 * sh_pad_len(plan->tc_y_lmax) * 4);
-  w.total = o + 256;
-  return w;
-}
-
-// layer-invariant part kept by the caller (mt_conv_layout_prepare): same regions as in the workspace
+// The per-batch edge layout: the padded column order of the receiver-sorted edge list and the pair-interleaved sh rows
+// the fused kernel streams per column.  mt_conv_layout_prepare builds it once per batch in the caller's buffer; a call
+// without a layout builds it at the start of its own workspace.
 struct TcLayout {
   size_t rowptr_pad, scan_tmp, orig_pad, src_pad, ypairs, total;
   int64_t cols_max;
@@ -84,7 +55,7 @@ static TcLayout tc_layout(int y_lmax, int64_t N, int64_t E) {
   cub::DeviceScan::ExclusiveSum(nullptr, w.scan_bytes, (const int32_t*)nullptr, (int32_t*)nullptr, (int)(N + 1));
   size_t o = 0;
   w.rowptr_pad = o;
-  o += align256((size_t)(N + 1) * 4 * 2);
+  o += align256((size_t)(N + 1) * 4 * 2);  // padded degrees, then their scan
   w.scan_tmp = o;
   o += align256(w.scan_bytes);
   w.orig_pad = o;
@@ -97,17 +68,32 @@ static TcLayout tc_layout(int y_lmax, int64_t N, int64_t E) {
   return w;
 }
 
-static int tc_prepare_order(const int32_t* rowptr, const int32_t* perm, const int32_t* src_sorted, int64_t N,
-                            int32_t* degp, int32_t* rowptr_pad, void* scan_tmp, size_t scan_bytes, int32_t* orig_pad,
-                            int32_t* src_pad, cudaStream_t st) {
+// workspace of a call: the layout, the h planes of the layer (192 bytes per column) and slack to align the buffer to
+// 256 bytes
+static size_t tc_workspace_bytes(const TcLayout& L) { return L.total + align256((size_t)L.cols_max * 192) + 256; }
+
+// fills the layout L at `base` (256-byte aligned): padded column order, then the sh pair rows
+static int tc_prepare_layout(const TcLayout& L, uintptr_t base, int y_lmax, const float* sh, const int32_t* rowptr,
+                             const int32_t* perm, const int32_t* src_sorted, int64_t N, cudaStream_t st) {
+  int32_t* degp = reinterpret_cast<int32_t*>(base + L.rowptr_pad);
+  int32_t* rowptr_pad = degp + (N + 1);
+  int32_t* orig_pad = reinterpret_cast<int32_t*>(base + L.orig_pad);
   tc_pad_degree_kernel<<<(unsigned)ceil_div<int64_t>(N + 1, 256), 256, 0, st>>>(rowptr, N, degp);
   MT_LAUNCH_OK();
-  MT_CUDA_OK(cub::DeviceScan::ExclusiveSum(scan_tmp, scan_bytes, degp, rowptr_pad, (int)(N + 1), st));
+  size_t scan_bytes = L.scan_bytes;
+  MT_CUDA_OK(cub::DeviceScan::ExclusiveSum(reinterpret_cast<void*>(base + L.scan_tmp), scan_bytes, degp, rowptr_pad,
+                                           (int)(N + 1), st));
   count_launch();
   int64_t g = ceil_div<int64_t>(N * 32, 256);
   if (g > (int64_t)kNumSMs * 32) g = (int64_t)kNumSMs * 32;
   if (g < 1) g = 1;
-  tc_pad_layout_kernel<<<(unsigned)g, 256, 0, st>>>(rowptr, rowptr_pad, perm, src_sorted, N, orig_pad, src_pad);
+  tc_pad_layout_kernel<<<(unsigned)g, 256, 0, st>>>(rowptr, rowptr_pad, perm, src_sorted, N, orig_pad,
+                                                    reinterpret_cast<int32_t*>(base + L.src_pad));
+  MT_LAUNCH_OK();
+  g = ceil_div<int64_t>(L.cols_max, 256);
+  if (g > (int64_t)kNumSMs * 8) g = (int64_t)kNumSMs * 8;
+  tc_ypairs_kernel<<<(unsigned)g, 256, 0, st>>>(sh, rowptr_pad, orig_pad, N, y_lmax,
+                                                reinterpret_cast<float*>(base + L.ypairs));
   MT_LAUNCH_OK();
   return MT_OK;
 }
@@ -127,25 +113,13 @@ extern "C" int mt_conv_layout_prepare(int y_lmax, const void* sh, const int32_t*
   MT_REQUIRE(layout && layout_bytes >= L.total && (reinterpret_cast<uintptr_t>(layout) & 255) == 0,
              "conv layout: buffer of mt_conv_layout_bytes() bytes, 256-byte aligned, required");
   MT_REQUIRE(rowptr && (E == 0 || (sh && perm && src_sorted)), "null pointer");
-  cudaStream_t st = as_stream(stream);
-  const uintptr_t base = reinterpret_cast<uintptr_t>(layout);
-  int32_t* degp = reinterpret_cast<int32_t*>(base + L.rowptr_pad);
-  int32_t* rowptr_pad = degp + (N + 1);
-  int32_t* orig_pad = reinterpret_cast<int32_t*>(base + L.orig_pad);
-  int rc = tc_prepare_order(rowptr, perm, src_sorted, N, degp, rowptr_pad, reinterpret_cast<void*>(base + L.scan_tmp),
-                            L.scan_bytes, orig_pad, reinterpret_cast<int32_t*>(base + L.src_pad), st);
-  if (rc != MT_OK) return rc;
-  int64_t g = ceil_div<int64_t>(L.cols_max, 256);
-  if (g > (int64_t)kNumSMs * 8) g = (int64_t)kNumSMs * 8;
-  tc_ypairs_kernel<<<(unsigned)g, 256, 0, st>>>(static_cast<const float*>(sh), rowptr_pad, orig_pad, N, y_lmax,
-                                                reinterpret_cast<float*>(base + L.ypairs));
-  MT_LAUNCH_OK();
-  return MT_OK;
+  return tc_prepare_layout(L, reinterpret_cast<uintptr_t>(layout), y_lmax, static_cast<const float*>(sh), rowptr, perm,
+                           src_sorted, N, as_stream(stream));
 }
 
 size_t conv_fwd_tc_workspace_bytes(const mt_conv_plan* plan, int64_t N, int64_t E) {
   if (!tc_plan_qualifies(plan) || N <= 0) return 0;
-  return tc_workspace(plan, N, E).total;
+  return tc_workspace_bytes(tc_layout(plan->tc_y_lmax, N, E));
 }
 
 static long long* g_tc_dbg = nullptr;  // phase-timing buffer of the next launches (mt_conv_set_debug_buffer)
@@ -178,8 +152,8 @@ int conv_fwd_tc_try(const mt_conv_plan* plan, const void* x, const void* sh, con
   *used = 0;
   if (!tc_plan_qualifies(plan)) return MT_OK;
   if (E + 3 * N >= (int64_t)2147483647 || N >= (int64_t)2147483647) return MT_OK;
-  const TcWorkspace W = tc_workspace(plan, N, E);
-  if (workspace == nullptr || workspace_bytes < W.total) return MT_OK;
+  const TcLayout L = tc_layout(plan->tc_y_lmax, N, E);
+  if (workspace == nullptr || workspace_bytes < tc_workspace_bytes(L)) return MT_OK;
   if ((reinterpret_cast<uintptr_t>(x) & 15) != 0) return MT_OK;
   EncodeTiledFn encode = encode_tiled_fn();
   if (encode == nullptr) return set_error(MT_ECUDA, "cuTensorMapEncodeTiled is not available from this driver");
@@ -194,7 +168,6 @@ int conv_fwd_tc_try(const mt_conv_plan* plan, const void* x, const void* sh, con
   for (int i = 0; i < p.nl; ++i) p.w[i] = static_cast<const float*>(mlp_weights[i]);
   p.act = plan->mlp_act;
   p.act_cst = (float)plan->mlp_act_cst;
-  p.sh = static_cast<const float*>(sh);
   p.emb = static_cast<const float*>(emb);
   p.rowptr = rowptr;
   p.perm = perm;
@@ -208,39 +181,27 @@ int conv_fwd_tc_try(const mt_conv_plan* plan, const void* x, const void* sh, con
   p.dbg = g_tc_dbg;
   {
     const uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255;
-    int32_t* degp = reinterpret_cast<int32_t*>(base + W.rowptr_pad);
-    p.rowptr_pad = degp + (N + 1);
-    p.orig_pad = reinterpret_cast<int32_t*>(base + W.orig_pad);
-    p.src_pad = reinterpret_cast<int32_t*>(base + W.src_pad);
-    p.hplanes = reinterpret_cast<__nv_bfloat16*>(base + W.hplanes);
-    p.ypairs = reinterpret_cast<float*>(base + W.ypairs);
-    p.cols_max = W.cols_max;
-    if (layout != nullptr) {
-      // prepared once per batch by mt_conv_layout_prepare: padded column order + sh pair rows
-      const TcLayout L = tc_layout(plan->tc_y_lmax, N, E);
-      const uintptr_t lb = reinterpret_cast<uintptr_t>(layout);
-      p.rowptr_pad = reinterpret_cast<int32_t*>(lb + L.rowptr_pad) + (N + 1);
-      p.orig_pad = reinterpret_cast<int32_t*>(lb + L.orig_pad);
-      p.src_pad = reinterpret_cast<int32_t*>(lb + L.src_pad);
-      p.ypairs = reinterpret_cast<float*>(lb + L.ypairs);
-      p.skip_y = 1;
-    } else {
-      // (1) padded column order
-      int rc = tc_prepare_order(rowptr, perm, src_sorted, N, degp, p.rowptr_pad, reinterpret_cast<void*>(base + W.scan_tmp),
-                                W.scan_bytes, p.orig_pad, p.src_pad, st);
+    if (layout == nullptr) {  // no per-batch layout from the caller: build it in the workspace
+      const int rc = tc_prepare_layout(L, base, plan->tc_y_lmax, static_cast<const float*>(sh), rowptr, perm, src_sorted,
+                                       N, st);
       if (rc != MT_OK) return rc;
+      layout = reinterpret_cast<const void*>(base);
     }
-    // (2) hidden layers of the radial MLP + sh pair rows, per padded column
-    {
-      const bool fast = p.nl == 3 && p.sizes[0] <= 8 && p.sizes[1] == kTcK && p.sizes[2] == kTcK &&
-                        p.act == MT_ACT_SILU;
-      int64_t g = ceil_div<int64_t>(W.cols_max, fast ? 256 : 64);
-      if (g > (int64_t)kNumSMs * 8) g = (int64_t)kNumSMs * 8;
-      if (g < 1) g = 1;
-      if (fast) tc_edge_hidden_fast_kernel<<<(unsigned)g, 256, 0, st>>>(p);
-      else tc_edge_hidden_kernel<<<(unsigned)g, kHidThreads, 0, st>>>(p);
-      MT_LAUNCH_OK();
-    }
+    const uintptr_t lb = reinterpret_cast<uintptr_t>(layout);
+    p.rowptr_pad = reinterpret_cast<int32_t*>(lb + L.rowptr_pad) + (N + 1);
+    p.orig_pad = reinterpret_cast<int32_t*>(lb + L.orig_pad);
+    p.src_pad = reinterpret_cast<int32_t*>(lb + L.src_pad);
+    p.ypairs = reinterpret_cast<float*>(lb + L.ypairs);
+    p.hplanes = reinterpret_cast<__nv_bfloat16*>(base + L.total);
+    p.cols_max = L.cols_max;
+    // hidden layers of the radial MLP, per padded column
+    const bool fast = p.nl == 3 && p.sizes[0] <= 8 && p.sizes[1] == kTcK && p.sizes[2] == kTcK && p.act == MT_ACT_SILU;
+    int64_t g = ceil_div<int64_t>(L.cols_max, fast ? 256 : 64);
+    if (g > (int64_t)kNumSMs * 8) g = (int64_t)kNumSMs * 8;
+    if (g < 1) g = 1;
+    if (fast) tc_edge_hidden_fast_kernel<<<(unsigned)g, 256, 0, st>>>(p);
+    else tc_edge_hidden_kernel<<<(unsigned)g, kHidThreads, 0, st>>>(p);
+    MT_LAUNCH_OK();
   }
   // CTAs per part follow the part's cost (every part walks all edges; heavy parts get more SMs)
   int64_t grid = kNumSMs;

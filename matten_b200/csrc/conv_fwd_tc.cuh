@@ -80,19 +80,17 @@ struct ConvTcParams {
   int act;
   float act_cst;
   const float* w[MT_MAX_MLP_LAYERS];
-  const float* sh;
   const float* emb;
   const int32_t* rowptr;
   const int32_t* perm;
   const int32_t* src;
-  // padded column order (workspace, written by the two preparation kernels)
+  // per-batch edge layout (kernels (0)), except hplanes (workspace, kernel (1))
   int32_t* rowptr_pad;        // [N+1] first padded column of every node (multiples of 4); [N] = number of columns
   int32_t* orig_pad;          // [cols] original edge id of the column (pad column: -1 - id of the node's last edge)
   int32_t* src_pad;           // [cols] sender row of the column
   __nv_bfloat16* hplanes;     // [3][4][cols_max][8] bf16: plane, k-group, column, k % 8
   float* ypairs;              // [cols_max / 2][2 * y_pad]: pair-interleaved padded sh rows
   int64_t cols_max;           // allocated columns (E + 3 N rounded up to 4)
-  int skip_y;                 // ypairs come prepared (mt_conv_layout_prepare): the hidden-layer kernel leaves them alone
   float avg;
   const float* num_neigh;
   float* out;
@@ -590,8 +588,8 @@ __global__ void __launch_bounds__(256) tc_pad_layout_kernel(const int32_t* __res
   }
 }
 
-// hidden layers + sh pair rows: four lanes per column (lane q4 produces outputs 8 q4 .. 8 q4 + 7), 8 columns per warp
-// pass; layer inputs / outputs are exchanged through a shared-memory row per column (stride 33: conflict free)
+// hidden layers: four lanes per column (lane q4 produces outputs 8 q4 .. 8 q4 + 7), 8 columns per warp pass; layer
+// inputs / outputs are exchanged through a shared-memory row per column (stride 33: conflict free)
 constexpr int kHidThreads = 256;
 __global__ void __launch_bounds__(kHidThreads) tc_edge_hidden_kernel(const ConvTcParams p) {
   __shared__ __align__(16) float sW[2 * kTcK * kTcK];
@@ -608,9 +606,7 @@ __global__ void __launch_bounds__(kHidThreads) tc_edge_hidden_kernel(const ConvT
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int q4 = lane & 3, cl = lane >> 2;
-  const int in0 = p.sizes[0], yn = p.y_dim;
-  const int yq = (yn + 3) >> 2;  // sh components per lane: [q4 * yq, min(yn, (q4 + 1) * yq))
-  const int ystride = 2 * sh_pad_len(p.y_lmax);
+  const int in0 = p.sizes[0];
   float* vrow = sV + (warp * 8 + cl) * 33;
   const int64_t cols = p.rowptr_pad[p.N];
   uint4* planes = reinterpret_cast<uint4*>(p.hplanes);
@@ -621,19 +617,6 @@ __global__ void __launch_bounds__(kHidThreads) tc_edge_hidden_kernel(const ConvT
     const int oe = in ? p.orig_pad[c] : 0;
     const bool real = in && oe >= 0;
     const int64_t orig = oe >= 0 ? oe : (-1 - oe);
-    if (in && !p.skip_y) {
-      // sh components -> pair-interleaved padded row: degree-l block at position sh_pad_pos(l)
-      const float* __restrict__ yr = p.sh + orig * yn;
-      float* yo = p.ypairs + (c >> 1) * ystride + (c & 1);
-#pragma unroll
-      for (int i = 0; i < 7; ++i) {
-        const int j = q4 * yq + i;
-        if (i < yq && j < yn) {
-          const int l = (j >= 16) ? 4 : (j >= 9) ? 3 : (j >= 4) ? 2 : (j >= 1) ? 1 : 0;
-          yo[2 * (sh_pad_pos(l) + j - l * l)] = yr[j];
-        }
-      }
-    }
     const float* er = p.emb + orig * in0;
     __syncwarp();
 #pragma unroll
@@ -690,8 +673,8 @@ __global__ void __launch_bounds__(kHidThreads) tc_edge_hidden_kernel(const ConvT
   }
 }
 
-// sh rows -> pair-interleaved padded rows, one lane per column (the layer-invariant half of the stage above, run once
-// per batch by mt_conv_layout_prepare)
+// sh rows -> pair-interleaved padded rows (degree-l block at position sh_pad_pos(l)), one lane per column: the only
+// writer of ypairs
 __global__ void __launch_bounds__(256) tc_ypairs_kernel(const float* __restrict__ sh, const int32_t* __restrict__ rowptr_pad,
                                                         const int32_t* __restrict__ orig_pad, int64_t N, int ylmax,
                                                         float* __restrict__ ypairs) {
@@ -727,27 +710,14 @@ __global__ void __launch_bounds__(256, 3) tc_edge_hidden_fast_kernel(const ConvT
     for (int t = threadIdx.x; t < kTcK * kTcK; t += 256) sW1[t] = p.w[1][t] * s1;
   }
   __syncthreads();
-  const int yn = p.y_dim, ylmax = p.y_lmax;
-  const int ystride = 2 * sh_pad_len(ylmax);
-  const int64_t cols = p.rowptr_pad[p.N];
+  const uint32_t cols = p.rowptr_pad[p.N];  // < 2^31 (E + 3 N < 2^31): 32-bit column indices save registers
   uint4* planes = reinterpret_cast<uint4*>(p.hplanes);
   const float cst = p.act_cst;
   const bool emb_vec = in0 == 8 && (reinterpret_cast<uintptr_t>(p.emb) & 15) == 0;
-  for (int64_t c = blockIdx.x * 256ll + threadIdx.x; c < cols; c += (int64_t)gridDim.x * 256) {
+  for (uint32_t c = blockIdx.x * 256 + threadIdx.x; c < cols; c += gridDim.x * 256) {
     const int oe = p.orig_pad[c];
     const bool real = oe >= 0;
     const int64_t orig = real ? oe : (-1 - oe);
-    if (!p.skip_y) {  // sh components -> pair-interleaved padded row: degree-l block at position sh_pad_pos(l)
-      const float* __restrict__ yr = p.sh + orig * yn;
-      float* yo = p.ypairs + (c >> 1) * ystride + (c & 1);
-#pragma unroll
-      for (int l = 0; l <= MT_LMAX; ++l) {
-        if (l <= ylmax) {
-#pragma unroll
-          for (int k = 0; k < 2 * l + 1; ++k) yo[2 * (sh_pad_pos(l) + k)] = yr[l * l + k];
-        }
-      }
-    }
     float h0[8];
     if (emb_vec) {
       const float4* er = reinterpret_cast<const float4*>(p.emb + orig * 8);

@@ -673,8 +673,6 @@ int mt_edge_radial(int dtype, const void* edge_len, int64_t E, int mode, int num
   return MT_OK;
 }
 
-static inline size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
-
 int mt_edge_sh_bwd(int dtype, const void* edge_vec, const void* grad_sh, int64_t E, int lmax, int normalize,
                    void* grad_vec, mt_stream stream) {
   MT_ENTRY_GUARD();
