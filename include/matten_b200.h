@@ -351,6 +351,8 @@ int mt_conv_bwd_full(const mt_conv_plan* plan, int dtype, const void* x, const v
  * For each block b:  out[n, out_off + w*dim + m] (+)= scale *
  *        sum_u weight[w_off + (u*S + s_n)*mul_out + w] * x[n, in_off + u*dim + m]
  * A block with mul_in == 0 zero-fills its output range (irreps with no path).
+ * dim must be 2l+1 for l <= 4 (1, 3, 5, 7 or 9); mt_linear_fwd and mt_linear_bwd return
+ * MT_EINVAL for any other dim, and for a block outside in_dim / out_dim, before any launch.
  * ------------------------------------------------------------------------- */
 typedef struct {
   int32_t in_off, out_off, mul_in, mul_out, dim, w_off;

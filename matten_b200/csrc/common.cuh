@@ -71,6 +71,18 @@ __host__ __device__ __forceinline__ int64_t imin64(int64_t a, int64_t b) { retur
 // workspace regions start at multiples of 256 bytes
 inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 
+// ------------------------------------------------------------ species-indexed linear (node_ops.cu) --
+// MT_OK iff every block has dim 2l+1 <= 9 and lies within in_dim / out_dim, and, when reads_weight, the weight is
+// given for every block with input channels.  mt_linear_fwd and mt_linear_bwd check their blocks with it.
+// Both are internal to the library: hidden from its dynamic symbol table, which holds the C ABI.
+__attribute__((visibility("hidden"))) int linear_check_blocks(const mt_lin_block* blocks, int num_blocks, int in_dim,
+                                                              int out_dim, const void* weight, bool reads_weight);
+// Backward of mt_linear_fwd w.r.t. x: the transposed weight slices applied to grad_out, for checked blocks.
+__attribute__((visibility("hidden"))) int linear_transposed(
+    int dtype, const mt_lin_block* blocks, int num_blocks, int in_dim, int out_dim, int num_species,
+    const void* grad_out, const void* weight, const int32_t* species_perm, const int32_t* species_ptr, int accumulate,
+    void* grad_x, int64_t N, cudaStream_t st);
+
 // padded size (8 / 16 / 32 / 64) of the last hidden layer of the radial MLP in the FMA-pipe kernels; -1: over 64
 inline int pad_hp(int h) {
   if (h <= 8) return 8;

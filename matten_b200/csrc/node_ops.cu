@@ -1,5 +1,8 @@
 // Node-side kernels: species-indexed irreps linear (a8/a11/a13/a14), Gate + BatchNorm
 // affine (a9/a10), segmented pooling (a12).  See include/matten_b200.h for the contract.
+#include <algorithm>
+#include <vector>
+
 #include "common.cuh"
 
 namespace mt {
@@ -10,21 +13,22 @@ namespace mt {
 //   src/matten/nn/conv.py:59-61,77-79,84-86 and e3nn.o3.Linear at
 //   src/matten/nn/nodewise.py:111.  With one-hot attributes the "uvw" tensor product is
 //   a per-species dense matrix per irrep type; nodes are grouped by species so each CTA
-//   multiplies a [rows x mul_in] tile (rows = (node, m)) by ONE [mul_in x mul_out]
-//   weight slice staged in shared memory (register-tiled 4x4 FMA micro-kernel).
+//   applies ONE species' [mul_in x mul_out] weight slices, staged in shared memory, to a tile of its nodes.
+//
+// Node-streaming: one CTA owns a tile of nodes of ONE species and walks ALL irrep blocks over it.
+//   * the species' weight slices of every block sit in shared memory for the CTA's lifetime;
+//   * each block's input columns of the tile's rows arrive by cp.async (16 B per lane, coalesced along the row), one
+//     block ahead of the arithmetic, so x is read from HBM exactly once and never passes through registers;
+//   * lanes <-> output channels w, NB nodes per lane in registers: per 4 input channels a lane issues 4 LDS.32 of
+//     weights (conflict free), NB x D LDS.128 of x (warp-wide broadcast) and NB x 4 x D FMAs.
+// The round-1 tiled kernel spent 152 k thread instructions per node on lin2 of the last layer for 14.8 k MACs (rows
+// of 1392 floats cut into 80-byte slivers per k-chunk, every chunk paying the DRAM latency): ncu r2_step_full.
+// Two pipelines share that arithmetic: linear_sync_kernel (CTA-synchronous tiles, short rows) and
+// linear_stream_kernel (warp-private, rows of >= 512 elements).  Blocks whose weight slice and rows fit neither in
+// shared memory are cut into rectangles of their weight on the host (linear_apply).
 // =========================================================================
 constexpr int kLinMaxBlocks = 24;
-constexpr int kLinStage = 4096;  // x elements staged per k-chunk: ROWS x KC
-constexpr int kLinMaxRows = 1024;
-constexpr int kLinMaxDim = 9;    // 2l+1 for l <= 4 takes the fast tables; larger dims fall back to divisions
-// Tile shapes (256 threads, thread tile TM rows x 4 columns):
-//   COLS  TM  ROWS  KC     stage elems 2 x (KC x (ROWS+4) + KC x COLS)     output tile ROWS x (COLS+1)
-//    64    8   128  32     12544                                            8320
-//    32    8   256  16      9344                                            8448
-//    16    8   512   8      8512                                            8704
-//     8    4   512   8      8384                                            4608
-//     4    4  1024   4      8256                                            5120
-constexpr int kLinSmemElems = 12544;
+constexpr int kStreamSmemBytes = 200 * 1024;
 
 template <typename T>
 __device__ __forceinline__ void lin_ld4(const T* p, T (&v)[4]);
@@ -58,11 +62,10 @@ struct LinParams {
   int num_blocks;
   int32_t in_off[kLinMaxBlocks], out_off[kLinMaxBlocks], mul_in[kLinMaxBlocks], mul_out[kLinMaxBlocks],
       dim[kLinMaxBlocks], w_off[kLinMaxBlocks];
+  // row stride of the weight: weight[w_off + (u * S + s) * ld + w] (transposed: [w_off + (w * S + s) * ld + u]).
+  // ld is the mul_out (transposed: mul_in) of the whole block, also when the block is one piece of a cut.
+  int32_t ld[kLinMaxBlocks];
   double scale[kLinMaxBlocks];
-  int32_t cta_begin[kLinMaxBlocks + 1];  // prefix of CTA counts per block
-  int32_t col_chunks[kLinMaxBlocks];     // ceil(mul_out / cols)
-  int32_t nodes_per_tile[kLinMaxBlocks];
-  int32_t tile_cols[kLinMaxBlocks];      // 64 / 32 / 16 / 8 / 4
   int in_dim, out_dim, S;
   const void* x;
   const void* weight;
@@ -74,191 +77,6 @@ struct LinParams {
   int64_t N;
 };
 
-struct LinTile {
-  int b, s, c0, ncols, tn, mi, mo, d, COLS, lc, ROWS, KC, XS;
-};
-
-// k loop + epilogue of one tile with a TM x 4 register tile per thread.  The k-chunks are double buffered in shared
-// memory and filled by cp.async one chunk ahead (round 1's kernel staged through registers with an integer division
-// per element and exposed the global latency: ncu r2_step_full, 38 % ALU pipe, 45 % long-scoreboard stalls, 8 % of
-// the instructions useful FMAs).  All index arithmetic in the loops is additive; the two (q / d, q % d) maps come from
-// tables filled once per CTA.
-template <typename T, int TM>
-__device__ __forceinline__ void lin_tile_run(const LinParams& p, const LinTile& t, T* smem, const int* s_nodes,
-                                             const int* qmap, const int* omap) {
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int COLS = t.COLS, KC = t.KC, XS = t.XS, d = t.d, mi = t.mi;
-  const int stage_elems = KC * XS + KC * COLS;
-  const T* __restrict__ X = static_cast<const T*>(p.x);
-  const T* __restrict__ W = static_cast<const T*>(p.weight);
-  T* __restrict__ OUT = static_cast<T*>(p.out);
-  const int tcn = COLS >> 2;
-  const int tc = tid % tcn, tr = tid / tcn;
-  using P = typename pair_of<T>::type;  // column pairs: one FFMA2 per pair in fp32
-  P acc[TM][2];
-#pragma unroll
-  for (int i = 0; i < TM; ++i)
-#pragma unroll
-    for (int j = 0; j < 2; ++j) { acc[i][j].x = T(0); acc[i][j].y = T(0); }
-
-  const int nchunks = (mi + KC - 1) / KC;
-  const int kcd = KC * d;
-  auto issue = [&](int c) {
-    T* xsT = smem + (size_t)(c & 1) * stage_elems;  // [KC][XS]
-    T* ws = xsT + KC * XS;                          // [KC][COLS]
-    const int u0 = c * KC;
-    const int ku = min(KC, mi - u0);
-    const int seg = ku * d;
-    // x rows: warps over nodes, lanes over the node's contiguous [u0 * d, (u0 + KC) * d) segment (coalesced)
-    for (int j = warp; j < t.tn; j += 8) {
-      const T* src = X + (size_t)s_nodes[j] * p.in_dim + p.in_off[t.b] + u0 * d;
-      T* dst = xsT + j * d;
-      for (int q = lane; q < kcd; q += 32) lin_cp_async<T>(dst + qmap[q], src + (q < seg ? q : 0), q < seg);
-    }
-    // weight slice ws[uu][c] = W[w_off + ((u0+uu)*S + s)*mo + c0 + c]  (transposed: roles of u and c swapped)
-    for (int e = tid; e < KC * COLS; e += 256) {
-      const int uu = e >> t.lc, c = e & (COLS - 1);
-      const bool ok = uu < ku && c < t.ncols;
-      const size_t off = p.transpose ? (size_t)p.w_off[t.b] + ((size_t)(t.c0 + c) * p.S + t.s) * mi + (u0 + uu)
-                                     : (size_t)p.w_off[t.b] + ((size_t)(u0 + uu) * p.S + t.s) * t.mo + t.c0 + c;
-      lin_cp_async<T>(ws + e, W + (ok ? off : 0), ok);
-    }
-    lin_cp_commit();
-  };
-
-  issue(0);
-  for (int c = 0; c < nchunks; ++c) {
-    if (c + 1 < nchunks) {
-      issue(c + 1);
-      lin_cp_wait<1>();
-    } else {
-      lin_cp_wait<0>();
-    }
-    __syncthreads();
-    const T* xsT = smem + (size_t)(c & 1) * stage_elems;
-    const T* ws = xsT + KC * XS;
-    const T* ap = xsT + tr * TM;
-    const T* bp = ws + tc * 4;
-#pragma unroll 4
-    for (int uu = 0; uu < KC; ++uu) {
-      T a[TM], bb[4];
-#pragma unroll
-      for (int i = 0; i < TM; i += 4) lin_ld4<T>(ap + uu * XS + i, *reinterpret_cast<T(*)[4]>(&a[i]));
-      lin_ld4<T>(bp + uu * COLS, bb);
-#pragma unroll
-      for (int i = 0; i < TM; ++i) {
-        fma_pair(a[i], bb[0], bb[1], acc[i][0]);
-        fma_pair(a[i], bb[2], bb[3], acc[i][1]);
-      }
-    }
-    __syncthreads();  // the buffer is refilled two chunks later
-  }
-  const T scale = T(p.scale[t.b]);
-  const int OS = COLS + 1;
-  T* ot = smem;  // [ROWS][COLS + 1], aliases the stages (all reads are behind the barrier above)
-#pragma unroll
-  for (int i = 0; i < TM; ++i)
-#pragma unroll
-    for (int j = 0; j < 2; ++j) {
-      ot[(tr * TM + i) * OS + tc * 4 + 2 * j] = acc[i][j].x * scale;
-      ot[(tr * TM + i) * OS + tc * 4 + 2 * j + 1] = acc[i][j].y * scale;
-    }
-  __syncthreads();
-  // coalesced write: per node the (w, m) range is contiguous
-  const int span = t.ncols * d;
-  for (int j = warp; j < t.tn; j += 8) {
-    T* dst = OUT + (size_t)s_nodes[j] * p.out_dim + p.out_off[t.b] + t.c0 * d;
-    const T* src = ot + j * d * OS;
-    for (int q = lane; q < span; q += 32) {
-      const T v = src[omap[q]];
-      dst[q] = p.accumulate ? (dst[q] + v) : v;
-    }
-  }
-}
-
-template <typename T>
-__global__ void __launch_bounds__(256, 2) linear_fwd_kernel(const LinParams p) {
-  extern __shared__ __align__(16) unsigned char lin_smem[];
-  __shared__ int s_nodes[kLinMaxRows];
-  __shared__ int s_qmap[32 * kLinMaxDim];  // q -> (q / d) * XS + q % d        (x staging, q < KC * d)
-  __shared__ int s_omap[64 * kLinMaxDim];  // q -> (q % d) * (COLS + 1) + q / d (output, q < ncols * d)
-
-  // which block / node tile / column chunk am I?
-  int b = 0;
-  while (b + 1 < p.num_blocks && (int)blockIdx.x >= p.cta_begin[b + 1]) ++b;
-  int local = blockIdx.x - p.cta_begin[b];
-  const int cc = local % p.col_chunks[b];
-  int tile = local / p.col_chunks[b];
-  const int TN = p.nodes_per_tile[b];
-  LinTile t;
-  t.b = b;
-  t.mi = p.mul_in[b]; t.mo = p.mul_out[b]; t.d = p.dim[b];
-  t.COLS = p.tile_cols[b];
-  t.lc = 31 - __clz(t.COLS);
-  const int TM = t.COLS >= 16 ? 8 : 4;
-  t.ROWS = (256 / (t.COLS >> 2)) * TM;
-  t.KC = kLinStage / t.ROWS;
-  t.XS = t.ROWS + 4;  // row stride of the transposed x stage
-  // locate (species, tile-in-species)
-  int s = 0;
-  int64_t begin = 0, end = 0;
-  if (p.S == 1 && p.sptr == nullptr) {
-    begin = (int64_t)tile * TN;
-    end = imin64(begin + TN, p.N);
-    if (begin >= p.N) return;
-  } else {
-    bool found = false;
-    for (s = 0; s < p.S; ++s) {
-      int cnt = p.sptr[s + 1] - p.sptr[s];
-      int nt = (cnt + TN - 1) / TN;
-      if (tile < nt) {
-        begin = p.sptr[s] + (int64_t)tile * TN;
-        end = imin64(begin + TN, (int64_t)p.sptr[s + 1]);
-        found = true;
-        break;
-      }
-      tile -= nt;
-    }
-    if (!found) return;
-  }
-  t.s = s;
-  t.tn = (int)(end - begin);
-  t.c0 = cc * t.COLS;
-  t.ncols = min(t.COLS, t.mo - t.c0);
-  const int tid = threadIdx.x;
-  const int d = t.d;
-  for (int i = tid; i < t.tn; i += blockDim.x) s_nodes[i] = p.sperm ? p.sperm[begin + i] : (int)(begin + i);
-  for (int q = tid; q < t.KC * d; q += blockDim.x) s_qmap[q] = (q / d) * t.XS + q % d;
-  for (int q = tid; q < t.ncols * d; q += blockDim.x) s_omap[q] = (q % d) * (t.COLS + 1) + q / d;
-  __syncthreads();
-
-  if (t.mi == 0) {  // irreps with no incoming path: zeros
-    if (!p.accumulate) {
-      T* __restrict__ OUT = static_cast<T*>(p.out);
-      const int span = t.ncols * d;
-      for (int j = tid >> 5; j < t.tn; j += 8)
-        for (int q = tid & 31; q < span; q += 32)
-          OUT[(size_t)s_nodes[j] * p.out_dim + p.out_off[b] + t.c0 * d + q] = T(0);
-    }
-    return;
-  }
-  T* smem = reinterpret_cast<T*>(lin_smem);
-  if (TM == 8) lin_tile_run<T, 8>(p, t, smem, s_nodes, s_qmap, s_omap);
-  else lin_tile_run<T, 4>(p, t, smem, s_nodes, s_qmap, s_omap);
-}
-
-// =========================================================================
-// Node-streaming linear: one CTA owns a tile of nodes of ONE species and walks ALL irrep blocks over it.
-//   * the species' weight slices of every block sit in shared memory for the CTA's lifetime;
-//   * each block's input columns of the tile's rows arrive by cp.async (16 B per lane, coalesced along the row), one
-//     block ahead of the arithmetic, so x is read from HBM exactly once and never passes through registers;
-//   * lanes <-> output channels w, NB nodes per lane in registers: per 4 input channels a lane issues 4 LDS.32 of
-//     weights (conflict free), NB x D LDS.128 of x (warp-wide broadcast) and NB x 4 x D FMAs.
-// The tiled kernel above spends 152 k thread instructions per node on lin2 of the last layer for 14.8 k MACs (rows
-// of 1392 floats cut into 80-byte slivers per k-chunk, every chunk paying the DRAM latency): ncu r2_step_full.
-// =========================================================================
-constexpr int kStreamSmemBytes = 200 * 1024;
-
 struct LinStream {
   int tnode;                        // nodes per CTA tile
   int rs;                           // row stride (elements) of the staged x rows: max over blocks, multiple of 4, + 4
@@ -269,65 +87,147 @@ struct LinStream {
   int tiles_per_cta;                // consecutive tiles of one species per CTA (weights staged once for all of them)
 };
 
+// Each species' nodes are cut into tiles of `super` nodes, numbered species after species; CTA blockIdx.x takes one.
+// false: a spare CTA (the grid counts a partial tile for every species).
+__device__ __forceinline__ bool lin_locate(const LinParams& p, int super, int& s, int64_t& begin, int64_t& end) {
+  int tile = blockIdx.x;
+  s = 0;
+  if (p.S == 1 && p.sptr == nullptr) {
+    begin = (int64_t)tile * super;
+    end = imin64(begin + super, p.N);
+    return begin < p.N;
+  }
+  for (s = 0; s < p.S; ++s) {
+    const int cnt = p.sptr[s + 1] - p.sptr[s];
+    const int nt = (cnt + super - 1) / super;
+    if (tile < nt) {
+      begin = p.sptr[s] + (int64_t)tile * super;
+      end = imin64(begin + super, (int64_t)p.sptr[s + 1]);
+      return true;
+    }
+    tile -= nt;
+  }
+  return false;
+}
+
+// Species s's weight slices into shared memory, [mi4][mo] per block (rows mi..mi4 zero); asynchronous copies, all in
+// flight at once, for the caller to commit as one group.  Rows of mo contiguous elements: 16 bytes per copy when mo
+// allows.
+template <typename T>
+__device__ __forceinline__ void lin_stage_weights(const LinParams& p, const LinStream& e, T* wsm, int s) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const T* __restrict__ W = static_cast<const T*>(p.weight);
+  constexpr int V = 16 / (int)sizeof(T);  // elements per 16-byte copy
+  for (int b = 0; b < p.num_blocks; ++b) {
+    const int mi = p.mul_in[b], mo = p.mul_out[b], ld = p.ld[b], mi4 = (mi + 3) & ~3;
+    T* dst = wsm + e.w_smem_off[b];
+    if (!p.transpose && e.w_vec[b]) {
+      const int rowv = mo / V;  // vectors per row
+      const int nvec = mi4 * rowv;
+      int u = tid / rowv, c = tid - u * rowv;          // one division per thread and block; then additive
+      const int du = 256 / rowv, dc = 256 - du * rowv;
+      for (int v = tid; v < nvec; v += 256) {
+        const bool ok = u < mi;
+        const T* src = W + (ok ? (size_t)p.w_off[b] + ((size_t)u * p.S + s) * ld + c * V : 0);
+        const uint32_t da = (uint32_t)__cvta_generic_to_shared(dst + u * mo + c * V);
+        asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(da), "l"(src), "r"(ok ? 16 : 0) : "memory");
+        u += du; c += dc;
+        if (c >= rowv) { c -= rowv; ++u; }
+      }
+    } else {
+      for (int u = warp; u < mi4; u += 8)
+        for (int w = lane; w < mo; w += 32) {
+          const bool ok = u < mi;
+          const size_t off = !ok ? 0
+                             : p.transpose ? (size_t)p.w_off[b] + ((size_t)w * p.S + s) * ld + u
+                                           : (size_t)p.w_off[b] + ((size_t)u * p.S + s) * ld + w;
+          lin_cp_async<T>(dst + u * mo + w, W + off, ok);
+        }
+    }
+  }
+}
+
+// One staged x row: the seg elements at src, then zeros up to segp (the padded length the arithmetic reads).  16 bytes
+// per copy when the row is aligned (vec), else one element per copy.
+template <typename T>
+__device__ __forceinline__ void lin_stage_row(T* dst, const T* src, int seg, int segp, bool vec, int lane) {
+  constexpr int V = 16 / (int)sizeof(T);  // elements per 16-byte copy
+  if (vec) {
+    const uint32_t drow = (uint32_t)__cvta_generic_to_shared(dst);
+    for (int q = lane * V; q < segp; q += 32 * V) {
+      const int n = min(V, seg - q);  // elements really there
+      asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(drow + q * (int)sizeof(T)),
+                   "l"(src + (n > 0 ? q : 0)), "r"(n > 0 ? n * (int)sizeof(T) : 0)
+                   : "memory");
+    }
+  } else {
+    for (int q = lane; q < segp; q += 32) lin_cp_async<T>(dst + q, src + (q < seg ? q : 0), q < seg);
+  }
+}
+
+// lanes per output channel group: the smallest of 32/16/8/4 covering mul_out (32 when mul_out > 16)
+__device__ __forceinline__ int lin_lpn(int mo) {
+  int lpn = 32;
+  while (lpn > 4 && (lpn >> 1) >= mo) lpn >>= 1;
+  return lpn;
+}
+
+// One block for the output channels w0 .. w0 + lpn - 1 (lpn = lin_lpn(mo)) of NB nodes whose staged rows are
+// xs + nb * RS, of which the first ncount are stored:
+//   out[nodes[nb], out_off + w * D + m] (+)= scale * sum_u ws[u][w] * xs[nb][u * D + m].
 // Lanes of a warp = (output channel w: lpn lanes) x (k-split ks: 32 / lpn lanes): every warp works on NB nodes
 // whatever mul_out is; narrow outputs (mul_out 16 or 4 for l >= 1) split the input channels over the spare lanes and
-// reduce with shuffles at the end.
+// reduce with shuffles at the end.  The loops over w0 and over node groups stay in the kernels: the CTA-synchronous
+// kernel runs node groups inside the w0 loop, and ptxas gives it fewer registers in that order.
 template <typename T, int D, int NB>
-__device__ __forceinline__ void lin_stream_block(const T* __restrict__ ws, const T* __restrict__ xs, int RS, int mi4,
-                                                 int mo, int tn, const int* __restrict__ s_nodes,
-                                                 T* __restrict__ OUT, int out_dim, int out_off, T scale,
-                                                 int accumulate) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  int lpn = 32;  // lanes per channel group: the smallest of 32/16/8/4 covering mul_out (32 when mul_out > 16)
-  while (lpn > 4 && (lpn >> 1) >= mo) lpn >>= 1;
+__device__ __forceinline__ void lin_block(const T* __restrict__ ws, const T* __restrict__ xs, int RS, int mi4, int mo,
+                                          int lpn, int w0, int ncount, const int* __restrict__ nodes,
+                                          T* __restrict__ OUT, int out_dim, int out_off, T scale, int accumulate) {
+  const int lane = threadIdx.x & 31;
   const int subs = 32 / lpn, ks = lane / lpn, wl = lane - ks * lpn;
   const int ustep = 4 * subs;
-  for (int w0 = 0; w0 < mo; w0 += lpn) {
-    const int w = w0 + wl;
-    const bool wok = w < mo;
-    for (int n0 = warp * NB; n0 < tn; n0 += 8 * NB) {
-      T acc[NB][D];
-      const T* xq[NB];
+  const int w = w0 + wl;
+  const bool wok = w < mo;
+  T acc[NB][D];
+  const T* xq[NB];
 #pragma unroll
-      for (int nb = 0; nb < NB; ++nb) {
+  for (int nb = 0; nb < NB; ++nb) {
 #pragma unroll
-        for (int m = 0; m < D; ++m) acc[nb][m] = T(0);
-        // rows past the tile repeat the last one; never stored
-        xq[nb] = xs + (size_t)min(n0 + nb, tn - 1) * RS + ks * 4 * D;
-      }
-      const T* wq = ws + (wok ? w : 0) + ks * 4 * mo;
-      for (int u = ks * 4; u < mi4; u += ustep) {
-        T wv[4];
+    for (int m = 0; m < D; ++m) acc[nb][m] = T(0);
+    // rows past ncount repeat the last one; never stored
+    xq[nb] = xs + (size_t)min(nb, ncount - 1) * RS + ks * 4 * D;
+  }
+  const T* wq = ws + (wok ? w : 0) + ks * 4 * mo;
+  for (int u = ks * 4; u < mi4; u += ustep) {
+    T wv[4];
 #pragma unroll
-        for (int k = 0; k < 4; ++k) wv[k] = wq[k * mo];
-        wq += ustep * mo;
+    for (int k = 0; k < 4; ++k) wv[k] = wq[k * mo];
+    wq += ustep * mo;
 #pragma unroll
-        for (int nb = 0; nb < NB; ++nb) {
-          T xv[4 * D];
+    for (int nb = 0; nb < NB; ++nb) {
+      T xv[4 * D];
 #pragma unroll
-          for (int i = 0; i < D; ++i) lin_ld4<T>(xq[nb] + 4 * i, *reinterpret_cast<T(*)[4]>(&xv[4 * i]));
-          xq[nb] += ustep * D;
+      for (int i = 0; i < D; ++i) lin_ld4<T>(xq[nb] + 4 * i, *reinterpret_cast<T(*)[4]>(&xv[4 * i]));
+      xq[nb] += ustep * D;
 #pragma unroll
-          for (int k = 0; k < 4; ++k)
+      for (int k = 0; k < 4; ++k)
 #pragma unroll
-            for (int m = 0; m < D; ++m) acc[nb][m] = fma(wv[k], xv[k * D + m], acc[nb][m]);
-        }
-      }
-      for (int off = lpn; off < 32; off <<= 1) {  // sum the k-splits (fixed order: deterministic)
+        for (int m = 0; m < D; ++m) acc[nb][m] = fma(wv[k], xv[k * D + m], acc[nb][m]);
+    }
+  }
+  for (int off = lpn; off < 32; off <<= 1) {  // sum the k-splits (fixed order: deterministic)
 #pragma unroll
-        for (int nb = 0; nb < NB; ++nb)
+    for (int nb = 0; nb < NB; ++nb)
 #pragma unroll
-          for (int m = 0; m < D; ++m) acc[nb][m] += __shfl_xor_sync(0xffffffffu, acc[nb][m], off);
-      }
-      if (wok && ks == 0) {
+      for (int m = 0; m < D; ++m) acc[nb][m] += __shfl_xor_sync(0xffffffffu, acc[nb][m], off);
+  }
+  if (wok && ks == 0) {
 #pragma unroll
-        for (int nb = 0; nb < NB; ++nb) {
-          if (n0 + nb < tn) {
-            T* dst = OUT + (size_t)s_nodes[n0 + nb] * out_dim + out_off + w * D;
+    for (int nb = 0; nb < NB; ++nb) {
+      if (nb < ncount) {
+        T* dst = OUT + (size_t)nodes[nb] * out_dim + out_off + w * D;
 #pragma unroll
-            for (int m = 0; m < D; ++m) dst[m] = accumulate ? (dst[m] + acc[nb][m] * scale) : acc[nb][m] * scale;
-          }
-        }
+        for (int m = 0; m < D; ++m) dst[m] = accumulate ? (dst[m] + acc[nb][m] * scale) : acc[nb][m] * scale;
       }
     }
   }
@@ -344,92 +244,29 @@ __global__ void __launch_bounds__(256) linear_sync_kernel(const LinParams p, con
   T* wsm = reinterpret_cast<T*>(lin_smem);
   T* xbuf = wsm + ((e.w_total + 3) & ~3);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int super = e.tnode * e.tiles_per_cta;
-  // locate (species, super-tile-in-species)
-  int tile = blockIdx.x, s = 0;
-  int64_t begin = 0, end = 0;
-  if (p.S == 1 && p.sptr == nullptr) {
-    begin = (int64_t)tile * super;
-    end = imin64(begin + super, p.N);
-    if (begin >= p.N) return;
-  } else {
-    bool found = false;
-    for (s = 0; s < p.S; ++s) {
-      const int cnt = p.sptr[s + 1] - p.sptr[s];
-      const int nt = (cnt + super - 1) / super;
-      if (tile < nt) {
-        begin = p.sptr[s] + (int64_t)tile * super;
-        end = imin64(begin + super, (int64_t)p.sptr[s + 1]);
-        found = true;
-        break;
-      }
-      tile -= nt;
-    }
-    if (!found) return;
-  }
+  int s;
+  int64_t begin, end;
+  if (!lin_locate(p, e.tnode * e.tiles_per_cta, s, begin, end)) return;
   const int tn_all = (int)(end - begin);
   const int ntiles = (tn_all + e.tnode - 1) / e.tnode;
   for (int i = tid; i < tn_all; i += 256) s_nodes[i] = p.sperm ? p.sperm[begin + i] : (int)(begin + i);
   const T* __restrict__ X = static_cast<const T*>(p.x);
-  const T* __restrict__ W = static_cast<const T*>(p.weight);
   T* __restrict__ OUT = static_cast<T*>(p.out);
-  constexpr int V = 16 / (int)sizeof(T);  // elements per 16-byte copy
-  // this species' weight slices, [mi4][mo] per block (rows mi..mi4 zero); asynchronous copies, all in flight at once
-  // (the first group the pipeline below waits for).  Rows of mo contiguous elements: 16 bytes per copy when mo allows.
-  for (int b = 0; b < p.num_blocks; ++b) {
-    const int mi = p.mul_in[b], mo = p.mul_out[b], mi4 = (mi + 3) & ~3;
-    T* dst = wsm + e.w_smem_off[b];
-    if (!p.transpose && e.w_vec[b]) {
-      const int rowv = mo / V;  // vectors per row
-      const int nvec = mi4 * rowv;
-      int u = tid / rowv, c = tid - u * rowv;          // one division per thread and block; then additive
-      const int du = 256 / rowv, dc = 256 - du * rowv;
-      for (int v = tid; v < nvec; v += 256) {
-        const bool ok = u < mi;
-        const T* src = W + (ok ? (size_t)p.w_off[b] + ((size_t)u * p.S + s) * mo + c * V : 0);
-        const uint32_t da = (uint32_t)__cvta_generic_to_shared(dst + u * mo + c * V);
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(da), "l"(src), "r"(ok ? 16 : 0) : "memory");
-        u += du; c += dc;
-        if (c >= rowv) { c -= rowv; ++u; }
-      }
-    } else {
-      for (int u = warp; u < mi4; u += 8)
-        for (int w = lane; w < mo; w += 32) {
-          const bool ok = u < mi;
-          const size_t off = !ok ? 0
-                             : p.transpose ? (size_t)p.w_off[b] + ((size_t)w * p.S + s) * mi + u
-                                           : (size_t)p.w_off[b] + ((size_t)u * p.S + s) * mo + w;
-          lin_cp_async<T>(dst + u * mo + w, W + off, ok);
-        }
-    }
-  }
+  lin_stage_weights<T>(p, e, wsm, s);  // the first group the pipeline below waits for
   lin_cp_commit();
   __syncthreads();  // s_nodes
   const int nb_ = p.num_blocks;
   const int nsteps = ntiles * nb_;
-  const uint32_t xbuf_s = (uint32_t)__cvta_generic_to_shared(xbuf);
   auto issue = [&](int step) {
     const int t = step / nb_, b = step - t * nb_;
     const int mi = p.mul_in[b], d = p.dim[b];
     const int seg = mi * d, segp = (((mi + 3) & ~3) * d + 3) & ~3;  // copied + zero-filled up to the padded length
     const int n0 = t * e.tnode, tn = min(e.tnode, tn_all - n0);
-    const uint32_t buf_s = xbuf_s + (uint32_t)((step & 1) * e.tnode * e.rs * (int)sizeof(T));
+    T* buf = xbuf + (size_t)(step & 1) * e.tnode * e.rs;
     if (mi > 0) {
-      for (int j = warp; j < tn; j += 8) {
-        const T* src = X + (size_t)s_nodes[n0 + j] * p.in_dim + p.in_off[b];
-        const uint32_t drow = buf_s + (uint32_t)(j * e.rs * (int)sizeof(T));
-        if (e.vec_ok[b]) {
-          for (int q = lane * V; q < segp; q += 32 * V) {
-            const int n = min(V, seg - q);  // elements really there
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(drow + q * (int)sizeof(T)),
-                         "l"(src + (n > 0 ? q : 0)), "r"(n > 0 ? n * (int)sizeof(T) : 0)
-                         : "memory");
-          }
-        } else {
-          T* dst = xbuf + (size_t)(step & 1) * e.tnode * e.rs + (size_t)j * e.rs;
-          for (int q = lane; q < segp; q += 32) lin_cp_async<T>(dst + q, src + (q < seg ? q : 0), q < seg);
-        }
-      }
+      for (int j = warp; j < tn; j += 8)
+        lin_stage_row<T>(buf + (size_t)j * e.rs, X + (size_t)s_nodes[n0 + j] * p.in_dim + p.in_off[b], seg, segp,
+                         e.vec_ok[b], lane);
     }
     lin_cp_commit();
   };
@@ -458,8 +295,11 @@ __global__ void __launch_bounds__(256) linear_sync_kernel(const LinParams p, con
       const int mi4 = (mi + 3) & ~3;
       const T sc = T(p.scale[b]);
       // nodes per lane: 8 warps x NB covers the tile (NB = 4 for 32-node tiles, 2 for 16-node tiles), fewer for wide irreps
-#define MT_LIN_BLOCK(DD, NBB) \
-  lin_stream_block<T, DD, NBB>(ws, xs, e.rs, mi4, mo, tn, nodes, OUT, p.out_dim, p.out_off[b], sc, p.accumulate)
+#define MT_LIN_BLOCK(DD, NBB)                                                                              \
+  for (int w0 = 0, lpn = lin_lpn(mo); w0 < mo; w0 += lpn)                                                  \
+    for (int n0 = warp * NBB; n0 < tn; n0 += 8 * NBB)                                                      \
+      lin_block<T, DD, NBB>(ws, xs + (size_t)n0 * e.rs, e.rs, mi4, mo, lpn, w0, tn - n0, nodes + n0, OUT,    \
+                            p.out_dim, p.out_off[b], sc, p.accumulate)
       if (e.tnode > 16) {
         switch (d) {
           case 1: MT_LIN_BLOCK(1, 4); break;
@@ -490,127 +330,20 @@ __global__ void __launch_bounds__(256) linear_sync_kernel(const LinParams p, con
 constexpr int kWarpNB = 2;       // nodes per warp and step
 constexpr int kWarpGroupsMax = 4;  // node groups per warp: a CTA covers 8 x kWarpNB x groups nodes of one species
 
-template <typename T, int D, int NB>
-__device__ __forceinline__ void lin_warp_block(const T* __restrict__ ws, const T* __restrict__ xs, int RS, int mi4,
-                                               int mo, int ncount, const int* __restrict__ nodes,
-                                               T* __restrict__ OUT, int out_dim, int out_off, T scale, int accumulate) {
-  const int lane = threadIdx.x & 31;
-  int lpn = 32;  // lanes per channel group: the smallest of 32/16/8/4 covering mul_out (32 when mul_out > 16)
-  while (lpn > 4 && (lpn >> 1) >= mo) lpn >>= 1;
-  const int subs = 32 / lpn, ks = lane / lpn, wl = lane - ks * lpn;
-  const int ustep = 4 * subs;
-  for (int w0 = 0; w0 < mo; w0 += lpn) {
-    const int w = w0 + wl;
-    const bool wok = w < mo;
-    T acc[NB][D];
-    const T* xq[NB];
-#pragma unroll
-    for (int nb = 0; nb < NB; ++nb) {
-#pragma unroll
-      for (int m = 0; m < D; ++m) acc[nb][m] = T(0);
-      xq[nb] = xs + (size_t)nb * RS + ks * 4 * D;  // rows past ncount hold stale finite data; never stored
-    }
-    const T* wq = ws + (wok ? w : 0) + ks * 4 * mo;
-    for (int u = ks * 4; u < mi4; u += ustep) {
-      T wv[4];
-#pragma unroll
-      for (int k = 0; k < 4; ++k) wv[k] = wq[k * mo];
-      wq += ustep * mo;
-#pragma unroll
-      for (int nb = 0; nb < NB; ++nb) {
-        T xv[4 * D];
-#pragma unroll
-        for (int i = 0; i < D; ++i) lin_ld4<T>(xq[nb] + 4 * i, *reinterpret_cast<T(*)[4]>(&xv[4 * i]));
-        xq[nb] += ustep * D;
-#pragma unroll
-        for (int k = 0; k < 4; ++k)
-#pragma unroll
-          for (int m = 0; m < D; ++m) acc[nb][m] = fma(wv[k], xv[k * D + m], acc[nb][m]);
-      }
-    }
-    for (int off = lpn; off < 32; off <<= 1) {  // sum the k-splits (fixed order: deterministic)
-#pragma unroll
-      for (int nb = 0; nb < NB; ++nb)
-#pragma unroll
-        for (int m = 0; m < D; ++m) acc[nb][m] += __shfl_xor_sync(0xffffffffu, acc[nb][m], off);
-    }
-    if (wok && ks == 0) {
-#pragma unroll
-      for (int nb = 0; nb < NB; ++nb) {
-        if (nb < ncount) {
-          T* dst = OUT + (size_t)nodes[nb] * out_dim + out_off + w * D;
-#pragma unroll
-          for (int m = 0; m < D; ++m) dst[m] = accumulate ? (dst[m] + acc[nb][m] * scale) : acc[nb][m] * scale;
-        }
-      }
-    }
-  }
-}
-
 template <typename T>
 __global__ void __launch_bounds__(256) linear_stream_kernel(const LinParams p, const LinStream e) {
   extern __shared__ __align__(16) unsigned char lin_smem[];
   __shared__ int s_nodes[8 * kWarpNB * kWarpGroupsMax];
   T* wsm = reinterpret_cast<T*>(lin_smem);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int super = e.tnode;  // 8 warps x kWarpNB x groups
-  // locate (species, tile-in-species)
-  int tile = blockIdx.x, s = 0;
-  int64_t begin = 0, end = 0;
-  if (p.S == 1 && p.sptr == nullptr) {
-    begin = (int64_t)tile * super;
-    end = imin64(begin + super, p.N);
-    if (begin >= p.N) return;
-  } else {
-    bool found = false;
-    for (s = 0; s < p.S; ++s) {
-      const int cnt = p.sptr[s + 1] - p.sptr[s];
-      const int nt = (cnt + super - 1) / super;
-      if (tile < nt) {
-        begin = p.sptr[s] + (int64_t)tile * super;
-        end = imin64(begin + super, (int64_t)p.sptr[s + 1]);
-        found = true;
-        break;
-      }
-      tile -= nt;
-    }
-    if (!found) return;
-  }
+  int s;
+  int64_t begin, end;
+  if (!lin_locate(p, e.tnode, s, begin, end)) return;  // tnode = 8 warps x kWarpNB x groups
   const int tn_all = (int)(end - begin);
   for (int i = tid; i < tn_all; i += 256) s_nodes[i] = p.sperm ? p.sperm[begin + i] : (int)(begin + i);
   const T* __restrict__ X = static_cast<const T*>(p.x);
-  const T* __restrict__ W = static_cast<const T*>(p.weight);
   T* __restrict__ OUT = static_cast<T*>(p.out);
-  constexpr int V = 16 / (int)sizeof(T);  // elements per 16-byte copy
-  // this species' weight slices, [mi4][mo] per block (rows mi..mi4 zero); asynchronous copies, all in flight at once.
-  // Rows of mo contiguous elements: 16 bytes per copy when mo allows.
-  for (int b = 0; b < p.num_blocks; ++b) {
-    const int mi = p.mul_in[b], mo = p.mul_out[b], mi4 = (mi + 3) & ~3;
-    T* dst = wsm + e.w_smem_off[b];
-    if (!p.transpose && e.w_vec[b]) {
-      const int rowv = mo / V;  // vectors per row
-      const int nvec = mi4 * rowv;
-      int u = tid / rowv, c = tid - u * rowv;          // one division per thread and block; then additive
-      const int du = 256 / rowv, dc = 256 - du * rowv;
-      for (int v = tid; v < nvec; v += 256) {
-        const bool ok = u < mi;
-        const T* src = W + (ok ? (size_t)p.w_off[b] + ((size_t)u * p.S + s) * mo + c * V : 0);
-        const uint32_t da = (uint32_t)__cvta_generic_to_shared(dst + u * mo + c * V);
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(da), "l"(src), "r"(ok ? 16 : 0) : "memory");
-        u += du; c += dc;
-        if (c >= rowv) { c -= rowv; ++u; }
-      }
-    } else {
-      for (int u = warp; u < mi4; u += 8)
-        for (int w = lane; w < mo; w += 32) {
-          const bool ok = u < mi;
-          const size_t off = !ok ? 0
-                             : p.transpose ? (size_t)p.w_off[b] + ((size_t)w * p.S + s) * mi + u
-                                           : (size_t)p.w_off[b] + ((size_t)u * p.S + s) * mo + w;
-          lin_cp_async<T>(dst + u * mo + w, W + off, ok);
-        }
-    }
-  }
+  lin_stage_weights<T>(p, e, wsm, s);
   lin_cp_commit();
   lin_cp_wait<0>();
   __syncthreads();  // weights and s_nodes in place: the only CTA-wide barrier
@@ -625,37 +358,22 @@ __global__ void __launch_bounds__(256) linear_stream_kernel(const LinParams p, c
   if (mygroups == 0) return;
   const int nsteps = mygroups * nb_;
   T* xw = wsm + ((e.w_total + 3) & ~3) + (size_t)warp * 2 * kWarpNB * e.rs;  // [2][kWarpNB][rs]
-  const uint32_t xw_s = (uint32_t)__cvta_generic_to_shared(xw);
   auto issue = [&](int step) {
     const int g = step / nb_, b = step - g * nb_;
     const int mi = p.mul_in[b], d = p.dim[b];
     const int seg = mi * d, segp = (((mi + 3) & ~3) * d + 3) & ~3;  // copied + zero-filled up to the padded length
     const int n0 = (g * 8 + warp) * kWarpNB;
-    const uint32_t buf_s = xw_s + (uint32_t)((step & 1) * kWarpNB * e.rs * (int)sizeof(T));
+    T* buf = xw + (size_t)(step & 1) * kWarpNB * e.rs;
     if (mi > 0) {
 #pragma unroll
       for (int nb = 0; nb < kWarpNB; ++nb) {
         if (n0 + nb >= tn_all) break;
-        const T* src = X + (size_t)s_nodes[n0 + nb] * p.in_dim + p.in_off[b];
-        const uint32_t drow = buf_s + (uint32_t)(nb * e.rs * (int)sizeof(T));
-        if (e.vec_ok[b]) {
-          for (int q = lane * V; q < segp; q += 32 * V) {
-            const int n = min(V, seg - q);  // elements really there
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(drow + q * (int)sizeof(T)),
-                         "l"(src + (n > 0 ? q : 0)), "r"(n > 0 ? n * (int)sizeof(T) : 0)
-                         : "memory");
-          }
-        } else {
-          T* dst = xw + (size_t)(step & 1) * kWarpNB * e.rs + (size_t)nb * e.rs;
-          for (int q = lane; q < segp; q += 32) lin_cp_async<T>(dst + q, src + (q < seg ? q : 0), q < seg);
-        }
+        lin_stage_row<T>(buf + (size_t)nb * e.rs, X + (size_t)s_nodes[n0 + nb] * p.in_dim + p.in_off[b], seg, segp,
+                         e.vec_ok[b], lane);
       }
     }
     lin_cp_commit();
   };
-  // rows of a partial last group are never copied: make them finite once (they are multiplied, never stored)
-  for (int i = lane; i < 2 * kWarpNB * e.rs; i += 32) xw[i] = T(0);
-  __syncwarp();
   issue(0);
   for (int step = 0; step < nsteps; ++step) {
     if (step + 1 < nsteps) {
@@ -681,8 +399,10 @@ __global__ void __launch_bounds__(256) linear_stream_kernel(const LinParams p, c
       const T* ws = wsm + e.w_smem_off[b];
       const int mi4 = (mi + 3) & ~3;
       const T sc = T(p.scale[b]);
-#define MT_LIN_BLOCK(DD) \
-  lin_warp_block<T, DD, kWarpNB>(ws, xs, e.rs, mi4, mo, ncount, nodes, OUT, p.out_dim, p.out_off[b], sc, p.accumulate)
+#define MT_LIN_BLOCK(DD)                                                                                   \
+  for (int w0 = 0, lpn = lin_lpn(mo); w0 < mo; w0 += lpn)                                                  \
+    lin_block<T, DD, kWarpNB>(ws, xs, e.rs, mi4, mo, lpn, w0, ncount, nodes, OUT, p.out_dim, p.out_off[b], sc, \
+                              p.accumulate)
       switch (d) {
         case 1: MT_LIN_BLOCK(1); break;
         case 3: MT_LIN_BLOCK(3); break;
@@ -748,201 +468,211 @@ __global__ void __launch_bounds__(256) segment_reduce_kernel(const T* __restrict
   out[t] = acc;
 }
 
-}  // namespace mt
+// ------------------------------------------------------------------ linear: host side
+// A block, or a rectangle of one, in the orientation the kernels apply it (transposed: in and out swapped).
+struct LinPiece {
+  int in_off, out_off, mul_in, mul_out, dim, w_off, ld;
+  double scale;
+  int round;  // pieces with the same out_off before this one (linear_apply)
+};
 
-using namespace mt;
+// Appends piece k as block b of a launch: its [mi4][mo] weight slice after the others, its staged rows within the
+// row stride.
+static void lin_layout_add(LinStream& e, int b, const LinPiece& k) {
+  const int mi4 = (k.mul_in + 3) & ~3;
+  e.w_smem_off[b] = e.w_total;
+  e.w_total += mi4 * k.mul_out;
+  e.w_total = (e.w_total + 3) & ~3;
+  const int rs = ((mi4 * k.dim + 3) & ~3) + 4;
+  if (rs > e.rs) e.rs = rs;
+}
 
-extern "C" {
+// dynamic shared memory of a launch that stages `rows` x rows next to its weight slices
+static size_t lin_need(const LinStream& e, int rows, size_t es) {
+  return ((size_t)((e.w_total + 3) & ~3) + (size_t)rows * e.rs) * es;
+}
 
-static int linear_fwd_round(int dtype, const mt_lin_block* const* blocks, int num_blocks, int in_dim,
-                            int out_dim, int num_species, const void* x, const void* weight,
-                            const int32_t* species_perm, const int32_t* species_ptr, int accumulate, void* out,
-                            int64_t N, cudaStream_t st, int transpose = 0) {
-  LinParams p;
-  memset(&p, 0, sizeof(p));
-  p.transpose = transpose;
-  p.num_blocks = num_blocks;
-  int64_t total = 0;
-  // ---- node-streaming kernel whenever the block dims are 2l+1 <= 9 and the tile fits in shared memory
-  {
-    LinStream e;
-    memset(&e, 0, sizeof(e));
-    const size_t es = dtype == MT_F64 ? 8 : 4;
-    const int V = 16 / (int)es;
-    bool ok = true;
-    int rs = 0;
-    for (int b = 0; b < num_blocks; ++b) {
-      const mt_lin_block& k = *blocks[b];
-      p.in_off[b] = k.in_off; p.out_off[b] = k.out_off; p.mul_in[b] = k.mul_in; p.mul_out[b] = k.mul_out;
-      p.dim[b] = k.dim; p.w_off[b] = k.w_off; p.scale[b] = k.scale;
-      if (!(k.dim == 1 || k.dim == 3 || k.dim == 5 || k.dim == 7 || k.dim == 9)) ok = false;
-      const int mi4 = (k.mul_in + 3) & ~3;
-      e.w_smem_off[b] = e.w_total;
-      e.w_total += mi4 * k.mul_out;
-      e.w_total = (e.w_total + 3) & ~3;
-      const int segp = (mi4 * k.dim + 3) & ~3;
-      if (segp > rs) rs = segp;
-      e.vec_ok[b] = (k.in_off % V == 0) && (in_dim % V == 0) && ((uintptr_t)x % 16 == 0);
-      e.w_vec[b] = (k.mul_out % V == 0) && (k.w_off % V == 0) && ((uintptr_t)weight % 16 == 0) && k.mul_out / V <= 256;
+// The CTA-synchronous kernel with 8-node tiles stages 16 rows: the least shared memory of any tile, so the bound of
+// what one launch can hold.
+constexpr int kLinMinRows = 2 * 8;
+
+// Cuts a piece whose weight slice and rows fit no launch into rectangles of its [mul_in x mul_out] weight that each
+// fit one.  Input channels go in chunks of a multiple of 4, as large as fit.  Output channels are cut only when even
+// 4 input channels of all of them do not fit: that depends on mul_out and dim alone, so the blocks that write one
+// output range are cut at the same output channels and their pieces still share out_off.
+static int lin_cut(const LinPiece& k, int S, int transpose, size_t es, std::vector<LinPiece>& out) {
+  LinStream one;
+  memset(&one, 0, sizeof(one));
+  lin_layout_add(one, 0, k);
+  if (lin_need(one, kLinMinRows, es) <= (size_t)kStreamSmemBytes) {
+    out.push_back(k);
+    return MT_OK;
+  }
+  const int cap = (int)(kStreamSmemBytes / es);  // elements
+  // ku input channels (a multiple of 4) x kw output channels take ku * kw + kLinMinRows * (ku * dim + 4) elements
+  int kw = k.mul_out;
+  if (4 * kw + kLinMinRows * (4 * k.dim + 4) > cap) kw = (cap / 8) & ~3;
+  const int ku = ((cap - 4 * kLinMinRows) / (kw + kLinMinRows * k.dim)) & ~3;
+  for (int u0 = 0; u0 < k.mul_in; u0 += ku)
+    for (int w0 = 0; w0 < k.mul_out; w0 += kw) {
+      LinPiece c = k;
+      c.in_off = k.in_off + u0 * k.dim;
+      c.out_off = k.out_off + w0 * k.dim;
+      c.mul_in = std::min(ku, k.mul_in - u0);
+      c.mul_out = std::min(kw, k.mul_out - w0);
+      // the weight of (u0, w0); the piece indexes from there with the whole block's row stride
+      const int64_t w_off =
+          k.w_off + (transpose ? (int64_t)w0 * S * k.ld + u0 : (int64_t)u0 * S * k.ld + w0);
+      MT_REQUIRE(w_off < (int64_t)2147483647, "weight offset too large");
+      c.w_off = (int)w_off;
+      out.push_back(c);
     }
-    e.rs = rs + 4;
-    if (in_dim < 512) {  // short rows: CTA-synchronous tiles
-    int tnode = 32;
-      auto need = [&](int tn) { return ((size_t)((e.w_total + 3) & ~3) + 2 * (size_t)tn * e.rs) * es; };
-      // two resident CTAs per SM (16 warps, one CTA's copies under the other's arithmetic) beat one big tile
-      while (tnode > 8 && need(tnode) > (size_t)(kStreamSmemBytes / 2 - 8 * 1024)) tnode >>= 1;
-      if (ok && need(tnode) <= (size_t)kStreamSmemBytes) {
-        e.tnode = tnode;
-        p.in_dim = in_dim; p.out_dim = out_dim; p.S = num_species;
-        p.x = x; p.weight = weight; p.sperm = species_perm; p.sptr = species_ptr;
-        p.accumulate = accumulate; p.out = out; p.N = N;
-        // several tiles per CTA only when that still leaves >= 4 CTAs per SM
-        int tpc = (int)(N / ((int64_t)tnode * 4 * kNumSMs));
-        tpc = tpc < 1 ? 1 : (tpc > kStreamTiles ? kStreamTiles : tpc);
-        e.tiles_per_cta = tpc;
-        const int64_t tiles = ceil_div<int64_t>(N, (int64_t)tnode * tpc) + (species_ptr ? num_species : 0);
-        MT_REQUIRE(tiles < (int64_t)2147483647, "grid too large");
-        const size_t smem = need(tnode);
-        MT_DISPATCH_DTYPE(dtype, {
-          static thread_local bool configured = false;
-          if (!configured) {
-            MT_CUDA_OK(cudaFuncSetAttribute(linear_sync_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                            kStreamSmemBytes));
-            configured = true;
-          }
-          linear_sync_kernel<T><<<(unsigned)tiles, 256, smem, st>>>(p, e);
-        });
-        MT_LAUNCH_OK();
-        return MT_OK;
-      }
-  
-    }
+  return MT_OK;
+}
+
+// One launch of pieces pc[0..n), laid out in e: the warp-private kernel for rows of >= 512 elements when its tile
+// fits, else the CTA-synchronous kernel with the largest tile that fits.
+static int linear_launch(int dtype, LinParams p, LinStream e, const LinPiece* pc, int n, int accumulate,
+                         cudaStream_t st) {
+  const size_t es = dtype == MT_F64 ? 8 : 4;
+  const int V = 16 / (int)es;
+  p.num_blocks = n;
+  p.accumulate = accumulate;
+  for (int b = 0; b < n; ++b) {
+    const LinPiece& k = pc[b];
+    p.in_off[b] = k.in_off; p.out_off[b] = k.out_off; p.mul_in[b] = k.mul_in; p.mul_out[b] = k.mul_out;
+    p.dim[b] = k.dim; p.w_off[b] = k.w_off; p.ld[b] = k.ld; p.scale[b] = k.scale;
+    e.vec_ok[b] = (k.in_off % V == 0) && (p.in_dim % V == 0) && ((uintptr_t)p.x % 16 == 0);
+    e.w_vec[b] = (k.mul_out % V == 0) && (k.ld % V == 0) && (k.w_off % V == 0) && ((uintptr_t)p.weight % 16 == 0) &&
+                 k.mul_out / V <= 256;
+  }
+  const bool stream = p.in_dim >= 512 && lin_need(e, 8 * 2 * kWarpNB, es) <= (size_t)kStreamSmemBytes;
+  size_t smem;
+  if (stream) {
     // a CTA covers 8 warps x kWarpNB nodes x groups of one species; more groups amortise the weight staging, fewer
     // keep the grid above ~4 CTAs per SM
     int groups = kWarpGroupsMax;
-    while (groups > 1 && N / (8 * kWarpNB * groups) < 4 * kNumSMs) groups >>= 1;
-    const int tnode = 8 * kWarpNB * groups;
-    auto need = [&](int) { return ((size_t)((e.w_total + 3) & ~3) + 8 * 2 * (size_t)kWarpNB * e.rs) * es; };
-    if (ok && need(tnode) <= (size_t)kStreamSmemBytes) {
-      e.tnode = tnode;
-      p.in_dim = in_dim; p.out_dim = out_dim; p.S = num_species;
-      p.x = x; p.weight = weight; p.sperm = species_perm; p.sptr = species_ptr;
-      p.accumulate = accumulate; p.out = out; p.N = N;
-      e.tiles_per_cta = 1;
-      const int64_t tiles = ceil_div<int64_t>(N, (int64_t)tnode) + (species_ptr ? num_species : 0);
-      MT_REQUIRE(tiles < (int64_t)2147483647, "grid too large");
-      const size_t smem = need(tnode);
-      MT_DISPATCH_DTYPE(dtype, {
-        static thread_local bool configured = false;
-        if (!configured) {
-          MT_CUDA_OK(cudaFuncSetAttribute(linear_stream_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          kStreamSmemBytes));
-          configured = true;
-        }
-        linear_stream_kernel<T><<<(unsigned)tiles, 256, smem, st>>>(p, e);
-      });
-      MT_LAUNCH_OK();
-      return MT_OK;
-    }
+    while (groups > 1 && p.N / (8 * kWarpNB * groups) < 4 * kNumSMs) groups >>= 1;
+    e.tnode = 8 * kWarpNB * groups;
+    e.tiles_per_cta = 1;
+    smem = lin_need(e, 8 * 2 * kWarpNB, es);
+  } else {
+    // two resident CTAs per SM (16 warps, one CTA's copies under the other's arithmetic) beat one big tile
+    int tnode = 32;
+    while (tnode > 8 && lin_need(e, 2 * tnode, es) > (size_t)(kStreamSmemBytes / 2 - 8 * 1024)) tnode >>= 1;
+    e.tnode = tnode;
+    // several tiles per CTA only when that still leaves >= 4 CTAs per SM
+    int tpc = (int)(p.N / ((int64_t)tnode * 4 * kNumSMs));
+    e.tiles_per_cta = tpc < 1 ? 1 : (tpc > kStreamTiles ? kStreamTiles : tpc);
+    smem = lin_need(e, 2 * tnode, es);
   }
-  for (int b = 0; b < num_blocks; ++b) {
-    const mt_lin_block& k = *blocks[b];
-    p.in_off[b] = k.in_off; p.out_off[b] = k.out_off; p.mul_in[b] = k.mul_in; p.mul_out[b] = k.mul_out;
-    p.dim[b] = k.dim; p.w_off[b] = k.w_off; p.scale[b] = k.scale;
-    int cols = 64;
-    while (cols > 4 && cols / 2 >= k.mul_out) cols /= 2;  // smallest of 64/32/16/8/4 that covers mul_out (<= 64)
-    const int rows = (256 / (cols / 4)) * (cols >= 16 ? 8 : 4);
-    int tn = rows / k.dim;
-    if (tn < 1) tn = 1;
-    p.tile_cols[b] = cols;
-    p.nodes_per_tile[b] = tn;
-    p.col_chunks[b] = ceil_div<int>(k.mul_out, cols);
-    int64_t tiles = ceil_div<int64_t>(N, tn) + (species_ptr ? num_species : 0);
-    p.cta_begin[b] = (int32_t)total;
-    total += tiles * p.col_chunks[b];
-    MT_REQUIRE(total < (int64_t)2147483647, "grid too large");
-  }
-  p.cta_begin[num_blocks] = (int32_t)total;
-  p.in_dim = in_dim; p.out_dim = out_dim; p.S = num_species;
-  p.x = x; p.weight = weight; p.sperm = species_perm; p.sptr = species_ptr;
-  p.accumulate = accumulate; p.out = out; p.N = N;
+  const int64_t tiles = ceil_div<int64_t>(p.N, (int64_t)e.tnode * e.tiles_per_cta) + (p.sptr ? p.S : 0);
+  MT_REQUIRE(tiles < (int64_t)2147483647, "grid too large");
   MT_DISPATCH_DTYPE(dtype, {
-    const size_t smem = (size_t)kLinSmemElems * sizeof(T);
     static thread_local bool configured = false;
     if (!configured) {
-      MT_CUDA_OK(cudaFuncSetAttribute(linear_fwd_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      MT_CUDA_OK(cudaFuncSetAttribute(linear_sync_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      kStreamSmemBytes));
+      MT_CUDA_OK(cudaFuncSetAttribute(linear_stream_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      kStreamSmemBytes));
       configured = true;
     }
-    linear_fwd_kernel<T><<<(unsigned)total, 256, smem, st>>>(p);
+    if (stream) linear_stream_kernel<T><<<(unsigned)tiles, 256, smem, st>>>(p, e);
+    else linear_sync_kernel<T><<<(unsigned)tiles, 256, smem, st>>>(p, e);
   });
   MT_LAUNCH_OK();
   return MT_OK;
 }
 
-static int linear_check_blocks(const mt_lin_block* blocks, int num_blocks, int in_dim, int out_dim,
-                               const void* weight) {
+// Applies the blocks (transposed: with in and out swapped, blocks without weights skipped) with the shapes and
+// pointers of p.  Blocks that write the same output range (several input irreps of one type feeding one output,
+// e3nn sums them; pieces of one cut block along its input channels) must not race: round r holds the r-th piece of
+// every distinct output range, and rounds after the first accumulate.  Simplified irreps (every matten model) need
+// one round.  The pieces of a round go into as few launches as fit, in order, so the result is deterministic.
+static int linear_apply(int dtype, const mt_lin_block* blocks, int num_blocks, const LinParams& p, int accumulate,
+                        cudaStream_t st) {
+  const size_t es = dtype == MT_F64 ? 8 : 4;
+  std::vector<LinPiece> pieces;  // one allocation per call; a cut block has no fixed bound on its pieces
+  pieces.reserve(num_blocks);
   for (int b = 0; b < num_blocks; ++b) {
     const mt_lin_block& k = blocks[b];
-    MT_REQUIRE(k.dim >= 1 && k.dim <= kLinMaxDim && k.mul_out > 0 && k.mul_in >= 0, "bad linear block %d", b);
-    MT_REQUIRE(k.out_off >= 0 && k.out_off + k.mul_out * k.dim <= out_dim, "block %d exceeds out_dim", b);
-    MT_REQUIRE(k.mul_in == 0 || (k.in_off >= 0 && k.in_off + k.mul_in * k.dim <= in_dim), "block %d exceeds in_dim", b);
-    MT_REQUIRE(k.mul_in == 0 || weight != nullptr, "null weight");
-  }
-  return MT_OK;
-}
-
-// Blocks that write the same output range (several input irreps of one type feeding one output,
-// e3nn sums them) must not race: round r holds the r-th block of every distinct output range;
-// rounds after the first accumulate.  Simplified irreps (every matten model) need one round.
-static int linear_rounds(int dtype, const mt_lin_block* blocks, int num_blocks, int in_dim, int out_dim,
-                         int num_species, const void* x, const void* weight, const int32_t* species_perm,
-                         const int32_t* species_ptr, int accumulate, void* out, int64_t N, cudaStream_t st,
-                         int transpose) {
-  int round_of[4 * kLinMaxBlocks];
-  int max_round = 0;
-  for (int b = 0; b < num_blocks; ++b) {
-    int r = 0;
-    for (int c = 0; c < b; ++c)
-      if (blocks[c].out_off == blocks[b].out_off) ++r;
-    round_of[b] = r;
-    if (r > max_round) max_round = r;
-  }
-  for (int r = 0; r <= max_round; ++r) {
-    const mt_lin_block* sel[kLinMaxBlocks];
-    int n = 0;
-    for (int b = 0; b < num_blocks; ++b) {
-      if (round_of[b] != r) continue;
-      MT_REQUIRE(n < kLinMaxBlocks, "more than %d linear blocks in one round", kLinMaxBlocks);
-      sel[n++] = &blocks[b];
+    LinPiece c = {k.in_off, k.out_off, k.mul_in, k.mul_out, k.dim, k.w_off, k.mul_out, k.scale, 0};
+    if (p.transpose) {
+      if (k.mul_in == 0) continue;  // zero-fill blocks carry no gradient
+      c.in_off = k.out_off; c.out_off = k.in_off; c.mul_in = k.mul_out; c.mul_out = k.mul_in;
     }
-    int rc = linear_fwd_round(dtype, sel, n, in_dim, out_dim, num_species, x, weight, species_perm, species_ptr,
-                              (accumulate || r > 0) ? 1 : 0, out, N, st, transpose);
+    int rc = lin_cut(c, p.S, p.transpose, es, pieces);
     if (rc != MT_OK) return rc;
   }
+  int rounds = 0;
+  for (size_t i = 0; i < pieces.size(); ++i) {
+    for (size_t j = 0; j < i; ++j)
+      if (pieces[j].out_off == pieces[i].out_off) ++pieces[i].round;
+    if (pieces[i].round + 1 > rounds) rounds = pieces[i].round + 1;
+  }
+  for (int r = 0; r < rounds; ++r) {
+    const int acc = (accumulate || r > 0) ? 1 : 0;
+    LinPiece sel[kLinMaxBlocks];
+    LinStream e;
+    memset(&e, 0, sizeof(e));
+    int n = 0;
+    for (size_t i = 0; i < pieces.size(); ++i) {
+      if (pieces[i].round != r) continue;
+      LinStream grown = e;
+      lin_layout_add(grown, n, pieces[i]);
+      if (n > 0 && (n == kLinMaxBlocks || lin_need(grown, kLinMinRows, es) > (size_t)kStreamSmemBytes)) {
+        int rc = linear_launch(dtype, p, e, sel, n, acc, st);
+        if (rc != MT_OK) return rc;
+        memset(&e, 0, sizeof(e));
+        n = 0;
+        grown = e;
+        lin_layout_add(grown, n, pieces[i]);
+      }
+      e = grown;
+      sel[n++] = pieces[i];
+    }
+    if (n > 0) {
+      int rc = linear_launch(dtype, p, e, sel, n, acc, st);
+      if (rc != MT_OK) return rc;
+    }
+  }
   return MT_OK;
 }
 
-// Backward of the linear w.r.t. x: the transposed weight slices applied to grad_out (train_ops.cu).
+int linear_check_blocks(const mt_lin_block* blocks, int num_blocks, int in_dim, int out_dim, const void* weight,
+                        bool reads_weight) {
+  for (int b = 0; b < num_blocks; ++b) {
+    const mt_lin_block& k = blocks[b];
+    // 2l+1 for l <= 4: the dims the kernels are instantiated for
+    const bool dim_ok = k.dim == 1 || k.dim == 3 || k.dim == 5 || k.dim == 7 || k.dim == 9;
+    MT_REQUIRE(dim_ok && k.mul_out > 0 && k.mul_in >= 0, "bad linear block %d", b);
+    MT_REQUIRE(k.out_off >= 0 && k.out_off + k.mul_out * k.dim <= out_dim, "block %d exceeds out_dim", b);
+    MT_REQUIRE(k.mul_in == 0 || (k.in_off >= 0 && k.in_off + k.mul_in * k.dim <= in_dim), "block %d exceeds in_dim", b);
+    MT_REQUIRE(!reads_weight || k.mul_in == 0 || weight != nullptr, "null weight");
+  }
+  return MT_OK;
+}
+
 int linear_transposed(int dtype, const mt_lin_block* blocks, int num_blocks, int in_dim, int out_dim,
                       int num_species, const void* grad_out, const void* weight, const int32_t* species_perm,
                       const int32_t* species_ptr, int accumulate, void* grad_x, int64_t N, cudaStream_t st) {
-  mt_lin_block tb[4 * kLinMaxBlocks];
-  int n = 0;
-  for (int b = 0; b < num_blocks; ++b) {
-    const mt_lin_block& k = blocks[b];
-    if (k.mul_in == 0) continue;  // zero-fill blocks carry no gradient
-    tb[n] = k;
-    tb[n].in_off = k.out_off; tb[n].out_off = k.in_off; tb[n].mul_in = k.mul_out; tb[n].mul_out = k.mul_in;
-    ++n;
-  }
   if (!accumulate) {
     const size_t es = dtype == MT_F64 ? 8 : 4;
     MT_CUDA_OK(cudaMemsetAsync(grad_x, 0, (size_t)N * in_dim * es, st));
   }
-  if (n == 0) return MT_OK;
-  return linear_rounds(dtype, tb, n, out_dim, in_dim, num_species, grad_out, weight, species_perm, species_ptr, 1,
-                       grad_x, N, st, 1);
+  LinParams p;
+  memset(&p, 0, sizeof(p));
+  p.in_dim = out_dim; p.out_dim = in_dim; p.S = num_species;
+  p.x = grad_out; p.weight = weight; p.sperm = species_perm; p.sptr = species_ptr;
+  p.transpose = 1; p.out = grad_x; p.N = N;
+  return linear_apply(dtype, blocks, num_blocks, p, 1, st);
 }
+
+}  // namespace mt
+
+using namespace mt;
+
+extern "C" {
 
 int mt_linear_fwd(int dtype, const mt_lin_block* blocks, int num_blocks, int in_dim, int out_dim,
                   int num_species, const void* x, const void* weight, const int32_t* species_perm,
@@ -953,14 +683,17 @@ int mt_linear_fwd(int dtype, const mt_lin_block* blocks, int num_blocks, int in_
   MT_REQUIRE(in_dim > 0 && out_dim > 0 && num_species >= 1, "bad dims");
   MT_REQUIRE((species_perm == nullptr) == (species_ptr == nullptr), "species_perm/ptr must be given together");
   MT_REQUIRE(num_species == 1 || species_ptr != nullptr, "species grouping required when num_species > 1");
+  int rc = linear_check_blocks(blocks, num_blocks, in_dim, out_dim, weight, true);
+  if (rc != MT_OK) return rc;
   if (N == 0) return MT_OK;
   MT_REQUIRE(x && out, "null pointer");
-  int rc = linear_check_blocks(blocks, num_blocks, in_dim, out_dim, weight);
-  if (rc != MT_OK) return rc;
-  return linear_rounds(dtype, blocks, num_blocks, in_dim, out_dim, num_species, x, weight, species_perm,
-                       species_ptr, accumulate, out, N, as_stream(stream), 0);
+  LinParams p;
+  memset(&p, 0, sizeof(p));
+  p.in_dim = in_dim; p.out_dim = out_dim; p.S = num_species;
+  p.x = x; p.weight = weight; p.sperm = species_perm; p.sptr = species_ptr;
+  p.out = out; p.N = N;
+  return linear_apply(dtype, blocks, num_blocks, p, accumulate, as_stream(stream));
 }
-
 int mt_gate_fwd(int dtype, const void* x, int in_dim, int out_dim, const int32_t* src_idx,
                 const int32_t* gate_idx, const int32_t* act_id, const void* act_cst, const void* affine_a,
                 const void* affine_b, void* out, int64_t N, mt_stream stream) {

@@ -3,11 +3,6 @@
 // Everything here is deterministic: reductions are per-CTA partial sums combined in a fixed order.
 #include "common.cuh"
 
-extern "C" int linear_transposed(int dtype, const mt_lin_block* blocks, int num_blocks, int in_dim, int out_dim,
-                                 int num_species, const void* grad_out, const void* weight,
-                                 const int32_t* species_perm, const int32_t* species_ptr, int accumulate,
-                                 void* grad_x, int64_t N, cudaStream_t st);
-
 namespace mt {
 
 constexpr int kWgMaxBlocks = 64;
@@ -337,6 +332,8 @@ int mt_linear_bwd(int dtype, const mt_lin_block* blocks, int num_blocks, int in_
   MT_REQUIRE(in_dim > 0 && out_dim > 0 && num_species >= 1, "bad dims");
   MT_REQUIRE((species_perm == nullptr) == (species_ptr == nullptr), "species_perm/ptr must be given together");
   MT_REQUIRE(num_species == 1 || species_ptr != nullptr, "species grouping required when num_species > 1");
+  int rc = linear_check_blocks(blocks, num_blocks, in_dim, out_dim, weight, grad_x != nullptr);
+  if (rc != MT_OK) return rc;
   cudaStream_t st = as_stream(stream);
   const size_t es = dtype == MT_F64 ? 8 : 4;
   if (N == 0) {
@@ -345,9 +342,8 @@ int mt_linear_bwd(int dtype, const mt_lin_block* blocks, int num_blocks, int in_
   }
   MT_REQUIRE(grad_out != nullptr, "null grad_out");
   if (grad_x) {
-    MT_REQUIRE(weight != nullptr, "null weight");
-    int rc = linear_transposed(dtype, blocks, num_blocks, in_dim, out_dim, num_species, grad_out, weight, species_perm,
-                               species_ptr, accumulate_x, grad_x, N, st);
+    rc = linear_transposed(dtype, blocks, num_blocks, in_dim, out_dim, num_species, grad_out, weight, species_perm,
+                           species_ptr, accumulate_x, grad_x, N, st);
     if (rc != MT_OK) return rc;
   }
   if (grad_w) {
@@ -367,7 +363,6 @@ int mt_linear_bwd(int dtype, const mt_lin_block* blocks, int num_blocks, int in_
     for (int b = 0; b < num_blocks; ++b) {
       const mt_lin_block& k = blocks[b];
       if (k.mul_in == 0) continue;
-      MT_REQUIRE(k.dim >= 1 && k.dim <= kWgRows, "bad linear block %d", b);
       p.in_off[nb] = k.in_off; p.out_off[nb] = k.out_off; p.mul_in[nb] = k.mul_in; p.mul_out[nb] = k.mul_out;
       p.dim[nb] = k.dim; p.w_off[nb] = k.w_off;
       p.scale[nb] = k.scale;

@@ -151,6 +151,13 @@ def test_species_embed_and_kat(dev):
     # input channels), short rows (CTA-synchronous kernel) and long rows (warp-private kernel)
     ("5x0e+3x1o+1x2e", "7x0e+3x1o+2x2e", 4),
     ("131x0e+77x1o+45x2e+3x3o", "9x0e+5x1o+3x2e+1x3o", 5),
+    # in fp64 too large for one launch: the blocks of one round go into two launches (the widest linear of the
+    # reference's hyperparameters), or a dense block is cut into rectangles of its weight
+    ("64x0o+64x0e+124x1o+124x1e+148x2o+148x2e+148x3o+148x3e+124x4o+124x4e",
+     "32x0o+32x0e+16x1o+16x1e+8x2o+8x2e+4x3o+4x3e+4x4o+4x4e", 2),
+    ("600x0e+300x1o", "600x0e+300x1o", 3),
+    # in fp64 cut along output channels too, the two blocks of one output range at the same channels
+    ("8x0e+4x0e", "7000x0e", 2),
 ])
 def test_species_linear_vs_fctp(dev, dtype, irr_in, irr_out, S):
     from matten_b200 import ops
@@ -186,6 +193,58 @@ def test_species_linear_vs_fctp(dev, dtype, irr_in, irr_out, S):
 
 
 @pytest.mark.parametrize("dtype", DTYPES)
+@pytest.mark.parametrize("irr_in,irr_out,S", [
+    ("32x0e+16x1o", "32x0e+16x1o", 1),  # grad_out rows of 80 elements: CTA-synchronous kernel
+    ("32x0e+16x1o", "128x0e+96x1o+32x2e", 3),  # rows of 576: warp-private kernel
+    ("600x0e+300x1o", "600x0e+300x1o", 3),  # cut along the 600 / 300 output channels of the forward
+    ("7000x0e", "8x0e", 2),  # in fp64 cut along the 7000 input channels of the forward as well
+])
+def test_species_linear_grad_x_vs_autograd(dev, dtype, irr_in, irr_out, S):
+    """dL/dx of the species linear (its weights applied transposed) against autograd through the oracle."""
+    from matten_b200 import ops
+    from matten_b200.nn.utils import SpeciesLinear
+    from oracle import e3nn_restated as E
+
+    torch.manual_seed(3)
+    N = 777
+    lin = SpeciesLinear(irr_in, S, irr_out).to(dtype)
+    ref = E.FullyConnectedTensorProduct(irr_in, f"{S}x0e", irr_out).to(dtype)
+    ref.weight.data.copy_(lin.weight.data)
+    x = torch.randn(N, lin.irreps_in.dim, dtype=dtype)
+    g = torch.randn(N, lin.irreps_out.dim, dtype=dtype)
+    sp = torch.randint(0, S, (N,))
+    xr = x.clone().requires_grad_(True)
+    ref(xr, torch.nn.functional.one_hot(sp, S).to(dtype)).backward(g)
+    lin = lin.to(dev)
+    flag = ops.new_flag(dev)
+    ptr, perm = ops.csr_by_key(sp.to(dev), S, True, flag)
+    xd = x.to(dev).requires_grad_(True)
+    lin(xd, perm, ptr).backward(g.to(dev))
+    assert rel_err(xd.grad, xr.grad) < tol(dtype)
+
+
+@pytest.mark.parametrize("dim", [2, 11])
+def test_linear_rejects_block_dims_before_any_launch(dev, dim):
+    """Block dims other than 2l+1 <= 9 are MT_EINVAL in the forward and the backward, and nothing runs."""
+    from types import SimpleNamespace
+
+    from matten_b200 import ops
+
+    block = SimpleNamespace(in_off=0, out_off=0, mul_in=4, mul_out=4, dim=dim, w_off=0, scale=1.0)
+    h = ops.LinPlanHandle([block], 4 * dim, 4 * dim, 1, 16)
+    x = torch.randn(37, 4 * dim, device=dev)
+    w = torch.randn(16, device=dev)
+    before = ops.launch_count()
+    with pytest.raises(RuntimeError, match=r"failed \(-1\): bad linear block 0"):
+        ops.linear_fwd(h, x, w)
+    for need_x, need_w in [(True, True), (True, False), (False, True)]:
+        with pytest.raises(RuntimeError, match=r"failed \(-1\): bad linear block 0"):
+            ops.linear_bwd(h, x, w, torch.randn_like(x), need_x=need_x, need_w=need_w)
+    torch.cuda.synchronize(dev)
+    assert ops.launch_count() == before
+
+
+@pytest.mark.parametrize("dtype", DTYPES)
 def test_irreps_linear_and_cartesian(dev, dtype):
     from matten_b200.nn.readout import CartesianTensorWrapper
     from matten_b200.nn.utils import IrrepsLinear
@@ -193,7 +252,8 @@ def test_irreps_linear_and_cartesian(dev, dtype):
 
     torch.manual_seed(2)
     for a, b in [("32x0o+32x0e+16x1o+16x1e+4x2o+4x2e+2x3o+2x3e+2x4e", "16x0e+2x2e+4e"),
-                 ("16x0e+2x2e+4e", "2x0e+2x2e+4e"), ("4x0e+6x0e+3x1o", "3x0e+2x1e")]:
+                 ("16x0e+2x2e+4e", "2x0e+2x2e+4e"), ("4x0e+6x0e+3x1o", "3x0e+2x1e"),
+                 ("8x0e+4x0e", "7000x0e")]:  # cut (in fp64 along output channels too) with a shared output range
         lin = IrrepsLinear(a, b).to(dtype)
         ref = E.Linear(a, b).to(dtype)
         ref.weight.data.copy_(lin.weight.data)
