@@ -189,6 +189,26 @@ int mt_neighbor_fill(int dtype, const void* pos, const int64_t* batch, const int
                      double r_max, const int32_t* offsets, const void* workspace, int64_t* edge_index,
                      void* edge_cell_shift, void* num_neigh, int64_t E, mt_stream stream);
 
+/* The same neighbour list from a cell-list search, in time linear in the atoms of a crystal (the calls above test
+ * every atom of a crystal against every atom and image, quadratic).  Arguments, outputs, the (i, j, S) set, the
+ * canonical order, edge_cell_shift and num_neigh are those of mt_neighbor_count / mt_neighbor_fill, bit for bit:
+ * binning only selects candidates, and each candidate is accepted by the pair search's own fp64 expressions
+ * (|S_k| <= R_k with its image bound R_k, then |pos[j] - pos[i] + S @ cell|^2 < r_max^2 in the given frame).
+ * Complete for every input the pair search takes: positions anywhere relative to the cell (they are wrapped into it
+ * for binning only), triclinic cells, cells thinner than r_max (more images are searched), and a zero cell
+ * (|det| == 0: no images, bins over the crystal's bounding box).  An atom with a non-finite coordinate has no edges,
+ * as in the pair search.  Bins are at most max(1, atoms) per crystal, so the workspace depends on N and B alone.
+ * offsets[N] is -1 when the search would give 2^31 edges or more (edge_index offsets are int32), or when a cell is
+ * about a millionth of r_max thin; mt_neighbor_cells_fill rejects such an E with MT_EINVAL.
+ * workspace: mt_neighbor_cells_workspace_bytes(N, B), shared by the two calls. */
+size_t mt_neighbor_cells_workspace_bytes(int64_t N, int64_t B);
+int mt_neighbor_cells_count(int dtype, const void* pos, const void* cell, const int64_t* batch, const int64_t* ptr,
+                            int64_t N, int64_t B, double r_max, int32_t* offsets, void* workspace,
+                            size_t workspace_bytes, mt_stream stream);
+int mt_neighbor_cells_fill(int dtype, const void* pos, const int64_t* batch, const int64_t* ptr, int64_t N, int64_t B,
+                           double r_max, const int32_t* offsets, const void* workspace, int64_t* edge_index,
+                           void* edge_cell_shift, void* num_neigh, int64_t E, mt_stream stream);
+
 /* a4: _AtomicNumberToIndex + one-hot + Linear(S, dim, bias), reference
  * src/matten/nn/embedding.py:85-110, 206-263.
  *   idx = lut[Z - min_Z] (MT_FLAG_BAD_SPECIES if Z out of range or lut == -1)

@@ -78,6 +78,9 @@ SIGNATURES = {
     "mt_neighbor_workspace_bytes": (_Z, [_L, _L]),
     "mt_neighbor_count": (_I, [_I, _V, _V, _V, _V, _L, _L, _D, _V, _V, _Z, _V]),
     "mt_neighbor_fill": (_I, [_I, _V, _V, _V, _L, _L, _D, _V, _V, _V, _V, _V, _L, _V]),
+    "mt_neighbor_cells_workspace_bytes": (_Z, [_L, _L]),
+    "mt_neighbor_cells_count": (_I, [_I, _V, _V, _V, _V, _L, _L, _D, _V, _V, _Z, _V]),
+    "mt_neighbor_cells_fill": (_I, [_I, _V, _V, _V, _L, _L, _D, _V, _V, _V, _V, _V, _L, _V]),
     "mt_species_embed": (_I, [_I, _V, _I, _V, _L, _L, _I, _I, _V, _V, _L, _V, _V, _V, _V, _V]),
     "mt_conv_fwd_workspace_bytes": (_Z, [C.POINTER(ConvPlanStruct), _I, _L, _L]),
     "mt_conv_fwd": (_I, [C.POINTER(ConvPlanStruct), _I, _V, _V, _V, C.POINTER(_V), _V, _V, _V, _D, _V, _V,

@@ -512,6 +512,42 @@ struct NlGraph {
   int pad;
 };
 
+// The pair and the cell search derive the determinant, the fractional coordinates, the heights and the squared
+// distance of a candidate (i, j, S) from these expressions alone, so that both compute the same bits for them.
+__device__ __forceinline__ double nl_det(const double* c) {
+  return c[0] * (c[4] * c[8] - c[5] * c[7]) - c[1] * (c[3] * c[8] - c[5] * c[6]) +
+         c[2] * (c[3] * c[7] - c[4] * c[6]);
+}
+
+// inverse (adjugate / det): frac = pos @ inv(cell)
+__device__ __forceinline__ void nl_inverse(const double* c, double det, double* inv) {
+  inv[0] = (c[4] * c[8] - c[5] * c[7]) / det; inv[1] = (c[2] * c[7] - c[1] * c[8]) / det; inv[2] = (c[1] * c[5] - c[2] * c[4]) / det;
+  inv[3] = (c[5] * c[6] - c[3] * c[8]) / det; inv[4] = (c[0] * c[8] - c[2] * c[6]) / det; inv[5] = (c[2] * c[3] - c[0] * c[5]) / det;
+  inv[6] = (c[3] * c[7] - c[4] * c[6]) / det; inv[7] = (c[1] * c[6] - c[0] * c[7]) / det; inv[8] = (c[0] * c[4] - c[1] * c[3]) / det;
+}
+
+__device__ __forceinline__ double nl_frac(double x, double y, double z, const double* inv, int k) {
+  return x * inv[k] + y * inv[3 + k] + z * inv[6 + k];
+}
+
+// distance between the lattice planes normal to axis k
+__device__ __forceinline__ double nl_height(const double* c, double vol, int k) {
+  const double* a = c + 3 * ((k + 1) % 3);
+  const double* d = c + 3 * ((k + 2) % 3);
+  const double cx = a[1] * d[2] - a[2] * d[1], cy = a[2] * d[0] - a[0] * d[2], cz = a[0] * d[1] - a[1] * d[0];
+  return vol / sqrt(cx * cx + cy * cy + cz * cz);
+}
+
+// offset = S @ cell, then d = (pos[j] - pos[i]) + offset, |d|^2 = (dx^2 + dy^2) + dz^2 without contraction
+__device__ __forceinline__ double nl_dist2(double dx0, double dy0, double dz0, int sx, int sy, int sz,
+                                           const double* c) {
+  const double ox = fma((double)sz, c[6], fma((double)sy, c[3], (double)sx * c[0]));
+  const double oy = fma((double)sz, c[7], fma((double)sy, c[4], (double)sx * c[1]));
+  const double oz = fma((double)sz, c[8], fma((double)sy, c[5], (double)sx * c[2]));
+  const double dx = dx0 + ox, dy = dy0 + oy, dz = dz0 + oz;
+  return __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz));
+}
+
 template <typename T>
 __global__ void __launch_bounds__(128) nl_setup_kernel(const T* __restrict__ pos, const T* __restrict__ cell,
                                                        const int64_t* __restrict__ ptr, int64_t B, double r_max,
@@ -521,38 +557,24 @@ __global__ void __launch_bounds__(128) nl_setup_kernel(const T* __restrict__ pos
   NlGraph g;
   for (int k = 0; k < 9; ++k) g.c[k] = (double)cell[b * 9 + k];
   const double* c = g.c;
-  const double det = c[0] * (c[4] * c[8] - c[5] * c[7]) - c[1] * (c[3] * c[8] - c[5] * c[6]) +
-                     c[2] * (c[3] * c[7] - c[4] * c[6]);
+  const double det = nl_det(c);
   const double vol = fabs(det);
   int span = 0;
   if (vol > 0) {
-    // inverse (adjugate / det): frac = pos @ inv(cell)
     double inv[9];
-    inv[0] = (c[4] * c[8] - c[5] * c[7]) / det; inv[1] = (c[2] * c[7] - c[1] * c[8]) / det; inv[2] = (c[1] * c[5] - c[2] * c[4]) / det;
-    inv[3] = (c[5] * c[6] - c[3] * c[8]) / det; inv[4] = (c[0] * c[8] - c[2] * c[6]) / det; inv[5] = (c[2] * c[3] - c[0] * c[5]) / det;
-    inv[6] = (c[3] * c[7] - c[4] * c[6]) / det; inv[7] = (c[1] * c[6] - c[0] * c[7]) / det; inv[8] = (c[0] * c[4] - c[1] * c[3]) / det;
+    nl_inverse(c, det, inv);
     double fmin = 1e300, fmax = -1e300;
     for (int64_t i = ptr[b]; i < ptr[b + 1]; ++i) {
       const double x = (double)pos[i * 3], y = (double)pos[i * 3 + 1], z = (double)pos[i * 3 + 2];
       for (int k = 0; k < 3; ++k) {
-        const double f = x * inv[k] + y * inv[3 + k] + z * inv[6 + k];
+        const double f = nl_frac(x, y, z, inv, k);
         fmin = f < fmin ? f : fmin;
         fmax = f > fmax ? f : fmax;
       }
     }
     if (ptr[b + 1] > ptr[b]) span = (int)ceil(fmax - fmin);
   }
-  for (int k = 0; k < 3; ++k) {
-    int r = 0;
-    if (vol > 0) {
-      const double* a = c + 3 * ((k + 1) % 3);
-      const double* d = c + 3 * ((k + 2) % 3);
-      const double cx = a[1] * d[2] - a[2] * d[1], cy = a[2] * d[0] - a[0] * d[2], cz = a[0] * d[1] - a[1] * d[0];
-      const double height = vol / sqrt(cx * cx + cy * cy + cz * cz);
-      r = (int)ceil(r_max / height) + span;
-    }
-    g.R[k] = r;
-  }
+  for (int k = 0; k < 3; ++k) g.R[k] = vol > 0 ? (int)ceil(r_max / nl_height(c, vol, k)) + span : 0;
   g.pad = 0;
   out[b] = g;
 }
@@ -578,12 +600,7 @@ __global__ void __launch_bounds__(128) nl_pairs_kernel(const T* __restrict__ pos
     for (int sx = -g.R[0]; sx <= g.R[0]; ++sx)
       for (int sy = -g.R[1]; sy <= g.R[1]; ++sy)
         for (int sz = -g.R[2]; sz <= g.R[2]; ++sz) {
-          // offset = S @ cell, then d = (pos[j] - pos[i]) + offset, |d|^2 = (dx^2 + dy^2) + dz^2 without contraction
-          const double ox = fma((double)sz, g.c[6], fma((double)sy, g.c[3], (double)sx * g.c[0]));
-          const double oy = fma((double)sz, g.c[7], fma((double)sy, g.c[4], (double)sx * g.c[1]));
-          const double oz = fma((double)sz, g.c[8], fma((double)sy, g.c[5], (double)sx * g.c[2]));
-          const double dx = dx0 + ox, dy = dy0 + oy, dz = dz0 + oz;
-          const double d2 = __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz));
+          const double d2 = nl_dist2(dx0, dy0, dz0, sx, sy, sz, g.c);
           if (d2 < r2 && !(j == i && sx == 0 && sy == 0 && sz == 0)) {
             if (FILL) {
               ei[w] = i;
@@ -599,6 +616,359 @@ __global__ void __launch_bounds__(128) nl_pairs_kernel(const T* __restrict__ pos
   else counts[i] = cnt;
 }
 
+// =========================================================================
+// cell-list neighbour search: the same (i, j, S) set, order and outputs as nl_pairs_kernel, in time linear in the
+// atoms of a crystal.  Binning is only a prefilter: a candidate (i, j, S) is accepted by nl_pairs_kernel's own
+// expressions (nl_dist2 against r_max^2 in the original frame, the image bound |S_k| <= R_k with the same R_k).
+//
+// Periodic crystal (|det cell| > 0): fractional coordinates f are wrapped, n = floor(f), w = f - n, bin
+// min(floor(w nb_k), nb_k - 1).  Bins are no thinner than r_max (1 + 2 eps) in each height h_k and the search covers
+// D_k = ceil(r_max (1 + eps) nb_k / h_k) bins on each side, so every pair closer than r_max is found also when the
+// cell is thinner than r_max (then nb_k = 1 and the window holds many images).  A window bin g maps to the wrapped
+// bin g mod nb and the image T = floor(g / nb) of the wrapped frame; S = T - n_j + n_i in the original frame.
+// Zero cell (no images): bins over the Cartesian bounding box of the crystal, D = 1, no wrapping.
+// =========================================================================
+constexpr double kNlEps = 1e-6;
+
+struct NlCells {
+  double c[9];         // cell rows
+  double inv[9];       // inverse of the cell (periodic crystals)
+  double lo[3];        // zero cell: lower corner of the bounding box
+  double scale[3];     // bins per unit of the binning coordinate (periodic: nb; zero cell: nb / extent)
+  uint64_t wprod;      // bins in the search window of a centre: (2 D0 + 1)(2 D1 + 1)(2 D2 + 1)
+  int R[3];            // image bound of nl_pairs_kernel
+  int nb[3];           // bins per axis
+  int D[3];            // window half-width in bins
+  int periodic;
+};
+
+// per atom: integer part of the fractional coordinates, and its bin in its crystal (-1: a non-finite coordinate)
+struct NlCentre {
+  int n[3];
+  int bin;
+};
+
+// per bin-sorted atom: what a candidate test reads
+struct NlAtom {
+  double p[3];
+  int j;
+  int n[3];
+};
+
+// order-preserving map of a (non-NaN) double onto uint64, for atomicMin / atomicMax
+__device__ __forceinline__ unsigned long long nl_ord(double v) {
+  const unsigned long long u = (unsigned long long)__double_as_longlong(v);
+  return (u >> 63) ? ~u : (u | 0x8000000000000000ull);
+}
+__device__ __forceinline__ double nl_unord(unsigned long long u) {
+  return __longlong_as_double((long long)((u >> 63) ? (u & 0x7fffffffffffffffull) : ~u));
+}
+
+__device__ __forceinline__ int nl_floor_div(int a, int n) { return a >= 0 ? a / n : -((-a + n - 1) / n); }
+
+// binning coordinates of an atom: fractional (periodic crystal) or Cartesian (zero cell)
+__device__ __forceinline__ void nl_cells_coords(const NlCells& g, double x, double y, double z, double* f) {
+  if (g.periodic) {
+#pragma unroll
+    for (int k = 0; k < 3; ++k) f[k] = nl_frac(x, y, z, g.inv, k);
+  } else {
+    f[0] = x; f[1] = y; f[2] = z;
+  }
+}
+
+// ext [B,6]: per axis min (0..2) and max (3..5) of the binning coordinates, starting at nl_setup_kernel's 1e300 / -1e300
+template <typename T>
+__global__ void __launch_bounds__(128) nl_cells_setup_kernel(const T* __restrict__ cell, int64_t B,
+                                                             NlCells* __restrict__ cs,
+                                                             unsigned long long* __restrict__ ext) {
+  const int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  NlCells g;
+  for (int k = 0; k < 9; ++k) g.c[k] = (double)cell[b * 9 + k];
+  const double det = nl_det(g.c);
+  g.periodic = fabs(det) > 0;
+  if (g.periodic) nl_inverse(g.c, det, g.inv);
+  else
+    for (int k = 0; k < 9; ++k) g.inv[k] = 0.0;
+  cs[b] = g;
+  for (int k = 0; k < 3; ++k) {
+    ext[b * 6 + k] = nl_ord(1e300);
+    ext[b * 6 + 3 + k] = nl_ord(-1e300);
+  }
+}
+
+// min / max of the binning coordinates per crystal, NaN skipped (as nl_setup_kernel's comparisons skip it): a block
+// of one crystal reduces in shared memory first, a block across crystals falls back to one atomic per atom and value
+template <typename T>
+__global__ void __launch_bounds__(256) nl_cells_extent_kernel(const T* __restrict__ pos,
+                                                              const int64_t* __restrict__ batch, int64_t N,
+                                                              const NlCells* __restrict__ cs,
+                                                              unsigned long long* __restrict__ ext) {
+  __shared__ double red[8][6];
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  const bool valid = i < N;
+  const int64_t b = valid && batch ? batch[i] : 0;
+  double v[6] = {1e300, 1e300, 1e300, -1e300, -1e300, -1e300};
+  if (valid) {
+    double f[3];
+    nl_cells_coords(cs[b], (double)pos[i * 3], (double)pos[i * 3 + 1], (double)pos[i * 3 + 2], f);
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      v[k] = f[k] < v[k] ? f[k] : v[k];
+      v[3 + k] = f[k] > v[3 + k] ? f[k] : v[3 + k];
+    }
+  }
+  const int64_t b0 = batch ? batch[blockIdx.x * (int64_t)blockDim.x] : 0;
+  if (__syncthreads_and(!valid || b == b0)) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int k = 0; k < 6; ++k) {
+      for (int o = 16; o > 0; o >>= 1) {
+        const double u = __shfl_xor_sync(0xffffffffu, v[k], o);
+        v[k] = k < 3 ? (u < v[k] ? u : v[k]) : (u > v[k] ? u : v[k]);
+      }
+      if (lane == 0) red[warp][k] = v[k];
+    }
+    __syncthreads();
+    if (threadIdx.x < 6) {
+      const int k = threadIdx.x;
+      double r = red[0][k];
+      for (int w = 1; w < 8; ++w) r = k < 3 ? (red[w][k] < r ? red[w][k] : r) : (red[w][k] > r ? red[w][k] : r);
+      if (k < 3) atomicMin(&ext[b0 * 6 + k], nl_ord(r));
+      else atomicMax(&ext[b0 * 6 + k], nl_ord(r));
+    }
+  } else if (valid) {
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      atomicMin(&ext[b * 6 + k], nl_ord(v[k]));
+      atomicMax(&ext[b * 6 + 3 + k], nl_ord(v[3 + k]));
+    }
+  }
+}
+
+// per crystal: nl_setup_kernel's R_k, then the bins (at most max(1, atoms) per crystal) and the search window.
+// nbins[b] = bins of crystal b (scanned into bin offsets next); status != 0 if a window cannot be indexed in 64 bits.
+__global__ void __launch_bounds__(128) nl_cells_grid_kernel(const int64_t* __restrict__ ptr, int64_t B, double r_max,
+                                                            NlCells* __restrict__ cs,
+                                                            const unsigned long long* __restrict__ ext,
+                                                            int32_t* __restrict__ nbins, int32_t* __restrict__ status) {
+  const int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (b == 0) nbins[B] = 0;
+  if (b >= B) return;
+  NlCells g = cs[b];
+  const int64_t n = ptr[b + 1] - ptr[b];
+  double lo[3], hi[3], len[3];
+  for (int k = 0; k < 3; ++k) {
+    lo[k] = nl_unord(ext[b * 6 + k]);
+    hi[k] = nl_unord(ext[b * 6 + 3 + k]);
+  }
+  if (g.periodic) {
+    const double f_lo = fmin(fmin(lo[0], lo[1]), lo[2]), f_hi = fmax(fmax(hi[0], hi[1]), hi[2]);
+    const int span = n > 0 ? (int)ceil(f_hi - f_lo) : 0;
+    const double vol = fabs(nl_det(g.c));
+    for (int k = 0; k < 3; ++k) {
+      len[k] = nl_height(g.c, vol, k);
+      g.R[k] = (int)ceil(r_max / len[k]) + span;
+    }
+  } else {
+    for (int k = 0; k < 3; ++k) {
+      len[k] = hi[k] - lo[k];
+      g.lo[k] = lo[k];
+      g.R[k] = 0;
+    }
+  }
+  const double cap = n > 1 ? (double)n : 1.0;
+  double nb[3];
+  for (int k = 0; k < 3; ++k) nb[k] = fmin(cap, fmax(1.0, floor(len[k] / (r_max * (1.0 + 2.0 * kNlEps)))));
+  for (double prod = nb[0] * nb[1] * nb[2]; prod > cap; prod = nb[0] * nb[1] * nb[2]) {
+    const int k = nb[0] >= nb[1] ? (nb[0] >= nb[2] ? 0 : 2) : (nb[1] >= nb[2] ? 1 : 2);
+    nb[k] = fmax(1.0, fmin(nb[k] - 1.0, floor(nb[k] * cap / prod)));
+  }
+  double wprod = 1.0;
+  bool ok = true;
+  for (int k = 0; k < 3; ++k) {
+    g.nb[k] = (int)nb[k];
+    const double d = g.periodic ? ceil(r_max * (1.0 + kNlEps) * nb[k] / len[k]) : 1.0;
+    ok = ok && d < 1e6;
+    g.D[k] = ok ? (int)d : 1;
+    g.scale[k] = g.periodic ? nb[k] : (len[k] > 0 ? nb[k] / len[k] : 0.0);
+    wprod *= 2.0 * g.D[k] + 1.0;
+  }
+  // a fill entry packs (j - ptr[b]) * wprod + (window index) into 63 bits
+  if (!ok || wprod * cap >= 4e18) atomicOr(status, 1);
+  g.wprod = (uint64_t)wprod;
+  cs[b] = g;
+  nbins[b] = g.nb[0] * g.nb[1] * g.nb[2];
+}
+
+// keys[i] = global bin of atom i (bin0[b] + local bin), `sentinel` for an atom with a non-finite coordinate
+template <typename T>
+__global__ void __launch_bounds__(256) nl_cells_bin_kernel(const T* __restrict__ pos, const int64_t* __restrict__ batch,
+                                                           int64_t N, const NlCells* __restrict__ cs,
+                                                           const int32_t* __restrict__ bin0, int64_t sentinel,
+                                                           int64_t* __restrict__ keys, NlCentre* __restrict__ cen) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i >= N) return;
+  const int64_t b = batch ? batch[i] : 0;
+  const NlCells& g = cs[b];
+  double f[3];
+  nl_cells_coords(g, (double)pos[i * 3], (double)pos[i * 3 + 1], (double)pos[i * 3 + 2], f);
+  NlCentre a = {{0, 0, 0}, -1};
+  int64_t key = sentinel;
+  if (isfinite(f[0]) && isfinite(f[1]) && isfinite(f[2])) {
+    int cb[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+      double w = f[k] - g.lo[k];
+      if (g.periodic) {
+        const double fl = floor(f[k]);
+        a.n[k] = (int)fl;
+        w = f[k] - fl;
+      }
+      const int c = (int)floor(w * g.scale[k]);
+      cb[k] = c < 0 ? 0 : (c < g.nb[k] ? c : g.nb[k] - 1);
+    }
+    a.bin = (cb[0] * g.nb[1] + cb[1]) * g.nb[2] + cb[2];
+    key = bin0[b] + a.bin;
+  }
+  keys[i] = key;
+  cen[i] = a;
+}
+
+template <typename T>
+__global__ void __launch_bounds__(256) nl_cells_gather_kernel(const T* __restrict__ pos, const int32_t* __restrict__ perm,
+                                                              const NlCentre* __restrict__ cen, int64_t N,
+                                                              NlAtom* __restrict__ rec) {
+  const int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (s >= N) return;
+  const int j = perm[s];
+  const NlCentre a = cen[j];
+  rec[s] = {{(double)pos[(int64_t)j * 3], (double)pos[(int64_t)j * 3 + 1], (double)pos[(int64_t)j * 3 + 2]},
+            j, {a.n[0], a.n[1], a.n[2]}};
+}
+
+// One thread per centre, centres in bin order (neighbouring threads search the same bins).  FILL == false: counts[i]
+// = neighbours of centre i; FILL == true: entries (j - ptr[b]) * wprod + (window index) at offsets[i] in edge_index
+// row 0, ordered by nl_cells_order_kernel, and num_neigh.
+template <typename T, bool FILL>
+__global__ void __launch_bounds__(128) nl_cells_pairs_kernel(
+    const int64_t* __restrict__ batch, const int64_t* __restrict__ ptr, const NlCells* __restrict__ cs,
+    const int32_t* __restrict__ bin0, const int32_t* __restrict__ rowptr, const NlAtom* __restrict__ rec,
+    const NlCentre* __restrict__ cen, int64_t N, double r2, int32_t* __restrict__ counts,
+    const int32_t* __restrict__ offsets, uint64_t* __restrict__ entries, T* __restrict__ num_neigh) {
+  const int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (s >= N) return;
+  const NlAtom a = rec[s];
+  const int i = a.j;
+  const NlCentre ci = cen[i];
+  int cnt = 0;
+  if (ci.bin >= 0) {
+    const int64_t b = batch ? batch[i] : 0;
+    const NlCells& g = cs[b];
+    double c[9];
+#pragma unroll
+    for (int k = 0; k < 9; ++k) c[k] = g.c[k];
+    const int nb0 = g.nb[0], nb1 = g.nb[1], nb2 = g.nb[2];
+    const int D0 = g.D[0], D1 = g.D[1], D2 = g.D[2];
+    const int R0 = g.R[0], R1 = g.R[1], R2 = g.R[2];
+    const bool periodic = g.periodic;
+    const uint64_t wprod = g.wprod;
+    const int cz = ci.bin % nb2, cy = (ci.bin / nb2) % nb1, cx = ci.bin / (nb2 * nb1);
+    const int64_t j0 = ptr[b];
+    const int32_t* bp = rowptr + bin0[b];
+    int64_t w = FILL ? offsets[i] : 0;
+    uint64_t t = 0;  // window index, lexicographic in (gx, gy, gz)
+    for (int gx = cx - D0; gx <= cx + D0; ++gx) {
+      const int tx = periodic ? nl_floor_div(gx, nb0) : 0, bx = gx - tx * nb0;
+      for (int gy = cy - D1; gy <= cy + D1; ++gy) {
+        const int ty = periodic ? nl_floor_div(gy, nb1) : 0, by = gy - ty * nb1;
+        for (int gz = cz - D2; gz <= cz + D2; ++gz, ++t) {
+          const int tz = periodic ? nl_floor_div(gz, nb2) : 0, bz = gz - tz * nb2;
+          if (bx < 0 || bx >= nb0 || by < 0 || by >= nb1 || bz < 0 || bz >= nb2) continue;  // zero cell only
+          const int bin = (bx * nb1 + by) * nb2 + bz;
+          for (int q = bp[bin], qe = bp[bin + 1]; q < qe; ++q) {
+            const NlAtom o = rec[q];
+            const int sx = tx - o.n[0] + ci.n[0], sy = ty - o.n[1] + ci.n[1], sz = tz - o.n[2] + ci.n[2];
+            if (abs(sx) > R0 || abs(sy) > R1 || abs(sz) > R2) continue;
+            const double d2 = nl_dist2(o.p[0] - a.p[0], o.p[1] - a.p[1], o.p[2] - a.p[2], sx, sy, sz, c);
+            if (d2 < r2 && !(o.j == i && sx == 0 && sy == 0 && sz == 0)) {
+              if (FILL) entries[w++] = (uint64_t)(o.j - j0) * wprod + t;
+              ++cnt;
+            }
+          }
+        }
+      }
+    }
+  }
+  if (FILL) { if (num_neigh) num_neigh[i] = (T)cnt; }
+  else counts[i] = cnt;
+}
+
+// One warp per centre: the rank of every entry among the centre's entries (all distinct) is its place in the
+// canonical (j, Sx, Sy, Sz) order -- the window index is lexicographic in the wrapped image T, and S = T - n_j + n_i.
+// Writes edge_index row 1 and the shifts at that place, then overwrites the entries with the centre.  Any degree.
+template <typename T>
+__global__ void __launch_bounds__(256) nl_cells_order_kernel(const int64_t* __restrict__ batch,
+                                                             const int64_t* __restrict__ ptr,
+                                                             const NlCells* __restrict__ cs,
+                                                             const NlCentre* __restrict__ cen,
+                                                             const int32_t* __restrict__ offsets, int64_t N, int64_t E,
+                                                             int64_t* __restrict__ ei, T* __restrict__ shifts) {
+  const int64_t i = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (i >= N) return;
+  const int64_t beg = offsets[i], end = offsets[i + 1];
+  if (beg == end) return;
+  const int64_t b = batch ? batch[i] : 0;
+  const NlCells& g = cs[b];
+  const NlCentre ci = cen[i];
+  const int nb0 = g.nb[0], nb1 = g.nb[1], nb2 = g.nb[2];
+  const int W1 = 2 * g.D[1] + 1, W2 = 2 * g.D[2] + 1;
+  const uint64_t wprod = g.wprod;
+  const int cz = ci.bin % nb2, cy = (ci.bin / nb2) % nb1, cx = ci.bin / (nb2 * nb1);
+  const int64_t j0 = ptr[b];
+  const uint64_t* entries = reinterpret_cast<const uint64_t*>(ei);
+  for (int64_t p0 = beg; p0 < end; p0 += 32) {
+    const int64_t p = p0 + lane;
+    const uint64_t key = p < end ? entries[p] : ~0ull;
+    int64_t rank = 0;
+    for (int64_t q0 = beg; q0 < end; q0 += 32) {
+      const uint64_t kq = q0 + lane < end ? entries[q0 + lane] : ~0ull;
+#pragma unroll 8
+      for (int l = 0; l < 32; ++l) rank += __shfl_sync(0xffffffffu, kq, l) < key;
+    }
+    if (p < end) {
+      const int64_t j = j0 + (int64_t)(key / wprod);
+      uint64_t t = key % wprod;
+      const int tz = (int)(t % W2);
+      t /= W2;
+      const int ty = (int)(t % W1), tx = (int)(t / W1);
+      const int gx = cx - g.D[0] + tx, gy = cy - g.D[1] + ty, gz = cz - g.D[2] + tz;
+      const NlCentre cj = cen[j];
+      int S[3] = {0, 0, 0};
+      if (g.periodic) {
+        S[0] = nl_floor_div(gx, nb0) - cj.n[0] + ci.n[0];
+        S[1] = nl_floor_div(gy, nb1) - cj.n[1] + ci.n[1];
+        S[2] = nl_floor_div(gz, nb2) - cj.n[2] + ci.n[2];
+      }
+      const int64_t e = beg + rank;
+      ei[E + e] = j;
+#pragma unroll
+      for (int k = 0; k < 3; ++k) shifts[e * 3 + k] = (T)S[k];
+    }
+  }
+  __syncwarp();
+  for (int64_t p = beg + lane; p < end; p += 32) ei[p] = i;
+}
+
+// offsets[N] = -1 when the int32 scan of the counts wrapped (2^31 edges or more) or a window could not be indexed
+__global__ void __launch_bounds__(256) nl_cells_total_kernel(int32_t* __restrict__ offsets, int64_t N,
+                                                             const int32_t* __restrict__ status) {
+  const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (i >= N) return;
+  if (offsets[i + 1] < offsets[i] || *status != 0) offsets[N] = -1;
+}
+
 }  // namespace mt
 
 // ===========================================================================
@@ -607,6 +977,8 @@ __global__ void __launch_bounds__(128) nl_pairs_kernel(const T* __restrict__ pos
 using namespace mt;
 
 static inline unsigned grid_for(int64_t n, int threads) { return (unsigned)ceil_div<int64_t>(n, threads); }
+static int csr_by_key_run(const int64_t* keys, int64_t E, int64_t num_keys, int32_t* rowptr, int32_t* perm,
+                          void* workspace, int32_t* err_flag, cudaStream_t st);
 
 extern "C" {
 
@@ -790,6 +1162,14 @@ int mt_csr_by_key(const int64_t* keys, int64_t E, int64_t num_keys, int32_t* row
     return MT_OK;
   }
   MT_REQUIRE(keys && workspace, "null pointer");
+  return csr_by_key_run(keys, E, num_keys, rowptr, perm, workspace, err_flag, st);
+}
+
+}  // extern "C"
+
+// the stable radix sort behind mt_csr_by_key (checked arguments, E > 0)
+static int csr_by_key_run(const int64_t* keys, int64_t E, int64_t num_keys, int32_t* rowptr, int32_t* perm,
+                          void* workspace, int32_t* err_flag, cudaStream_t st) {
   char* ws = (char*)workspace;
   size_t eb = align256((size_t)E * 4);
   int32_t* k0 = (int32_t*)ws;
@@ -833,6 +1213,8 @@ int mt_csr_by_key(const int64_t* keys, int64_t E, int64_t num_keys, int32_t* row
   MT_LAUNCH_OK();
   return MT_OK;
 }
+
+extern "C" {
 
 int mt_gather_i64_to_i32(const int64_t* src, const int32_t* perm, int64_t n, int32_t* out,
                          mt_stream stream) {
@@ -917,6 +1299,127 @@ int mt_neighbor_fill(int dtype, const void* pos, const int64_t* batch, const int
     nl_pairs_kernel<T, true><<<grid_for(N, 128), 128, 0, as_stream(stream)>>>(
         (const T*)pos, batch, ptr, graphs, N, r_max * r_max, nullptr, offsets, edge_index, E, (T*)edge_cell_shift,
         (T*)num_neigh);
+  });
+  MT_LAUNCH_OK();
+  return MT_OK;
+}
+
+
+// Workspace of the cell search, shared by count and fill; sized from N and B alone (at most N + B bins in all).
+struct NlCellsLayout {
+  size_t cells, ext, bin0, status, keys, rowptr, perm, cen, rec, scan, csr, total;
+  NlCellsLayout(int64_t N, int64_t B) {
+    if (N < 0) N = 0;
+    if (B < 1) B = 1;
+    size_t o = 0;
+    auto take = [&o](size_t bytes) { const size_t at = o; o += align256(bytes); return at; };
+    cells = take((size_t)B * sizeof(NlCells));
+    ext = take((size_t)B * 6 * sizeof(unsigned long long));
+    bin0 = take((size_t)(B + 1) * 4);
+    status = take(4);
+    keys = take((size_t)N * 8);
+    rowptr = take((size_t)(N + B + 2) * 4);
+    perm = take((size_t)N * 4);
+    cen = take((size_t)N * sizeof(NlCentre));
+    rec = take((size_t)N * sizeof(NlAtom));
+    scan = take(scan_tmp_elems((N > B ? N : B) + 1) * 4);
+    csr = take(mt_csr_workspace_bytes(N + B + 1, N));
+    total = o;
+  }
+};
+
+size_t mt_neighbor_cells_workspace_bytes(int64_t N, int64_t B) { return NlCellsLayout(N, B).total; }
+
+int mt_neighbor_cells_count(int dtype, const void* pos, const void* cell, const int64_t* batch, const int64_t* ptr,
+                            int64_t N, int64_t B, double r_max, int32_t* offsets, void* workspace,
+                            size_t workspace_bytes, mt_stream stream) {
+  MT_ENTRY_GUARD();
+  MT_REQUIRE(N >= 0 && B >= 1 && r_max > 0, "bad arguments");
+  MT_REQUIRE(N + B + 2 < (int64_t)2147483647, "N + B must fit int32");
+  MT_REQUIRE(pos && cell && ptr && offsets && workspace, "null pointer");
+  MT_REQUIRE(B == 1 || batch != nullptr, "batch vector required for more than one graph");
+  MT_REQUIRE(workspace_bytes >= mt_neighbor_cells_workspace_bytes(N, B), "neighbour-list workspace too small");
+  cudaStream_t st = as_stream(stream);
+  const NlCellsLayout L(N, B);
+  unsigned char* ws = static_cast<unsigned char*>(workspace);
+  NlCells* cs = reinterpret_cast<NlCells*>(ws + L.cells);
+  unsigned long long* ext = reinterpret_cast<unsigned long long*>(ws + L.ext);
+  int32_t* bin0 = reinterpret_cast<int32_t*>(ws + L.bin0);
+  int32_t* status = reinterpret_cast<int32_t*>(ws + L.status);
+  int64_t* keys = reinterpret_cast<int64_t*>(ws + L.keys);
+  int32_t* rowptr = reinterpret_cast<int32_t*>(ws + L.rowptr);
+  int32_t* perm = reinterpret_cast<int32_t*>(ws + L.perm);
+  NlCentre* cen = reinterpret_cast<NlCentre*>(ws + L.cen);
+  NlAtom* rec = reinterpret_cast<NlAtom*>(ws + L.rec);
+  int32_t* tmp = reinterpret_cast<int32_t*>(ws + L.scan);
+  MT_CUDA_OK(cudaMemsetAsync(offsets + N, 0, sizeof(int32_t), st));
+  if (N == 0) return MT_OK;
+  MT_CUDA_OK(cudaMemsetAsync(status, 0, sizeof(int32_t), st));
+  MT_DISPATCH_DTYPE(dtype, {
+    nl_cells_setup_kernel<T><<<grid_for(B, 128), 128, 0, st>>>((const T*)cell, B, cs, ext);
+  });
+  MT_LAUNCH_OK();
+  MT_DISPATCH_DTYPE(dtype, {
+    nl_cells_extent_kernel<T><<<grid_for(N, 256), 256, 0, st>>>((const T*)pos, batch, N, cs, ext);
+  });
+  MT_LAUNCH_OK();
+  nl_cells_grid_kernel<<<grid_for(B, 128), 128, 0, st>>>(ptr, B, r_max, cs, ext, bin0, status);
+  MT_LAUNCH_OK();
+  int rc = exclusive_scan_i32(bin0, B + 1, tmp, st);
+  if (rc != MT_OK) return rc;
+  const int64_t sentinel = N + B;  // bins of all crystals number at most N + B
+  MT_DISPATCH_DTYPE(dtype, {
+    nl_cells_bin_kernel<T><<<grid_for(N, 256), 256, 0, st>>>((const T*)pos, batch, N, cs, bin0, sentinel, keys, cen);
+  });
+  MT_LAUNCH_OK();
+  rc = csr_by_key_run(keys, N, sentinel + 1, rowptr, perm, ws + L.csr, nullptr, st);
+  if (rc != MT_OK) return rc;
+  MT_DISPATCH_DTYPE(dtype, {
+    nl_cells_gather_kernel<T><<<grid_for(N, 256), 256, 0, st>>>((const T*)pos, perm, cen, N, rec);
+  });
+  MT_LAUNCH_OK();
+  MT_DISPATCH_DTYPE(dtype, {
+    nl_cells_pairs_kernel<T, false><<<grid_for(N, 128), 128, 0, st>>>(batch, ptr, cs, bin0, rowptr, rec, cen, N,
+                                                                       r_max * r_max, offsets, nullptr, nullptr,
+                                                                       nullptr);
+  });
+  MT_LAUNCH_OK();
+  rc = exclusive_scan_i32(offsets, N + 1, tmp, st);  // offsets[N] = number of edges
+  if (rc != MT_OK) return rc;
+  nl_cells_total_kernel<<<grid_for(N, 256), 256, 0, st>>>(offsets, N, status);
+  MT_LAUNCH_OK();
+  return MT_OK;
+}
+
+int mt_neighbor_cells_fill(int dtype, const void* pos, const int64_t* batch, const int64_t* ptr, int64_t N, int64_t B,
+                           double r_max, const int32_t* offsets, const void* workspace, int64_t* edge_index,
+                           void* edge_cell_shift, void* num_neigh, int64_t E, mt_stream stream) {
+  MT_ENTRY_GUARD();
+  MT_REQUIRE(N >= 0 && B >= 1, "bad arguments");
+  MT_REQUIRE(E >= 0 && E < (int64_t)2147483647,
+             "the cell search found 2^31 edges or more, or a cell too thin to search (offsets[N] = %lld)",
+             (long long)E);
+  if (N == 0) return MT_OK;
+  MT_REQUIRE(pos && ptr && offsets && workspace, "null pointer");
+  MT_REQUIRE(E == 0 || (edge_index && edge_cell_shift), "null output pointer");
+  cudaStream_t st = as_stream(stream);
+  const NlCellsLayout L(N, B);
+  const unsigned char* ws = static_cast<const unsigned char*>(workspace);
+  const NlCells* cs = reinterpret_cast<const NlCells*>(ws + L.cells);
+  const int32_t* bin0 = reinterpret_cast<const int32_t*>(ws + L.bin0);
+  const int32_t* rowptr = reinterpret_cast<const int32_t*>(ws + L.rowptr);
+  const NlCentre* cen = reinterpret_cast<const NlCentre*>(ws + L.cen);
+  const NlAtom* rec = reinterpret_cast<const NlAtom*>(ws + L.rec);
+  MT_DISPATCH_DTYPE(dtype, {
+    nl_cells_pairs_kernel<T, true><<<grid_for(N, 128), 128, 0, st>>>(
+        batch, ptr, cs, bin0, rowptr, rec, cen, N, r_max * r_max, nullptr, offsets,
+        reinterpret_cast<uint64_t*>(edge_index), (T*)num_neigh);
+  });
+  MT_LAUNCH_OK();
+  if (E == 0) return MT_OK;
+  MT_DISPATCH_DTYPE(dtype, {
+    nl_cells_order_kernel<T><<<grid_for(N * 32, 256), 256, 0, st>>>(batch, ptr, cs, cen, offsets, N, E, edge_index,
+                                                                     (T*)edge_cell_shift);
   });
   MT_LAUNCH_OK();
   return MT_OK;

@@ -136,7 +136,8 @@ def batch_from_structures(structs: Sequence[dict], r_cut: float, device, dtype=t
         "num_graphs": len(structs),
     }
     # the search itself runs in fp64 from the fp64 inputs (like the reference's numpy/ASE path), whatever `dtype` is
-    ei, sh, nn = ops.neighbor_list(pos.to(device), cell.to(device), out["batch"], out["ptr"], r_cut)
+    ei, sh, nn = ops.neighbor_list(pos.to(device), cell.to(device), out["batch"], out["ptr"], r_cut,
+                                   max_atoms=max(n_nodes, default=0))
     out["edge_index"] = ei
     out["edge_cell_shift"] = sh.to(dtype)
     out["num_neigh"] = nn.to(dtype)

@@ -203,29 +203,57 @@ def edge_vectors_bwd(edge_vec, grad_vec, grad_len, edge_cell_shift, rowptr, perm
     return gpos, gcell
 
 
+#: Crystals of at least this many atoms take the cell-list search (mt_neighbor_cells_*) under method="auto", smaller
+#: ones the all-pairs search (mt_neighbor_count / mt_neighbor_fill).  profiles/neighbor_list_b200.jsonl, "crossover"
+#: line (one NVIDIA B200, 1000 W): 64 atoms, the smallest size swept, where the cell search took 0.22 ms against 0.95
+#: for one crystal and 0.28 against 0.97 for 64 of them.  Batches of smaller crystals, such as the 100 example
+#: crystals (at most 48 atoms), stay on the pair kernels they used before.
+NL_CELLS_MIN_ATOMS = 64
+
+
+def neighbor_method(ptr, max_atoms: Optional[int] = None, method: str = "auto") -> str:
+    """The search ``neighbor_list`` runs on a batch with node offsets ``ptr``: ``method`` unless it is "auto", else
+    "cells" when the largest crystal (``max_atoms``, or read from ``ptr`` when not given) has at least
+    NL_CELLS_MIN_ATOMS atoms, "pairs" otherwise."""
+    if method not in ("auto", "pairs", "cells"):
+        raise ValueError(f"neighbour-list method must be 'auto', 'pairs' or 'cells', got {method!r}")
+    if method != "auto":
+        return method
+    if max_atoms is None:
+        max_atoms = int((ptr[1:] - ptr[:-1]).max()) if ptr.numel() > 1 else 0
+    return "cells" if max_atoms >= NL_CELLS_MIN_ATOMS else "pairs"
+
+
 @_on_device
-def neighbor_list(pos, cell, batch, ptr, r_max: float):
+def neighbor_list(pos, cell, batch, ptr, r_max: float, max_atoms: Optional[int] = None, method: str = "auto"):
     """Periodic neighbour list of a batch of crystals on the GPU (reference data/data.py:285-413 semantics).
     pos [N,3], cell [B,3,3] (same float dtype), batch [N] int64, ptr [B+1] int64.
-    Returns (edge_index [2,E] int64, edge_cell_shift [E,3], num_neigh [N]) in the canonical (i, j, S) order."""
+    Returns (edge_index [2,E] int64, edge_cell_shift [E,3], num_neigh [N]) in the canonical (i, j, S) order.
+    ``method``: "pairs" (all pairs, quadratic per crystal), "cells" (cell list, linear) or "auto" (cells when the
+    largest crystal has at least NL_CELLS_MIN_ATOMS atoms); both give the same outputs bit for bit.  ``max_atoms``
+    (atoms of the largest crystal) spares "auto" a read of ``ptr`` from the device."""
     lib = _lib.load()
     pos = _req(pos, "pos")
     cell = _req(cell, "cell", pos.dtype).reshape(-1, 3, 3)
     ptr = _req(ptr, "ptr", torch.int64)
     N, B = pos.shape[0], cell.shape[0]
+    cells = neighbor_method(ptr, max_atoms, method) == "cells"
     if B > 1:
         batch = _req(batch, "batch", torch.int64)
+    workspace_bytes, count, fill = (
+        (lib.mt_neighbor_cells_workspace_bytes, lib.mt_neighbor_cells_count, lib.mt_neighbor_cells_fill) if cells else
+        (lib.mt_neighbor_workspace_bytes, lib.mt_neighbor_count, lib.mt_neighbor_fill))
     offsets = torch.empty(N + 1, dtype=torch.int32, device=pos.device)
-    nbytes = lib.mt_neighbor_workspace_bytes(N, B)
+    nbytes = workspace_bytes(N, B)
     ws = torch.empty(nbytes, dtype=torch.uint8, device=pos.device)
-    check(lib.mt_neighbor_count(_dt(pos), _p(pos), _p(cell), _p(batch) if B > 1 else None, _p(ptr), N, B, float(r_max),
-                                _p(offsets), _p(ws), nbytes, _stream(pos)))
+    check(count(_dt(pos), _p(pos), _p(cell), _p(batch) if B > 1 else None, _p(ptr), N, B, float(r_max),
+                _p(offsets), _p(ws), nbytes, _stream(pos)))
     E = int(offsets[-1].item())  # the one synchronisation of graph building: the edge count sizes the outputs
-    ei = torch.empty((2, E), dtype=torch.int64, device=pos.device)
-    shifts = torch.empty((E, 3), dtype=pos.dtype, device=pos.device)
+    ei = torch.empty((2, max(E, 0)), dtype=torch.int64, device=pos.device)
+    shifts = torch.empty((max(E, 0), 3), dtype=pos.dtype, device=pos.device)
     num_neigh = torch.empty(N, dtype=pos.dtype, device=pos.device)
-    check(lib.mt_neighbor_fill(_dt(pos), _p(pos), _p(batch) if B > 1 else None, _p(ptr), N, B, float(r_max),
-                               _p(offsets), _p(ws), _p(ei), _p(shifts), _p(num_neigh), E, _stream(pos)))
+    check(fill(_dt(pos), _p(pos), _p(batch) if B > 1 else None, _p(ptr), N, B, float(r_max),
+               _p(offsets), _p(ws), _p(ei), _p(shifts), _p(num_neigh), E, _stream(pos)))
     return ei, shifts, num_neigh
 
 
