@@ -299,9 +299,13 @@ typedef struct {
  *   (sum_{e: dst(e)=n} msg_e) / sqrt(avg_num_neighbors)        if num_neigh == NULL
  *   (sum ...)             / sqrt(num_neigh[n])                  otherwise (reference
  *   src/matten/nn/conv.py:116-120). Summation order is the CSR order: deterministic. */
-/* workspace (bytes) of the tcgen05 path: room for the per-batch edge layout of mt_conv_layout_prepare, which a call
+/* Radial MLP sizes: 1 .. MT_MAX_MLP_LAYERS weight matrices; input / hidden sizes up to 256 when the last hidden size
+ * is at most 64, up to 128 when the last hidden size is in (64, 128]; a last hidden size above 128 is MT_EINVAL.
+ * workspace (bytes) of the tcgen05 path: room for the per-batch edge layout of mt_conv_layout_prepare, which a call
  * without `layout` builds there, and the last hidden activation of the radial MLP as bf16 hi/mid/lo planes (192 B per
- * column).  0 when the plan / dtype runs on the FMA-pipe kernel, which needs none. */
+ * column).  0 when the plan / dtype runs on the FMA-pipe kernel, which needs none.  A plan whose last hidden size is
+ * above 64 (both dtypes) needs E * mlp_sizes[last] values, 256-byte aligned, for the per-edge weights; a smaller
+ * workspace is MT_EINVAL. */
 size_t mt_conv_fwd_workspace_bytes(const mt_conv_plan* plan, int dtype, int64_t N, int64_t E);
 int mt_conv_fwd(const mt_conv_plan* plan, int dtype, const void* x, const void* sh,
                 const void* emb, const void* const* mlp_weights, const int32_t* rowptr,
@@ -340,7 +344,8 @@ void mt_conv_set_debug_buffer(void* device_buffer);
  *   grad_mlp_weights[i]             : dL/d weights[i], same shapes as mlp_weights[i]; per-CTA partial sums
  *                                     reduced in a fixed order (deterministic for a fixed N, E)
  * workspace: mt_conv_bwd_workspace_bytes bytes (hidden pre-activations, per-edge dw / dx scratch, partial
- * weight gradients). */
+ * weight gradients; when an input / hidden size is above 64, also the per-edge weights [E, mlp_sizes[last]]).
+ * MLP input / hidden sizes up to 128; above that MT_EINVAL. */
 size_t mt_conv_bwd_workspace_bytes(const mt_conv_plan* plan, int dtype, int64_t N, int64_t E);
 int mt_conv_bwd(const mt_conv_plan* plan, int dtype, const void* x, const void* sh, const void* emb,
                 const void* const* mlp_weights, const int32_t* rowptr, const int32_t* perm,

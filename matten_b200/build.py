@@ -29,7 +29,7 @@ NVCC_FLAGS = [
 ]
 
 PLAIN_SOURCES = ["api.cu", "graph_ops.cu", "node_ops.cu", "train_ops.cu", "norm_ops.cu", "conv.cu", "conv_fwd_tc.cu", "conv_bwd.cu"]
-CONV_INST = [(t, hp) for t in ("float", "double") for hp in (8, 16, 32, 64)]
+CONV_INST = [(t, hp) for t in ("float", "double") for hp in (8, 16, 32, 64, 0)]  # 0: per-edge weights from memory
 
 
 def _nvcc() -> str:

@@ -1,5 +1,6 @@
 // Host side of the fused convolution entry points (include/matten_b200.h: mt_conv_fwd).
 #include "conv_fwd.cuh"
+#include "radial_mlp.cuh"
 
 namespace mt {
 
@@ -10,6 +11,7 @@ int launch_conv_fwd(const ConvFwdParams& p, int grid, int threads, size_t smem, 
   template <> int launch_conv_fwd<T, HP>(const ConvFwdParams&, int, int, size_t, cudaStream_t);
 MT_DECL(float, 8) MT_DECL(float, 16) MT_DECL(float, 32) MT_DECL(float, 64)
 MT_DECL(double, 8) MT_DECL(double, 16) MT_DECL(double, 32) MT_DECL(double, 64)
+MT_DECL(float, 0) MT_DECL(double, 0)
 #undef MT_DECL
 
 int conv_fwd_tc_try(const mt_conv_plan* plan, const void* x, const void* sh, const void* emb,
@@ -29,18 +31,25 @@ static int validate_plan(const mt_conv_plan* plan) {
   MT_REQUIRE(plan->mlp_num_layers >= 1 && plan->mlp_num_layers <= MT_MAX_MLP_LAYERS,
              "mlp_num_layers %d not in 1..%d", plan->mlp_num_layers, MT_MAX_MLP_LAYERS);
   for (int i = 0; i <= plan->mlp_num_layers; ++i) MT_REQUIRE(plan->mlp_sizes[i] > 0, "bad mlp size");
-  MT_REQUIRE(pad_hp(plan->mlp_sizes[plan->mlp_num_layers - 1]) > 0,
-             "last hidden size %d > 64 not supported", plan->mlp_sizes[plan->mlp_num_layers - 1]);
-  for (int i = 0; i < plan->mlp_num_layers; ++i)
+  const int last = plan->mlp_sizes[plan->mlp_num_layers - 1];
+  MT_REQUIRE(last <= kWideMaxH, "last hidden size %d > %d not supported", last, kWideMaxH);
+  for (int i = 0; i < plan->mlp_num_layers; ++i) {
     MT_REQUIRE(plan->mlp_sizes[i] <= 256, "mlp layer size %d > 256 not supported", plan->mlp_sizes[i]);
+    MT_REQUIRE(pad_hp(last) > 0 || plan->mlp_sizes[i] <= kWideMaxH,
+               "a radial MLP with last hidden size > 64 supports layer sizes <= %d, got %d", kWideMaxH,
+               plan->mlp_sizes[i]);
+  }
   return MT_OK;
 }
+
+// last hidden size above 64: the radial MLP runs on its own (radial_mlp_kernel) into the workspace
+static bool wide_fwd(const mt_conv_plan* plan) { return pad_hp(plan->mlp_sizes[plan->mlp_num_layers - 1]) < 0; }
 
 template <typename T>
 static int conv_fwd_impl(const mt_conv_plan* plan, const void* x, const void* sh, const void* emb,
                          const void* const* mlp_weights, const int32_t* rowptr, const int32_t* perm,
-                         const int32_t* src_sorted, double avg, const void* num_neigh, void* out, int64_t N,
-                         int64_t E, cudaStream_t st) {
+                         const int32_t* src_sorted, double avg, const void* num_neigh, void* out, void* workspace,
+                         size_t workspace_bytes, int64_t N, int64_t E, cudaStream_t st) {
   ConvFwdParams p;
   memset(&p, 0, sizeof(p));
   p.x_dim = plan->x_dim;
@@ -57,8 +66,10 @@ static int conv_fwd_impl(const mt_conv_plan* plan, const void* x, const void* sh
     int h8 = (plan->mlp_sizes[i] + 7) / 8 * 8;
     if (h8 > hp_max) hp_max = h8;
   }
-  const int HP = pad_hp(p.sizes[p.nl - 1]);
+  const bool wide = wide_fwd(plan);
+  const int HP = wide ? 0 : pad_hp(p.sizes[p.nl - 1]);
   if (HP > hp_max) hp_max = HP;
+  if (wide) hp_max = 0;  // no hidden activations in shared memory: the weights come from p.wpe
   p.hp_max = hp_max;
   p.act = plan->mlp_act;
   p.act_cst = plan->mlp_act_cst;
@@ -67,6 +78,12 @@ static int conv_fwd_impl(const mt_conv_plan* plan, const void* x, const void* sh
   p.avg = avg; p.num_neigh = num_neigh; p.out = out;
   p.N = N; p.E = E;
   p.xs_stride = p.x_dim | 1;
+  if (wide) {
+    MT_REQUIRE(E == 0 || workspace != nullptr && workspace_bytes >= radial_mlp_out_bytes(plan, sizeof(T), E),
+               "conv_fwd workspace too small for the per-edge weights: %zu < %zu", workspace_bytes,
+               radial_mlp_out_bytes(plan, sizeof(T), E));
+    p.wpe = workspace;
+  }
 
   // chunk size from the shared-memory budget
   const size_t per_edge = (size_t)(2 * hp_max + p.xs_stride + p.y_dim) * sizeof(T);
@@ -82,7 +99,7 @@ static int conv_fwd_impl(const mt_conv_plan* plan, const void* x, const void* sh
   if (TN > 32) TN = 32;
   p.tile_nodes = TN;
   size_t hidden_w = 0;
-  for (int i = 0; i + 1 < p.nl; ++i) hidden_w += (size_t)p.sizes[i] * p.sizes[i + 1];
+  for (int i = 0; !wide && i + 1 < p.nl; ++i) hidden_w += (size_t)p.sizes[i] * p.sizes[i + 1];
   const size_t smem = (size_t)EC * per_edge + hidden_w * sizeof(T);
   MT_REQUIRE(smem <= 227 * 1024, "conv tile needs %zu bytes of shared memory", smem);
   // Resident warps per SM follow the number of contraction types the plan can touch (instruction-cache footprint: every
@@ -100,7 +117,21 @@ static int conv_fwd_impl(const mt_conv_plan* plan, const void* x, const void* sh
   int64_t grid = (int64_t)kNumSMs * ctas_per_sm;
   if (grid > tiles) grid = tiles;
   if (grid < 1) grid = 1;
+  if (wide) {
+    RadialMlpParams m;
+    memset(&m, 0, sizeof(m));
+    m.nl = p.nl;
+    for (int i = 0; i <= p.nl; ++i) m.sizes[i] = p.sizes[i];
+    for (int i = 0; i < p.nl; ++i) m.w[i] = p.w[i];
+    m.act = p.act; m.act_cst = p.act_cst;
+    m.emb = emb; m.perm = perm; m.E = E;
+    m.rows = radial_mlp_rows(plan);
+    m.out = workspace;
+    const int rc = launch_radial_mlp<T, false>(m, st);
+    if (rc != MT_OK) return rc;
+  }
   switch (HP) {
+    case 0: return launch_conv_fwd<T, 0>(p, (int)grid, threads, smem, st);
     case 8: return launch_conv_fwd<T, 8>(p, (int)grid, threads, smem, st);
     case 16: return launch_conv_fwd<T, 16>(p, (int)grid, threads, smem, st);
     case 32: return launch_conv_fwd<T, 32>(p, (int)grid, threads, smem, st);
@@ -124,6 +155,9 @@ int mt_conv_select_impl(int impl) {
 }
 
 size_t mt_conv_fwd_workspace_bytes(const mt_conv_plan* plan, int dtype, int64_t N, int64_t E) {
+  if (plan != nullptr && plan->mlp_num_layers >= 1 && plan->mlp_num_layers <= MT_MAX_MLP_LAYERS && wide_fwd(plan) &&
+      (dtype == MT_F32 || dtype == MT_F64) && E > 0)
+    return radial_mlp_out_bytes(plan, dtype == MT_F64 ? 8 : 4, E);
   if (plan == nullptr || dtype != MT_F32 || g_conv_impl == 2) return 0;
   return conv_fwd_tc_workspace_bytes(plan, N, E);
 }
@@ -158,7 +192,7 @@ int mt_conv_fwd(const mt_conv_plan* plan, int dtype, const void* x, const void* 
   }
   MT_DISPATCH_DTYPE(dtype, {
     return conv_fwd_impl<T>(plan, x, sh, emb, mlp_weights, rowptr, perm, src_sorted, avg_num_neighbors,
-                            num_neigh, out, N, E, as_stream(stream));
+                            num_neigh, out, workspace, workspace_bytes, N, E, as_stream(stream));
   });
   return MT_OK;
 }

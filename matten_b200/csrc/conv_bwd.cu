@@ -7,7 +7,15 @@ struct BwdLayout {
   size_t z_off[MT_MAX_MLP_LAYERS];
   size_t dw_off, dxe_off, dhp_off, partl_off, parth_off, total;
   int ncg, grid2, grid3, hid_numel, hid_eb, rs;
+  bool wide;                 // an input / hidden size above kBwdMaxH: the wide kernels
+  size_t wpe_off, da_off[2];  // wide: per-edge weights [E][Wn]; da of the hidden layers [E][<= 128], ping-pong
 };
+
+static bool wide_bwd(const mt_conv_plan* plan) {
+  for (int i = 0; i < plan->mlp_num_layers; ++i)
+    if (plan->mlp_sizes[i] > kBwdMaxH) return true;
+  return false;
+}
 
 static BwdLayout bwd_layout(const mt_conv_plan* plan, size_t es, int64_t E) {
   BwdLayout L;
@@ -22,8 +30,9 @@ static BwdLayout bwd_layout(const mt_conv_plan* plan, size_t es, int64_t E) {
     hid += plan->mlp_sizes[l] * plan->mlp_sizes[l + 1];
   }
   L.hid_numel = hid;
+  L.wide = wide_bwd(plan);
   L.ncg = ceil_div<int>(Wn, kLastCW);
-  const int64_t chunks2 = ceil_div<int64_t>(E, kLastEB);
+  const int64_t chunks2 = ceil_div<int64_t>(E, L.wide && H > kBwdMaxH ? kLastEBWide : kLastEB);
   L.grid2 = (int)(chunks2 < 2 * kNumSMs ? (chunks2 > 0 ? chunks2 : 1) : 2 * kNumSMs);
   int hmax = 1;
   for (int i = 0; i < nl; ++i) hmax = plan->mlp_sizes[i] > hmax ? plan->mlp_sizes[i] : hmax;
@@ -32,6 +41,11 @@ static BwdLayout bwd_layout(const mt_conv_plan* plan, size_t es, int64_t E) {
   while (L.hid_eb > 16 && ((size_t)3 * L.hid_eb * L.rs + (size_t)L.rs * L.rs + hid) * es > 36 * 1024) L.hid_eb >>= 1;
   const int64_t chunks3 = ceil_div<int64_t>(E, L.hid_eb);
   L.grid3 = (int)(chunks3 < 6 * kNumSMs ? (chunks3 > 0 ? chunks3 : 1) : 6 * kNumSMs);  // small tiles: 6 CTAs per SM
+  if (L.wide) {  // one CTA per SM in fp64 (W_l of 128 x 129 plus the tiles: ~200 KB), two in fp32
+    const int64_t chunks3w = ceil_div<int64_t>(E, kHidWideEB);
+    const int64_t cap = (int64_t)kNumSMs * (es == 4 ? 2 : 1);
+    L.grid3 = (int)(chunks3w < cap ? (chunks3w > 0 ? chunks3w : 1) : cap);
+  }
   L.dw_off = o;
   o += align256((size_t)E * Wn * es);
   L.dxe_off = o;
@@ -45,6 +59,14 @@ static BwdLayout bwd_layout(const mt_conv_plan* plan, size_t es, int64_t E) {
     const size_t rows = (size_t)L.grid3 > (size_t)kHidFastCtas * kHidFastWarps ? (size_t)L.grid3
                                                                                : (size_t)kHidFastCtas * kHidFastWarps;
     o += align256(rows * (hid > 0 ? hid : 1) * es);
+  }
+  if (L.wide) {
+    L.wpe_off = o;
+    o += radial_mlp_out_bytes(plan, es, E);
+    for (int i = 0; i < 2 && nl > 2; ++i) {
+      L.da_off[i] = o;
+      o += align256((size_t)E * hmax * es);
+    }
   }
   L.total = o;
   return L;
@@ -60,15 +82,63 @@ static int launch_last(const ConvBwdParams& p, cudaStream_t st) {
   return MT_OK;
 }
 
+template <typename T>
+static int launch_last_wide(const ConvBwdParams& p, cudaStream_t st) {
+  const size_t smem = ((size_t)kLastEBWide * (kLastCW + 4) + (size_t)kLastEBWide * kWideMaxH +
+                       (size_t)kLastCW * kWideMaxH) * sizeof(T);
+  MT_CUDA_OK(cudaFuncSetAttribute(mlp_bwd_last_wide_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  dim3 grid(p.grid2, p.ncg);
+  mlp_bwd_last_wide_kernel<T><<<grid, 256, smem, st>>>(p);
+  MT_LAUNCH_OK();
+  return MT_OK;
+}
+
+// wide K3: one launch per hidden layer, from the last down, then the fixed-order sums of the per-CTA partials
+template <typename T>
+static int launch_hidden_wide(const ConvBwdParams& p, const BwdLayout& L, unsigned char* ws, void* const* grad_w,
+                              bool emb, cudaStream_t st) {
+  int woff = p.hid_numel;
+  const T* da_in = static_cast<const T*>(p.DHP);
+  int parts = p.ncg;
+  for (int l = p.nl - 2; l >= 0; --l) {
+    const int fi = p.sizes[l], fo = p.sizes[l + 1];
+    woff -= fi * fo;
+    T* da_out = l > 0 ? reinterpret_cast<T*>(ws + L.da_off[l & 1]) : nullptr;
+    const size_t smem = ((size_t)2 * kHidWideEB * kHidWideRS + (size_t)fi * (fo + 1)) * sizeof(T);
+    if (l == 0 && emb) {
+      MT_CUDA_OK(cudaFuncSetAttribute(mlp_bwd_hidden_wide_kernel<T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)smem));
+      mlp_bwd_hidden_wide_kernel<T, true><<<p.grid3, 256, smem, st>>>(p, l, da_in, parts, da_out, woff);
+    } else {
+      MT_CUDA_OK(cudaFuncSetAttribute(mlp_bwd_hidden_wide_kernel<T, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)smem));
+      mlp_bwd_hidden_wide_kernel<T, false><<<p.grid3, 256, smem, st>>>(p, l, da_in, parts, da_out, woff);
+    }
+    MT_LAUNCH_OK();
+    da_in = da_out;
+    parts = 1;
+  }
+  int64_t off = 0;
+  for (int l = 0; grad_w && l + 1 < p.nl; ++l) {
+    const int64_t cnt = (int64_t)p.sizes[l] * p.sizes[l + 1];
+    reduce_partials_kernel<T><<<(unsigned)ceil_div<int64_t>(cnt, 32), 256, 0, st>>>(
+        static_cast<const T*>(p.PARTH), p.hid_numel, p.grid3, off, cnt, T(1) / sqrt(T(p.sizes[l])),
+        static_cast<T*>(grad_w[l]));
+    MT_LAUNCH_OK();
+    off += cnt;
+  }
+  return MT_OK;
+}
+
 // K1: tile geometry from the shared-memory budget (two CTAs per SM when possible)
-template <typename T, bool EG>
+template <typename T, bool EG, bool WIDE>
 static int launch_conv_bwd_k1(ConvBwdParams& p, int64_t N, int64_t E, cudaStream_t st) {
   const double avg_deg = N > 0 ? (double)E / (double)N : 1.0;
   const size_t fixed = (size_t)p.num_paths * 16;
   // resident CTAs per SM the register budget allows (launch bounds of conv_bwd_kernel) -> shared-memory budget per CTA:
   // the kernel alternates staging / GEMM / contraction phases between barriers, so more small CTAs hide more of it
   const int threads1 = 128;  // more, smaller CTAs hide the phase barriers better (r1 sweep)
-  const int per_sm_regs = (sizeof(T) == 4 ? 3 : 2) * (256 / threads1);
+  const int per_sm_regs = (sizeof(T) == 4 ? 3 : 2) * (256 / threads1) - (WIDE ? 256 / threads1 : 0);
   const size_t budget = (size_t)(227 * 1024) / per_sm_regs - 1024;
   // EG: one sh-gradient partial row per (item, staged edge)
   const size_t per_edge_eg = EG ? (size_t)p.num_items * p.y_dim : 0;
@@ -91,8 +161,9 @@ static int launch_conv_bwd_k1(ConvBwdParams& p, int64_t N, int64_t E, cudaStream
   p.chunk_edges = EC;
   p.tile_nodes = TN;
   static thread_local size_t cfg1 = 0;
+  const auto kernel = WIDE ? conv_bwd_wide_kernel<T, EG> : conv_bwd_kernel<T, EG>;
   if (smem > cfg1) {
-    MT_CUDA_OK(cudaFuncSetAttribute(conv_bwd_kernel<T, EG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    MT_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cfg1 = smem;
   }
   const int64_t tiles = ceil_div<int64_t>(N, TN);
@@ -101,7 +172,7 @@ static int launch_conv_bwd_k1(ConvBwdParams& p, int64_t N, int64_t E, cudaStream
   if (per_sm < 1) per_sm = 1;
   int64_t grid = (int64_t)kNumSMs * per_sm;
   if (grid > tiles) grid = tiles;
-  conv_bwd_kernel<T, EG><<<(int)grid, threads1, smem, st>>>(p);
+  kernel<<<(int)grid, threads1, smem, st>>>(p);
   MT_LAUNCH_OK();
   return MT_OK;
 }
@@ -143,18 +214,32 @@ static int conv_bwd_impl(const mt_conv_plan* plan, const void* x, const void* sh
   p.N = N; p.E = E;
   p.ncg = L.ncg; p.grid2 = L.grid2; p.grid3 = L.grid3; p.hid_numel = L.hid_numel;
   p.xs_stride = p.x_dim | 1;
-  p.hs_stride = (H + 3) / 4 * 4;
+  p.hs_stride = L.wide ? 0 : (H + 3) / 4 * 4;  // the wide K1 stages no last-layer input
   p.wt_stride = Wn;
   p.rs = L.rs;
   p.hid_eb = L.hid_eb;
   p.gsh = grad_sh;
   p.gemb = grad_emb;
+  if (L.wide) p.wpe = ws + L.wpe_off;
 
   // the MLP shape of the matten configs in fp32 takes the lane-per-edge kernels
   const bool fast_mlp = sizeof(T) == 4 && nl == 3 && p.sizes[0] <= 8 && p.sizes[1] == 32 && p.sizes[2] == 32 &&
                         p.act == MT_ACT_SILU;
-  // K0: hidden pre-activations
-  if (fast_mlp) {
+  // K0: hidden pre-activations (wide: and the per-edge weights)
+  if (L.wide) {
+    RadialMlpParams m;
+    memset(&m, 0, sizeof(m));
+    m.nl = nl;
+    for (int i = 0; i <= nl; ++i) m.sizes[i] = p.sizes[i];
+    for (int i = 0; i < nl; ++i) m.w[i] = p.w[i];
+    for (int i = 0; i + 1 < nl; ++i) m.z[i] = p.z[i];
+    m.act = p.act; m.act_cst = p.act_cst;
+    m.emb = emb; m.perm = perm; m.E = E;
+    m.rows = radial_mlp_rows(plan);
+    m.out = ws + L.wpe_off;
+    const int rc = launch_radial_mlp<T, true>(m, st);
+    if (rc != MT_OK) return rc;
+  } else if (fast_mlp) {
     int64_t g0 = ceil_div<int64_t>(E, 256);
     if (g0 > (int64_t)kNumSMs * 8) g0 = (int64_t)kNumSMs * 8;
     edge_hidden_fast_kernel<<<(unsigned)g0, 256, 0, st>>>(p);
@@ -172,7 +257,10 @@ static int conv_bwd_impl(const mt_conv_plan* plan, const void* x, const void* sh
     MT_LAUNCH_OK();
   }
   {
-    const int rc = grad_sh ? launch_conv_bwd_k1<T, true>(p, N, E, st) : launch_conv_bwd_k1<T, false>(p, N, E, st);
+    const int rc = L.wide ? (grad_sh ? launch_conv_bwd_k1<T, true, true>(p, N, E, st)
+                                     : launch_conv_bwd_k1<T, false, true>(p, N, E, st))
+                          : (grad_sh ? launch_conv_bwd_k1<T, true, false>(p, N, E, st)
+                                     : launch_conv_bwd_k1<T, false, false>(p, N, E, st));
     if (rc != MT_OK) return rc;
   }
   // per-sender sum of the per-edge input gradients
@@ -183,7 +271,8 @@ static int conv_bwd_impl(const mt_conv_plan* plan, const void* x, const void* sh
   // K2 / K3 give the weight gradients and, through da of the first layer, the embedding gradient
   if (grad_w || grad_emb) {
     int rc = MT_OK;
-    switch (pad_hp(H)) {
+    if (H > kBwdMaxH) rc = launch_last_wide<T>(p, st);
+    else switch (pad_hp(H)) {
       case 8: rc = launch_last<T, 8>(p, st); break;
       case 16: rc = launch_last<T, 16>(p, st); break;
       case 32: rc = launch_last<T, 32>(p, st); break;
@@ -203,6 +292,9 @@ static int conv_bwd_impl(const mt_conv_plan* plan, const void* x, const void* sh
         emb_grad_last_kernel<T><<<(unsigned)ge, 256, 0, st>>>(p);
         MT_LAUNCH_OK();
       }
+    } else if (L.wide) {
+      rc = launch_hidden_wide<T>(p, L, ws, grad_w, grad_emb != nullptr, st);
+      if (rc != MT_OK) return rc;
     } else if (fast_mlp) {
       int64_t gf = ceil_div<int64_t>(ceil_div<int64_t>(E, 32), kHidFastWarps);
       if (gf > kHidFastCtas) gf = kHidFastCtas;
@@ -278,8 +370,8 @@ int mt_conv_bwd_full(const mt_conv_plan* plan, int dtype, const void* x, const v
              "plan has no backward tables");
   MT_REQUIRE(plan->mlp_num_layers >= 1 && plan->mlp_num_layers <= MT_MAX_MLP_LAYERS, "bad mlp_num_layers");
   for (int i = 0; i < plan->mlp_num_layers; ++i)
-    MT_REQUIRE(plan->mlp_sizes[i] > 0 && plan->mlp_sizes[i] <= kBwdMaxH,
-               "conv_bwd supports MLP input/hidden sizes <= %d, got %d", kBwdMaxH, plan->mlp_sizes[i]);
+    MT_REQUIRE(plan->mlp_sizes[i] > 0 && plan->mlp_sizes[i] <= kWideMaxH,
+               "conv_bwd supports MLP input/hidden sizes <= %d, got %d", kWideMaxH, plan->mlp_sizes[i]);
   MT_REQUIRE(N >= 0 && E >= 0, "negative size");
   if (N == 0) return MT_OK;
   MT_REQUIRE(x && rowptr && mlp_weights && grad_out, "null pointer");

@@ -24,17 +24,28 @@
 //             (item, staged edge) in shared memory; after phase B the rows are summed over the items in item order.
 //   grad_emb  dz0 W0^T / sqrt(fan_in) in K3 (both forms), or the column-group sum of K2's da_last for a one-layer MLP.
 // Both are written through perm (a permutation) in the caller's edge order.
+//
+// MLPs with an input or hidden size in (64, 128] ("wide", up to kWideMaxH) take separate kernels, so that the ones above
+// keep their code:
+//   K0 radial_mlp_kernel<T, true> (radial_mlp.cuh)   z_l and the per-edge weights w [E][Wn] into the workspace
+//   K1 conv_bwd_wide_kernel                          phase A copies the staged edges' w rows instead of a_last W_last
+//   K2 mlp_bwd_last_wide_kernel                      K2 with 32-edge chunks for H in (64, 128] (fits fp64 in 227 KB)
+//   K3 mlp_bwd_hidden_wide_kernel                    one launch per hidden layer, one layer's weights resident
 #pragma once
 #include "common.cuh"
 #include "generated/cg_gen.cuh"
+#include "radial_mlp.cuh"
 
 namespace mt {
 
-constexpr int kBwdMaxH = 64;     // largest MLP layer input/hidden size the backward supports
+constexpr int kBwdMaxH = 64;     // largest MLP layer input/hidden size of the kernels above; up to kWideMaxH: wide path
 constexpr int kBwdET = 8;        // edges per register pass of phase A (chunk_edges is a multiple of it)
 constexpr int kLastEB = 64;      // edges per chunk of K2
 constexpr int kLastCW = 128;     // weight columns per CTA column group of K2
 constexpr int kHidEBMax = 64;    // edges per chunk of K0 / K3 (halved until the tiles fit: ConvBwdParams::hid_eb)
+constexpr int kLastEBWide = 32;  // edges per chunk of the wide K2
+constexpr int kHidWideEB = 32;   // edges per chunk of the wide K3
+constexpr int kHidWideRS = kWideMaxH + 4;  // row stride of the wide K3's [edge][k] tiles (16-byte aligned rows)
 
 struct ConvBwdParams {
   int x_dim, y_dim, out_dim, Wn;
@@ -69,6 +80,7 @@ struct ConvBwdParams {
   int rs;  // row stride of the per-edge activation tiles of K0 / K3: largest input / hidden size + 1
   void* gsh;   // [E][y_dim] gradient w.r.t. sh (original edge order), written by conv_bwd_kernel<T, true>
   void* gemb;  // [E][sizes[0]] gradient w.r.t. the edge embedding (original edge order)
+  const void* wpe;  // wide path: per-edge weights [E][Wn] (receiver-sorted order), written by K0
 };
 
 template <typename T>
@@ -260,8 +272,9 @@ __device__ __forceinline__ void bwd_unit(const ConvBwdParams& p, const int4* __r
   }
 }
 
-template <typename T, bool EG>
-__global__ void __launch_bounds__(256, sizeof(T) == 4 ? 3 : 2) conv_bwd_kernel(const ConvBwdParams p) {
+// WIDE: phase A copies the per-edge weights from p.wpe (hs_stride is 0: no staged last-layer input)
+template <typename T, bool EG, bool WIDE>
+__device__ __forceinline__ void conv_bwd_body(const ConvBwdParams& p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int EC = p.chunk_edges;
   int4* spath = reinterpret_cast<int4*>(smem_raw);     // [num_paths]
@@ -315,7 +328,7 @@ __global__ void __launch_bounds__(256, sizeof(T) == 4 ? 3 : 2) conv_bwd_kernel(c
         ys[t] = SH[(size_t)p.perm[c0 + el] * p.y_dim + j];
       }
       // a_last / sqrt(H), TRANSPOSED [k][EC] so that the 8 edges of a register pass are one 128-bit broadcast load
-      for (int t = tid; t < EC * H; t += blockDim.x) {
+      for (int t = tid; !WIDE && t < EC * H; t += blockDim.x) {
         const int k = t / EC, el = t - k * EC;  // lanes walk the edges: conflict-free stores
         hs[(size_t)k * EC + el] = (el < ne) ? last_input<T>(p, (int64_t)c0 + el, k) * inv_sqrt_h : T(0);
       }
@@ -329,8 +342,15 @@ __global__ void __launch_bounds__(256, sizeof(T) == 4 ? 3 : 2) conv_bwd_kernel(c
       if (tid == 0) s_counter = 0;
       __syncthreads();
       // ------------------------------------------------------------ (A) per-edge weights into shared memory
+      if constexpr (WIDE) {
+        const T* __restrict__ WPE = static_cast<const T*>(p.wpe) + (size_t)c0 * Wn;
+        for (int t = tid; t < ne * Wn; t += blockDim.x) {
+          const int el = t / Wn, c = t - el * Wn;
+          wt[(size_t)el * p.wt_stride + c] = WPE[t];
+        }
+      }
       // register tile: 8 edges x 2 columns (c, c + blockDim) per thread
-      for (int ep = 0; ep < ne; ep += kBwdET) {
+      for (int ep = 0; !WIDE && ep < ne; ep += kBwdET) {
         for (int c = tid; c < Wn; c += 2 * blockDim.x) {
           const int c2 = c + blockDim.x;
           const bool two = c2 < Wn;
@@ -401,6 +421,17 @@ __global__ void __launch_bounds__(256, sizeof(T) == 4 ? 3 : 2) conv_bwd_kernel(c
   }
 }
 
+template <typename T, bool EG>
+__global__ void __launch_bounds__(256, sizeof(T) == 4 ? 3 : 2) conv_bwd_kernel(const ConvBwdParams p) {
+  conv_bwd_body<T, EG, false>(p);
+}
+
+// one CTA fewer per SM than conv_bwd_kernel: at that register budget this body spills
+template <typename T, bool EG>
+__global__ void __launch_bounds__(256, sizeof(T) == 4 ? 2 : 1) conv_bwd_wide_kernel(const ConvBwdParams p) {
+  conv_bwd_body<T, EG, true>(p);
+}
+
 // ---------------------------------------------------------------------------------------------- K2
 // grid (grid2, ncg): CTA (bx, cg) walks edge chunks bx, bx + grid2, ... for the weight columns of group cg.
 template <typename T, int HP>
@@ -449,6 +480,100 @@ __global__ void __launch_bounds__(256) mlp_bwd_last_kernel(const ConvBwdParams p
     // dW_last[k][c] += sum_e a[e][k] dw[e][c]
     if (tk < HP) {
       for (int el = 0; el < kLastEB; ++el) {
+        const T* dr = dws + el * DS + tc * 4;
+        const T d0 = dr[0], d1 = dr[1], d2 = dr[2], d3 = dr[3];
+#pragma unroll
+        for (int i = 0; i < KP; ++i) {
+          const T hv = hs2[el * HP + tk + 8 * i];
+          fma_pair(hv, d0, d1, accw[i][0]);
+          fma_pair(hv, d2, d3, accw[i][1]);
+        }
+      }
+    }
+    // dH[e][k] (this column group) = sum_c dw[e][c] W[k][c] / sqrt(H)
+    {
+      P acch[KD / 2];
+#pragma unroll
+      for (int i = 0; i < KD / 2; ++i) acch[i].x = acch[i].y = T(0);
+      const T* dr = dws + te * DS;
+      for (int c = 0; c < kLastCW; ++c) {
+        const T dv = dr[c];
+        const T* wr = WlT + c * HP + kq * KD;
+#pragma unroll
+        for (int i = 0; i < KD / 2; ++i) fma_pair(dv, wr[2 * i], wr[2 * i + 1], acch[i]);
+      }
+      if (te < ne) {
+        T* dh = static_cast<T*>(p.DHP) + ((size_t)cg * p.E + (e0 + te)) * H;
+#pragma unroll
+        for (int i = 0; i < KD; ++i)
+          if (kq * KD + i < H) dh[kq * KD + i] = (i & 1) ? acch[i >> 1].y : acch[i >> 1].x;
+      }
+    }
+  }
+  // partial dW_last of this CTA: PARTL[bx][k][c]
+  T* part = static_cast<T*>(p.PARTL) + (size_t)blockIdx.x * H * Wn;
+#pragma unroll
+  for (int i = 0; i < KP; ++i) {
+    const int k = tk + 8 * i;
+    if (k < H) {
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const int c = tc * 4 + j;
+        if (c < ncol) part[(size_t)k * Wn + cbase + c] = (j & 1) ? accw[i][j >> 1].y : accw[i][j >> 1].x;
+      }
+    }
+  }
+}
+
+// K2 for H in (64, 128]: mlp_bwd_last_kernel<T, 128> with chunks of kLastEBWideWide = 32 edges, so that fp64 fits in
+// shared memory (193 KB instead of 264 KB); 8 threads per edge in the dH tile.
+template <typename T>
+__global__ void __launch_bounds__(256) mlp_bwd_last_wide_kernel(const ConvBwdParams p) {
+  constexpr int HP = kWideMaxH;
+  constexpr int KP = HP / 8 > 0 ? HP / 8 : 1;  // k per thread of the dW tile (k = tk + 8 i)
+  constexpr int KD = HP / 8;                   // k per thread of the dH tile
+  constexpr int DS = kLastCW + 4;              // row stride of the dw tile
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  T* dws = reinterpret_cast<T*>(smem_raw);             // [kLastEBWide][DS]
+  T* hs2 = dws + (size_t)kLastEBWide * DS;                 // [kLastEBWide][HP]
+  T* WlT = hs2 + (size_t)kLastEBWide * HP;                 // [kLastCW][HP]  (pre-scaled by 1/sqrt(H))
+  const int tid = threadIdx.x;
+  const int H = p.sizes[p.nl - 1], Wn = p.Wn;
+  const int cg = blockIdx.y;
+  const int cbase = cg * kLastCW;
+  const int ncol = min(kLastCW, Wn - cbase);
+  const T inv_sqrt_h = T(1) / sqrt(T(H));
+  const T* __restrict__ Wlast = static_cast<const T*>(p.w[p.nl - 1]);
+  const T* __restrict__ DW = static_cast<const T*>(p.DW);
+  for (int t = tid; t < kLastCW * HP; t += blockDim.x) {
+    const int c = t / HP, k = t - c * HP;
+    WlT[t] = (c < ncol && k < H) ? Wlast[(size_t)k * Wn + cbase + c] * inv_sqrt_h : T(0);
+  }
+  const int tc = tid & 31, tk = tid >> 5;   // dW tile: columns 4 tc .. 4 tc + 3, k = tk + 8 i
+  const int te = tid >> 3, kq = tid & 7;    // dH tile: edge te, k = kq * KD .. + KD - 1
+  using P = typename pair_of<T>::type;  // pairs of columns / of k: one FFMA2 per pair in fp32
+  P accw[KP][2];
+#pragma unroll
+  for (int i = 0; i < KP; ++i)
+#pragma unroll
+    for (int j = 0; j < 2; ++j) accw[i][j].x = accw[i][j].y = T(0);
+  const int64_t nchunks = ceil_div<int64_t>(p.E, kLastEBWide);
+  for (int64_t ch = blockIdx.x; ch < nchunks; ch += gridDim.x) {
+    const int64_t e0 = ch * kLastEBWide;
+    const int ne = (int)imin64(kLastEBWide, p.E - e0);
+    __syncthreads();
+    for (int t = tid; t < kLastEBWide * kLastCW; t += blockDim.x) {
+      const int el = t / kLastCW, c = t - el * kLastCW;
+      dws[el * DS + c] = (el < ne && c < ncol) ? DW[(size_t)(e0 + el) * Wn + cbase + c] : T(0);
+    }
+    for (int t = tid; t < kLastEBWide * HP; t += blockDim.x) {
+      const int el = t / HP, k = t - el * HP;
+      hs2[t] = (el < ne && k < H) ? last_input<T>(p, e0 + el, k) : T(0);
+    }
+    __syncthreads();
+    // dW_last[k][c] += sum_e a[e][k] dw[e][c]
+    if (tk < HP) {
+      for (int el = 0; el < kLastEBWide; ++el) {
         const T* dr = dws + el * DS + tc * 4;
         const T d0 = dr[0], d1 = dr[1], d2 = dr[2], d3 = dr[3];
 #pragma unroll
@@ -790,6 +915,132 @@ __global__ void __launch_bounds__(256) emb_grad_last_kernel(const ConvBwdParams 
     T s = T(0);
     for (int cg = 0; cg < p.ncg; ++cg) s += DHP[((size_t)cg * p.E + e) * H + k];
     static_cast<T*>(p.gemb)[(size_t)p.perm[e] * H + k] = s;
+  }
+}
+
+// ---------------------------------------------------------------------------------------------- K3, wide form
+// One launch per hidden layer l (fi -> fo, both <= kWideMaxH), from the last hidden layer down.  CTA <-> chunks of
+// kHidWideEB edges bx, bx + grid, ...:
+//   dz[e][j] = da[e][j] act'(z_l[e][j]) cst       da: sum of the `da_parts` slices [part][E][fo] of da_in, in order
+//   dW_l[k][j] += sum_e a_l[e][k] dz[e][j]         thread <-> 8 x 8 block of dW_l, in registers over all chunks
+//   da_l[e][k] = sum_j dz[e][j] W_l[k][j] / sqrt(fi)  -> da_out [E][fi] (l > 0), or grad_emb through perm (l == 0, EMB)
+// Only W_l is resident.  The CTA's dW_l block goes to PARTH[bx][woff + k fo + j] (the generic K3's layout), summed in
+// fixed order by reduce_partials_kernel.
+template <typename T, bool EMB>
+__global__ void __launch_bounds__(256) mlp_bwd_hidden_wide_kernel(const ConvBwdParams p, int l,
+                                                                  const T* __restrict__ da_in, int da_parts,
+                                                                  T* __restrict__ da_out, int woff) {
+  constexpr int EB = kHidWideEB, RS = kHidWideRS;
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int fi = p.sizes[l], fo = p.sizes[l + 1];
+  const int WS = fo + 1;                     // row stride of W_l: lanes walk k, conflict free
+  T* DZ = reinterpret_cast<T*>(smem_raw);    // [EB][RS]
+  T* A = DZ + (size_t)EB * RS;               // [EB][RS]  the layer's input activation
+  T* Wl = A + (size_t)EB * RS;               // [fi][WS]  pre-scaled by 1/sqrt(fi)
+  const int tid = threadIdx.x;
+  const T cst = T(p.act_cst);
+  {
+    const T s = T(1) / sqrt(T(fi));
+    const T* __restrict__ Wg = static_cast<const T*>(p.w[l]);
+    for (int t = tid; t < fi * fo; t += blockDim.x) Wl[(t / fo) * WS + (t % fo)] = Wg[t] * s;
+  }
+  // dW tile: rows 8 tk .. 8 tk + 7, columns 8 tj .. 8 tj + 7
+  const int tk = tid >> 4, tj = tid & 15;
+  const bool wactive = tk * 8 < fi && tj * 8 < fo;
+  using P = typename pair_of<T>::type;
+  P gw[8][4];
+#pragma unroll
+  for (int a = 0; a < 8; ++a)
+#pragma unroll
+    for (int b = 0; b < 4; ++b) gw[a][b].x = gw[a][b].y = T(0);
+  // da tile: edges te + 8 a, k = tq + 32 b
+  const int te = tid >> 5, tq = tid & 31;
+  const T* __restrict__ Z = static_cast<const T*>(p.z[l]);
+  const int64_t nchunks = ceil_div<int64_t>(p.E, EB);
+  for (int64_t ch = blockIdx.x; ch < nchunks; ch += gridDim.x) {
+    const int64_t e0 = ch * EB;
+    const int ne = (int)imin64(EB, p.E - e0);
+    __syncthreads();  // W_l staged / the previous chunk consumed
+    for (int t = tid; t < EB * fo; t += blockDim.x) {
+      const int el = t / fo, j = t - el * fo;
+      T v = T(0);
+      if (el < ne) {
+        T s = T(0);
+        for (int q = 0; q < da_parts; ++q) s += da_in[((size_t)q * p.E + (e0 + el)) * fo + j];
+        v = s * apply_act_grad<T>(p.act, Z[(size_t)(e0 + el) * fo + j]) * cst;
+      }
+      DZ[el * RS + j] = v;
+    }
+    for (int t = tid; t < EB * fi; t += blockDim.x) {
+      const int el = t / fi, k = t - el * fi;
+      T v = T(0);
+      if (el < ne) {
+        if (l == 0) v = static_cast<const T*>(p.emb)[(size_t)p.perm[e0 + el] * fi + k];
+        else v = apply_act<T>(p.act, static_cast<const T*>(p.z[l - 1])[(size_t)(e0 + el) * fi + k]) * cst;
+      }
+      A[el * RS + k] = v;
+    }
+    __syncthreads();
+    if (wactive) {
+      for (int el = 0; el < EB; ++el) {
+        T a0[4], a1[4], d0[4], d1[4];
+        mlp_load4<T>(A + el * RS + tk * 8, a0);
+        mlp_load4<T>(A + el * RS + tk * 8 + 4, a1);
+        mlp_load4<T>(DZ + el * RS + tj * 8, d0);
+        mlp_load4<T>(DZ + el * RS + tj * 8 + 4, d1);
+#pragma unroll
+        for (int a = 0; a < 8; ++a) {
+          const T av = a < 4 ? a0[a & 3] : a1[a & 3];
+          fma_pair(av, d0[0], d0[1], gw[a][0]);
+          fma_pair(av, d0[2], d0[3], gw[a][1]);
+          fma_pair(av, d1[0], d1[1], gw[a][2]);
+          fma_pair(av, d1[2], d1[3], gw[a][3]);
+        }
+      }
+    }
+    if (l > 0 || EMB) {
+      T acc[4][4];
+#pragma unroll
+      for (int a = 0; a < 4; ++a)
+#pragma unroll
+        for (int b = 0; b < 4; ++b) acc[a][b] = T(0);
+      for (int j = 0; j < fo; ++j) {
+        T dz[4], wv[4];
+#pragma unroll
+        for (int a = 0; a < 4; ++a) dz[a] = DZ[(te + 8 * a) * RS + j];
+#pragma unroll
+        for (int b = 0; b < 4; ++b) wv[b] = tq + 32 * b < fi ? Wl[(tq + 32 * b) * WS + j] : T(0);
+#pragma unroll
+        for (int a = 0; a < 4; ++a)
+#pragma unroll
+          for (int b = 0; b < 4; ++b) acc[a][b] = fma(dz[a], wv[b], acc[a][b]);
+      }
+#pragma unroll
+      for (int a = 0; a < 4; ++a) {
+        const int el = te + 8 * a;
+        if (el >= ne) continue;
+#pragma unroll
+        for (int b = 0; b < 4; ++b) {
+          const int k = tq + 32 * b;
+          if (k >= fi) continue;
+          if (l > 0) da_out[(size_t)(e0 + el) * fi + k] = acc[a][b];
+          else static_cast<T*>(p.gemb)[(size_t)p.perm[e0 + el] * fi + k] = acc[a][b];
+        }
+      }
+    }
+  }
+  T* part = static_cast<T*>(p.PARTH) + (size_t)blockIdx.x * p.hid_numel + woff;
+  if (wactive) {
+#pragma unroll
+    for (int a = 0; a < 8; ++a) {
+      const int k = tk * 8 + a;
+      if (k >= fi) continue;
+#pragma unroll
+      for (int b = 0; b < 8; ++b) {
+        const int j = tj * 8 + b;
+        if (j < fo) part[(size_t)k * fo + j] = (b & 1) ? gw[a][b >> 1].y : gw[a][b >> 1].x;
+      }
+    }
   }
 }
 

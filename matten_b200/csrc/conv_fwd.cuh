@@ -20,6 +20,9 @@
 //   The per-node sum is a register accumulation in CSR order: deterministic, no atomics.
 //   Types with fewer than 32 columns split the node's edges over lane groups
 //   ("phases") and finish with a fixed-order shuffle reduction.
+// HP == 0 is the variant for radial MLPs wider than 64 (radial_mlp.cuh): the per-edge weights are read from
+// ConvFwdParams::wpe [E][Wn] (lanes hold consecutive columns: coalesced) instead of being formed from the staged
+// hidden activations; there is no embedding staging and no hidden layer.
 #pragma once
 #include "common.cuh"
 #include "generated/cg_gen.cuh"
@@ -49,6 +52,7 @@ struct ConvFwdParams {
   int chunk_edges;  // EC
   int xs_stride;    // smem row stride of staged x rows
   int hp_max;       // smem row stride of the hidden-activation buffers
+  const void* wpe;  // HP == 0: per-edge weights [E][sizes[nl]], receiver-sorted order
 };
 
 template <typename T>
@@ -66,8 +70,9 @@ __device__ __forceinline__ void load4<double>(const double* p, double (&v)[4]) {
 }
 
 // One warp, one item, one node: walk the node's staged edges [el0, el1).
+// HP == 0: hs points at the lane's column of the chunk's first per-edge weight row, hstride = Wn.
 template <typename T, int HP, int L1, int L2, int L3>
-__device__ __forceinline__ void conv_unit(const T (&wreg)[HP], const T* __restrict__ hs, int hstride,
+__device__ __forceinline__ void conv_unit(const T (&wreg)[HP > 0 ? HP : 1], const T* __restrict__ hs, int hstride,
                                           const T* __restrict__ xs, int xstride,
                                           const T* __restrict__ ys, int ystride, int xoff, int yoff,
                                           int el0, int el1, int phase, int nphase, int cpw,
@@ -77,23 +82,28 @@ __device__ __forceinline__ void conv_unit(const T (&wreg)[HP], const T* __restri
 #pragma unroll
   for (int m = 0; m < D3; ++m) acc[m] = T(0);
   for (int el = el0 + phase; el < el1; el += nphase) {
-    const T* h = hs + (size_t)el * hstride;
-    T w0 = T(0), w1 = T(0);
+    T w;
+    if constexpr (HP == 0) {
+      w = hs[(size_t)el * hstride];
+    } else {
+      const T* h = hs + (size_t)el * hstride;
+      T w0 = T(0), w1 = T(0);
 #pragma unroll
-    for (int k = 0; k < HP; k += 8) {
-      T a[4], b[4];
-      load4<T>(h + k, a);
-      load4<T>(h + k + 4, b);
-      w0 = fma(a[0], wreg[k + 0], w0);
-      w1 = fma(b[0], wreg[k + 4], w1);
-      w0 = fma(a[1], wreg[k + 1], w0);
-      w1 = fma(b[1], wreg[k + 5], w1);
-      w0 = fma(a[2], wreg[k + 2], w0);
-      w1 = fma(b[2], wreg[k + 6], w1);
-      w0 = fma(a[3], wreg[k + 3], w0);
-      w1 = fma(b[3], wreg[k + 7], w1);
+      for (int k = 0; k < HP; k += 8) {
+        T a[4], b[4];
+        load4<T>(h + k, a);
+        load4<T>(h + k + 4, b);
+        w0 = fma(a[0], wreg[k + 0], w0);
+        w1 = fma(b[0], wreg[k + 4], w1);
+        w0 = fma(a[1], wreg[k + 1], w0);
+        w1 = fma(b[1], wreg[k + 5], w1);
+        w0 = fma(a[2], wreg[k + 2], w0);
+        w1 = fma(b[2], wreg[k + 6], w1);
+        w0 = fma(a[3], wreg[k + 3], w0);
+        w1 = fma(b[3], wreg[k + 7], w1);
+      }
+      w = w0 + w1;
     }
-    const T w = w0 + w1;
     T xv[D1], yv[D2];
     const T* xr = xs + (size_t)el * xstride + xoff;
 #pragma unroll
@@ -144,7 +154,7 @@ __global__ void __launch_bounds__(256, (conv_fwd_min_blocks<T, HP>())) conv_fwd_
   const int Wn = p.sizes[p.nl];
   const T inv_sqrt_h = T(1) / sqrt(T(H_last));
 
-  {
+  if constexpr (HP > 0) {
     int off = 0;
     for (int li = 0; li + 1 < p.nl; ++li) {
       const int fi = p.sizes[li], fo = p.sizes[li + 1];
@@ -176,7 +186,7 @@ __global__ void __launch_bounds__(256, (conv_fwd_min_blocks<T, HP>())) conv_fwd_
         int el = t / p.y_dim, j = t - el * p.y_dim;
         ys[t] = SH[(size_t)p.perm[c0 + el] * p.y_dim + j];
       }
-      {
+      if constexpr (HP > 0) {
         const int in0 = p.sizes[0];
         for (int t = tid; t < ne * p.hp_max; t += blockDim.x) {
           int el = t / p.hp_max, j = t - el * p.hp_max;
@@ -189,7 +199,7 @@ __global__ void __launch_bounds__(256, (conv_fwd_min_blocks<T, HP>())) conv_fwd_
       T* hin = ha;
       T* hout = hb;
       int woff = 0;
-      for (int li = 0; li + 1 < p.nl; ++li) {
+      for (int li = 0; HP > 0 && li + 1 < p.nl; ++li) {
         const int fi = p.sizes[li], fo = p.sizes[li + 1];
         const T* Wl = wh + woff;
         woff += fi * fo;
@@ -225,7 +235,7 @@ __global__ void __launch_bounds__(256, (conv_fwd_min_blocks<T, HP>())) conv_fwd_
         const int4 slot = reinterpret_cast<const int4*>(p.slot_tab)[item * 32 + lane];
         const int wcol = slot.x, xoff = slot.y, yoff = slot.z, ooff = slot.w;
         const int phase = lane / cpw, nphase = 32 / cpw;
-        T wreg[HP];
+        T wreg[HP > 0 ? HP : 1];
 #pragma unroll
         for (int k = 0; k < HP; ++k)
           wreg[k] = (wcol >= 0 && k < H_last) ? Wlast[(size_t)k * Wn + wcol] * inv_sqrt_h : T(0);
@@ -236,15 +246,30 @@ __global__ void __launch_bounds__(256, (conv_fwd_min_blocks<T, HP>())) conv_fwd_
         const T den = p.num_neigh ? sqrt(static_cast<const T*>(p.num_neigh)[n]) : sqrt(T(p.avg));
         T* o = OUT + (size_t)n * p.out_dim + ooff;
         const bool do_write = (wcol >= 0) && (phase == 0);
-        switch (type) {
+        if constexpr (HP == 0) {
+          // idle lanes (wcol < 0) read column 0 and write nothing
+          const T* wsrc = static_cast<const T*>(p.wpe) + (size_t)c0 * Wn + (wcol >= 0 ? wcol : 0);
+          switch (type) {
+#define MT_CONV_CASE(ID, A, B, C)                                                                   \
+  case ID:                                                                                          \
+    conv_unit<T, HP, A, B, C>(wreg, wsrc, Wn, xs, p.xs_stride, ys, p.y_dim, xoff, yoff, lo - c0,     \
+                              hi - c0, phase, nphase, cpw, o, den, first, do_write);                \
+    break;
+            MT_FOR_EACH_CG_TYPE(MT_CONV_CASE)
+#undef MT_CONV_CASE
+            default: break;
+          }
+        } else {
+          switch (type) {
 #define MT_CONV_CASE(ID, A, B, C)                                                                   \
   case ID:                                                                                          \
     conv_unit<T, HP, A, B, C>(wreg, hs, p.hp_max, xs, p.xs_stride, ys, p.y_dim, xoff, yoff, lo - c0, \
                               hi - c0, phase, nphase, cpw, o, den, first, do_write);                \
     break;
-          MT_FOR_EACH_CG_TYPE(MT_CONV_CASE)
+            MT_FOR_EACH_CG_TYPE(MT_CONV_CASE)
 #undef MT_CONV_CASE
-          default: break;
+            default: break;
+          }
         }
       }
       __syncthreads();

@@ -3,7 +3,7 @@
 #include "conv_fwd.cuh"
 
 #ifndef MT_INST_T
-#error "compile with -DMT_INST_T=float|double -DMT_INST_HP=8|16|32|64"
+#error "compile with -DMT_INST_T=float|double -DMT_INST_HP=8|16|32|64|0"
 #endif
 
 namespace mt {
